@@ -23,6 +23,8 @@ cpu_baseline  : the reference's own sources (oracle/_ref, OSQP restated) on all 
 Other workloads (supplementary lines, same JSON shape): --config 3 (BASELINE configs[2]: 65 536 shared-KKT variants on the
 FP64 tensor cores, --groups 1|8|64), --config 4 (configs[3]: 262 144 mixed trp + cub), --config 5 (configs[4]: the 1 M-scenario
 sweep, strong scaling, NCCL arg-min through the C-ABI).
+--dump-outputs DIR : after the timed steps, the outputs of the last timed step as DIR/<name>.npy (float64), so that two builds
+        can be compared output for output on the same seeded inputs (see dump_outputs).
 """
 import argparse
 import json
@@ -117,6 +119,64 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_LIMIT = 64 << 20   # bytes --dump-outputs writes at most
+DUMP_SEED = 20231020    # the scenario sample it writes when a step's outputs are larger
+# Cube fields the path defines (the reference never initialises t_dif; count is bookkeeping of its push loop)
+DUMP_SEG_FIELDS = ("beg_t", "end_t", "t", "beg_l", "end_l", "upp_skew", "upp_bias", "down_skew", "down_bias",
+                   "l_upp_skew", "l_upp_bias", "l_down_skew", "l_down_bias", "merge", "split")
+
+
+def dump_outputs(path, per_scenario, whole=None):
+    """Writes one step's outputs as <path>/<name>.npy in float64 (the integer fields convert exactly).
+
+    per_scenario: name -> array or CUDA tensor with one row per scenario (K, segs, ctrl, obj, a_cost, status, ...); `segs`
+    (raw 112-byte Cube records or a Cube structured array) is written as one segs_<field>.npy per field.  whole: name ->
+    small array written as is (the step's arg-min).  When the rows would take more than 64 MB, a fixed seeded sample of
+    scenarios is written instead, in index order, with the sampled scenario indices as scenario_index.npy."""
+    from spectral_b200.api import CUBE_DTYPE
+
+    def structured(a):
+        return getattr(a.dtype, "names", None) is not None
+
+    def values_per_row(name, a):
+        if name == "segs":
+            cubes = a.shape[1] if structured(a) else a.shape[1] // CUBE_DTYPE.itemsize
+            return cubes * len(DUMP_SEG_FIELDS)
+        return int(np.prod(a.shape[1:]))
+
+    n = len(per_scenario["K"])
+    row_bytes = 8 * sum(values_per_row(name, a) for name, a in per_scenario.items())
+    idx = None
+    if n * row_bytes > DUMP_LIMIT:
+        # (1 MB of the budget left for the .npy headers and `whole`; 8 bytes per row for scenario_index)
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, (DUMP_LIMIT - (1 << 20)) // (row_bytes + 8), replace=False))
+    os.makedirs(path, exist_ok=True)
+
+    def save(name, a):
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+    for name, a in per_scenario.items():
+        if hasattr(a, "cpu"):  # CUDA tensor: only the sampled rows leave the device
+            import torch
+            a = (a if idx is None else a.index_select(0, torch.from_numpy(idx).to(a.device))).cpu().numpy()
+        elif idx is not None:
+            a = a[idx]
+        if name == "segs":
+            cubes = a if structured(a) else np.ascontiguousarray(a).view(CUBE_DTYPE)
+            for f in DUMP_SEG_FIELDS:
+                save("segs_" + f, cubes[f])
+        else:
+            save(name, a)
+    if idx is not None:
+        save("scenario_index", idx)
+    for name, a in (whole or {}).items():
+        save(name, a.cpu().numpy() if hasattr(a, "cpu") else a)
+
+
+def _dump_dir(path, rank, world):
+    return path if world == 1 else os.path.join(path, "rank%d" % rank)
+
+
 def _host_threads():
     try:
         return max(1, len(os.sched_getaffinity(0)))
@@ -150,9 +210,11 @@ def run_reference(args):
     times = []
     kind = "port"
     for i in range(args.warmup + args.steps):
-        dt, kind, _ = _cpu_reference(batch, wl["weights"], sample, 0, wl["variant"])
+        dt, kind, result = _cpu_reference(batch, wl["weights"], sample, 0, wl["variant"])
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, result)
     total = sum(times)
     value = sample * len(times) / total
     line = {"metric": METRIC, "value": value, "unit": UNIT, "impl": "reference", "n_gpus": args.gpus,
@@ -281,6 +343,14 @@ def run_ours(args):
         dist.all_reduce(t_ms, op=dist.ReduceOp.MAX)
     ms_max = float(t_ms.item())
     value = world * B * args.steps / (ms_max * 1e-3)
+    if args.dump_outputs:  # before the supplementary passes below overwrite the output buffers
+        last = args.warmup + args.steps - 1
+        whole = {"best_cost": best_cost[last % NS], "best_index": best_idx[last % NS]}
+        if world > 1:  # what the exchange hands every rank: the arg-min over the ranks' (cost, index), ties -> lowest index
+            g = gather_buf.cpu().numpy()
+            k = np.lexsort((g[:, 1], g[:, 0]))[0]
+            whole.update(global_best_cost=g[k:k + 1, 0], global_best_index=g[k:k + 1, 1])
+        dump_outputs(_dump_dir(args.dump_outputs, rank, world), outs[last % POOL], whole)
 
     # ---- supplementary (not the headline): the same timed loop with one option changed
     def timed_variant(opts):
@@ -517,6 +587,9 @@ def run_sweep5(args):
     launches = planner.launch_count() - l0
     clk = clocks.stop() if rank == 0 else None
     value = total * args.steps / (float(ms.item()) * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(_dump_dir(args.dump_outputs, rank, world), {k: t[:n_local] for k, t in outs.items()},
+                     {"winner_" + k: np.asarray(winner[k]) for k in ("cost", "index", "rank", "K", "ctrl")})
     # every rank must hold the same winner
     chk = torch.tensor([winner["cost"], float(winner["index"]), float(winner["rank"]), float(winner["K"])], dtype=torch.float64, device=dev)
     if world > 1:
@@ -631,7 +704,7 @@ def _side_kernel_rooflines(planner, dev, peaks, peak_src):
     return out
 
 
-def main():
+def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=40)
@@ -644,7 +717,16 @@ def main():
     ap.add_argument("--no-shared", action="store_true", help="config 3 through the per-scenario kernels (A/B of the shared-KKT path)")
     ap.add_argument("--groups", type=int, default=8, help="config 3: number of shared-KKT groups (1, 8, 64)")
     ap.add_argument("--impl", default="ours", choices=("ours", "reference"))
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float64, at most 64 MB; with several ranks "
+                         "one DIR/rank<r>/ per rank)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def main(args):
     if args.impl == "reference":
         run_reference(args)
     elif args.config in (4, 5):
@@ -654,8 +736,9 @@ def main():
 
 
 if __name__ == "__main__":
+    args = parse_args()  # (outside the handler below: a usage error exits with argparse's code 2 and no traceback)
     try:
-        main()
+        main(args)
     except BaseException as exc:  # a rank that dies must not leave its peers waiting in a collective until the launcher's timeout
         if isinstance(exc, SystemExit) and exc.code in (0, None):
             raise

@@ -137,6 +137,13 @@ def test_reference_wrapper_surface_is_mirrored():
     names = [f[0] for f in api.Params._fields_]
     assert names == ["s_acc_weight", "s_jerk_weight", "l_acc_weight", "l_jerk_weight", "weight_s_ref", "weight_ds_ref",
                      "weight_l_ref", "weight_dl_ref", "weight_end_s", "weight_end_l", "iteration"]
+    # the wrapper's Params field by field (ten c_double, then the c_int iteration) and its binding of the plugin symbol,
+    # find_traj(POINTER(Params)) -> c_double (trp_wrapper.py:19-32,45-54): what an unchanged wrapper module relies on
+    assert [f[1] for f in api.Params._fields_] == [ctypes.c_double] * 10 + [ctypes.c_int]
+    assert [getattr(api.Params, n).offset for n in names] == [8 * i for i in range(11)]
+    for variant in ("trp", "cub"):
+        fn = api._plugin(variant).find_traj
+        assert fn.argtypes == (ctypes.POINTER(api.Params),) and fn.restype is ctypes.c_double
     for fn in ("find_traj", "run_btrapz", "_run_btrapz"):
         assert callable(getattr(api, fn))
 

@@ -7,6 +7,7 @@ The CPU restatement (oracle/liboracle.so) is checked against
   * tests/golden/shipped_sampling.npz  trajectory file + return value the SHIPPED binary writes for given
                                    control points (a9 sampling, a10 cost, %.3f writer),
   * tests/golden/s1_{slt,cub}_3d_31.txt  the reference's shipped known-answer outputs (SURVEY.md D.2),
+  * tests/golden/std_sort.npz      the order libstdc++'s std::sort gives equal keys (CollisionCheck's sort),
 and, where oracle/_ref was built (container with /root/reference), against the recompiled reference itself.
 Nothing here reads /root/reference at run time.
 """
@@ -135,15 +136,15 @@ def test_port_equals_recompiled_reference_on_perturbed_batch(variant):
     assert np.allclose(a["a_cost"][ok], b["a_cost"][ok], rtol=1e-9)
 
 
-@pytest.mark.skipif(not po.have_reference(), reason="oracle/_ref not built")
 def test_std_sort_restatement_equals_libstdcxx():
     """CollisionCheck's std::sort by beg_t (solve_3d.cc:630) is unstable past 16 elements; the restated
-    introsort must order equal keys exactly like libstdc++."""
-    rng = np.random.default_rng(3)
-    for n in (1, 2, 5, 16, 17, 23, 40, 64):
-        for _ in range(6):
-            keys = rng.integers(0, 8, n).astype(np.int32) * 10
-            assert np.array_equal(po.std_sort_check(keys, "port"), po.std_sort_check(keys, "reference"))
+    introsort must order equal keys exactly like libstdc++ (tests/golden/std_sort.npz: the permutations the real
+    std::sort with the reference's comparator produced, oracle/gen_std_sort_golden.py)."""
+    z = H.golden("std_sort")
+    assert int(z["n_cases"]) == 48
+    for c in range(int(z["n_cases"])):
+        keys = z["case%02d/keys" % c]
+        assert np.array_equal(po.std_sort_check(keys, "port"), z["case%02d/perm" % c]), (c, len(keys))
 
 
 def test_oracle_mixed_structure_runs_and_is_deterministic():
