@@ -18,6 +18,7 @@
  *                               (osqp_setup/osqp_solve, :1246-1249) and the Bezier sampling (:1279-1392),
  *                               and the wrapper cost (src/trp_wrapper.cpp:217-286).
  *   spectral_argmin_device()    new (the reference has no batch): best trajectory of a sweep.
+ *   spectral_topk_device()      new: the k best trajectories of a sweep (spectral_sweep_topk across GPUs).
  *   SpectralCube                struct Cube, include/btrapz/cube_type.h:2-24 (same 112-byte layout).
  *   SpectralParams              struct Params, include/btrapz/py_cpp_.h:6-21 (same 88-byte layout).
  */
@@ -243,6 +244,36 @@ int spectral_comm_init(spectral_handle_t *h, int nranks, int rank, const unsigne
 int spectral_comm_destroy(spectral_handle_t *h);
 int spectral_sweep_argmin(spectral_handle_t *h, int B_local, const SpectralOutputs *dev_out, long long index_offset,
                           SpectralWinner *winner, void *cuda_stream);
+
+/* The k best trajectories of a batch / of a multi-GPU sweep (a ranked shortlist instead of the single winner above).
+ *
+ * Order: ascending lexicographic on (cost, global index), global index = index_offset + i (index_offset >= 0).
+ *   -0.0 and +0.0 compare equal (as in spectral_argmin_device); NaN sorts after every other value, +inf included, and NaNs
+ *   rank among themselves by index.  Failed scenarios (SPECTRAL_FAIL_COST) are ordinary entries: filter with
+ *   cost < SPECTRAL_FAIL_COST.  The returned cost is the stored a_cost[i], bit for bit (a -0.0 comes back as -0.0).
+ * 1 <= k <= SPECTRAL_TOPK_MAX.  With fewer than k entries, the trailing slots hold index = -1, cost = +inf.
+ * When some cost is below 1e300, k = 1 returns exactly what spectral_argmin_device returns.
+ * B is limited only by int (not by the handle's max_batch).  Deterministic: the same bits on every call, stream and SM count.
+ *
+ * spectral_topk_device  out_cost_dev[k] / out_index_dev[k] are DEVICE pointers.  Enqueued on cuda_stream with no host
+ *                       synchronisation: an exact radix select over B costs (a fixed number of passes), compaction of the
+ *                       <= k selected entries and one sort of those (DESIGN.md 3.4).  Scratch belongs to the handle, is
+ *                       allocated on first use and does not grow with B; as for spectral_argmin_device, calls on one handle
+ *                       must not overlap in time (one stream at a time, or ordered by events).
+ * spectral_sweep_topk   collective, like spectral_sweep_argmin: local top-k -> NCCL all-gather of k 16-byte (cost, global index)
+ *                       records per rank -> the same select over the nranks x k records -> each rank packs the payloads
+ *                       (K, segments, control points) of the winners it owns into a zeroed [k] buffer, which one NCCL
+ *                       all-reduce (sum over bytes: exactly one rank writes each byte) hands to every rank.  Fills
+ *                       winners[0..k) on EVERY rank, sorted, and returns the number of real entries in *n_out
+ *                       (min(k, total scenarios)); winners[j >= *n_out] have index -1, cost +inf, rank -1, K 0.
+ *                       B_local = 0 is allowed: the rank takes part and contributes nothing (dev_out's arrays may then be
+ *                       NULL).  Shards must not overlap in global index.  Synchronises cuda_stream.  Handles without a
+ *                       communicator of more than one rank take the single-rank path (no NCCL). */
+#define SPECTRAL_TOPK_MAX 1024
+int spectral_topk_device(spectral_handle_t *h, int B, const double *a_cost_dev, long long index_offset, int k,
+                         double *out_cost_dev, long long *out_index_dev, void *cuda_stream);
+int spectral_sweep_topk(spectral_handle_t *h, int B_local, const SpectralOutputs *dev_out, long long index_offset, int k,
+                        SpectralWinner *winners, int *n_out, void *cuda_stream);
 
 /* Number of kernel launches enqueued by this handle so far (for bench accounting). */
 long long spectral_launch_count(const spectral_handle_t *h);

@@ -1,7 +1,7 @@
 """Host-side mirror of the reference's plugin interface on top of the C-ABI (include/spectral.h).
 
 * ``SpectralPlanner``       one handle per GPU around ``libspectral.so`` -- batch entry points
-  (host buffers = the end-to-end path; device tensors = the resident path; argmin).
+  (host buffers = the end-to-end path; device tensors = the resident path; argmin, top-k).
 * ``Params`` / ``find_traj`` / ``run_btrapz``  the same names, argument meaning and return values as
   the reference's ``src/trp_wrapper.py:19-32,56-121`` (``cub_wrapper.py`` likewise), bound to OUR
   ``libtrp.so`` / ``libcub.so``.
@@ -34,6 +34,7 @@ FAIL_COST = 100000000000.0
 NUM_KERNELS = 6
 NUM_CLASSES = 5
 NUM_WORK = 12
+TOPK_MAX = 1024   # SPECTRAL_TOPK_MAX
 KERNEL_NAMES = ("tables", "corridor", "classify", "qp", "finalize", "argmin")
 
 CUBE_DTYPE = np.dtype([
@@ -73,6 +74,11 @@ class SpectralWinner(ctypes.Structure):
     """SpectralWinner of include/spectral.h: the best trajectory of a (multi-GPU) sweep."""
     _fields_ = [("cost", ctypes.c_double), ("index", ctypes.c_longlong), ("rank", ctypes.c_int), ("K", ctypes.c_int),
                 ("segs", ctypes.c_ubyte * (32 * 112)), ("ctrl", ctypes.c_double * (12 * 32))]
+
+
+WINNER_DTYPE = np.dtype([("cost", np.float64), ("index", np.int64), ("rank", np.int32), ("K", np.int32),
+                         ("segs", CUBE_DTYPE, (32,)), ("ctrl", np.float64, (12 * 32,))])
+assert WINNER_DTYPE.itemsize == ctypes.sizeof(SpectralWinner)
 
 
 class Params(ctypes.Structure):
@@ -135,6 +141,10 @@ def load_library() -> ctypes.CDLL:
     lib.spectral_frenet_to_cartesian_device.argtypes = [ctypes.c_void_p, ctypes.c_longlong] + [ctypes.c_void_p] * 5
     lib.spectral_comm_unique_id.argtypes = [ctypes.POINTER(ctypes.c_ubyte)]
     lib.spectral_sweep_argmin.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_longlong, ctypes.c_void_p, ctypes.c_void_p]
+    lib.spectral_topk_device.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_longlong, ctypes.c_int,
+                                         ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
+    lib.spectral_sweep_topk.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_longlong, ctypes.c_int,
+                                        ctypes.c_void_p, ctypes.POINTER(ctypes.c_int), ctypes.c_void_p]
     _lib = lib
     return lib
 
@@ -375,6 +385,49 @@ class SpectralPlanner:
                                                      int(index_offset), ctypes.c_void_p(out_cost.data_ptr()),
                                                      ctypes.c_void_p(out_index.data_ptr()), ctypes.c_void_p(stream)))
 
+    @staticmethod
+    def _check_k(k) -> int:
+        k = int(k)
+        if not 1 <= k <= TOPK_MAX:
+            raise ValueError("k must be in [1, %d], got %d" % (TOPK_MAX, k))
+        return k
+
+    def _check_tensor(self, t, name: str, dtype, rows: int, row_elems: Optional[int] = None):
+        """`t` must be a contiguous tensor of `dtype` on this planner's GPU with at least `rows` rows (of `row_elems`
+        elements each, when given): the kernels read it through a raw pointer."""
+        import torch
+        if not isinstance(t, torch.Tensor) or not t.is_cuda or t.device.index != self.device:
+            raise ValueError("%s must be a CUDA tensor on cuda:%d" % (name, self.device))
+        if t.dtype != dtype or not t.is_contiguous():
+            raise ValueError("%s must be a contiguous %s tensor" % (name, dtype))
+        if row_elems is None:
+            if t.numel() < rows:
+                raise ValueError("%s holds %d elements, %d are needed" % (name, t.numel(), rows))
+        elif t.dim() == 0 or t.shape[0] < rows or t[0].numel() != row_elems:
+            raise ValueError("%s must have shape [>= %d, %d elements per row], got %s" % (name, rows, row_elems, tuple(t.shape)))
+
+    def topk_device(self, a_cost, k: int, index_offset: int = 0, out_cost=None, out_index=None, stream: Optional[int] = None):
+        """The k best entries of a CUDA float64 tensor, ascending on (cost, index_offset + i) (spectral_topk_device: -0.0 equals
+        +0.0, NaN last, costs returned as stored; slots beyond the number of entries are (+inf, -1)).  Returns
+        (cost float64[k], index int64[k]) on the device, enqueued on `stream` (default: the current torch stream)."""
+        import torch
+        k = self._check_k(k)
+        if index_offset < 0:
+            raise ValueError("index_offset must be non-negative")
+        self._check_tensor(a_cost, "a_cost", torch.float64, 1)
+        if out_cost is None:
+            out_cost = torch.empty(k, dtype=torch.float64, device=a_cost.device)
+        if out_index is None:
+            out_index = torch.empty(k, dtype=torch.int64, device=a_cost.device)
+        self._check_tensor(out_cost, "out_cost", torch.float64, k)
+        self._check_tensor(out_index, "out_index", torch.int64, k)
+        if stream is None:
+            stream = torch.cuda.current_stream().cuda_stream
+        self._check(self._lib.spectral_topk_device(self._h, int(a_cost.numel()), ctypes.c_void_p(a_cost.data_ptr()), int(index_offset),
+                                                   k, ctypes.c_void_p(out_cost.data_ptr()), ctypes.c_void_p(out_index.data_ptr()),
+                                                   ctypes.c_void_p(stream)))
+        return out_cost, out_index
+
     # ---- multi-GPU exchange through the C-ABI (NCCL inside libspectral.so)
     @staticmethod
     def comm_unique_id() -> bytes:
@@ -406,6 +459,41 @@ class SpectralPlanner:
         segs = np.frombuffer(bytes(w.segs), dtype=CUBE_DTYPE)[:max(K, 0)].copy()
         return dict(cost=float(w.cost), index=int(w.index), rank=int(w.rank), K=K, segs=segs,
                     ctrl=np.array(w.ctrl[:12 * max(K, 0)], dtype=np.float64))
+
+    def sweep_topk(self, outputs: dict, index_offset: int, k: int, B: Optional[int] = None, stream: Optional[int] = None) -> list:
+        """Collective over all ranks of the communicator (spectral_sweep_topk): this rank's shard results -> the sweep's k best
+        trajectories on every rank, as a list of min(k, total scenarios) dicts shaped like sweep_argmin's.  B = 0: this rank
+        takes part without scenarios."""
+        import torch
+        k = self._check_k(k)
+        if stream is None:
+            stream = torch.cuda.current_stream().cuda_stream
+        B = int(outputs["a_cost"].numel()) if B is None else int(B)
+        if B < 0:
+            raise ValueError("B must be non-negative")
+        if index_offset < 0:
+            raise ValueError("index_offset must be non-negative")
+        out = SpectralOutputs()
+        if B > 0:
+            self._check_tensor(outputs["a_cost"], "a_cost", torch.float64, B)
+            self._check_tensor(outputs["K"], "K", torch.int32, B)
+            self._check_tensor(outputs["segs"], "segs", torch.uint8, B, self.k_max * 112)
+            self._check_tensor(outputs["ctrl"], "ctrl", torch.float64, B, 12 * self.k_max)
+            out.K = ctypes.cast(ctypes.c_void_p(outputs["K"].data_ptr()), _ip)
+            out.segs = outputs["segs"].data_ptr()
+            out.ctrl = ctypes.cast(ctypes.c_void_p(outputs["ctrl"].data_ptr()), _dp)
+            out.a_cost = ctypes.cast(ctypes.c_void_p(outputs["a_cost"].data_ptr()), _dp)
+        ws = (SpectralWinner * k)()
+        n = ctypes.c_int()
+        self._check(self._lib.spectral_sweep_topk(self._h, B, ctypes.byref(out), int(index_offset), k, ws, ctypes.byref(n),
+                                                  ctypes.c_void_p(stream)))
+        arr = np.frombuffer(ws, dtype=WINNER_DTYPE, count=n.value)
+        res = []
+        for w in arr:
+            K = max(int(w["K"]), 0)
+            res.append(dict(cost=float(w["cost"]), index=int(w["index"]), rank=int(w["rank"]), K=int(w["K"]),
+                            segs=w["segs"][:K].copy(), ctrl=w["ctrl"][:12 * K].copy()))
+        return res
 
     # ---- upstream of the path (Car.getCar / get_bounds of src/cart_frenet.py:644-1026), CUDA tensors in and out
     def bounds_device(self, obstacles, n_knots: int, r_cap: int, n_obs=None, road=ROAD, stream: Optional[int] = None):

@@ -24,6 +24,7 @@
 #include "qp_shared.cuh"
 #include "qp_shared4.cuh"
 #include "tables.cuh"
+#include "topk.cuh"
 
 static_assert(SPECTRAL_NUM_CLASSES == SP_NUM_CLASSES && SPECTRAL_NUM_WORK >= 6 + SP_NUM_CLASSES, "include/spectral.h");
 
@@ -403,6 +404,13 @@ struct spectral_handle {
   int nranks = 1, rank = 0;
   double *xg_rec = nullptr;        // [1 + nranks] (cost, index) records, 16 bytes each
   unsigned char *xg_pay = nullptr; // winner payload
+  // top-k selection (topk.cuh), allocated on first use: select scratch (independent of B), then the sweep_topk exchange
+  TopkScratch tk{};
+  double *tk_rec = nullptr;             // (2 + nranks) x k_cap 16-byte records: local, merged, gathered
+  unsigned char *tk_pay = nullptr;      // [k_cap][kPayBytes] winner payloads (device)
+  unsigned char *tk_hostpay = nullptr;  // the same, page-locked host copy
+  double *tk_hostrec = nullptr;         // [k_cap] merged records, page-locked host copy
+  int tk_cap = 0, tk_cap_ranks = 0;
   int classes_timed = 0;    // solver classes launched per call (k_max dependent)
   int corridor_smem = 0;    // dynamic shared memory the corridor kernel is opted in for on this handle's device
   bool legacy_qpd = false;  // SPECTRAL_LEGACY_QPD=1: the round-1 full-row kernels for K <= 10 (A/B measurements)
@@ -486,6 +494,10 @@ extern "C" int spectral_destroy(spectral_handle_t *h) {
   if (h->comm) spectral_comm_destroy(h);
   if (h->xg_rec) cudaFree(h->xg_rec);
   if (h->xg_pay) cudaFree(h->xg_pay);
+  void *tkb[] = {h->tk.hist, h->tk.st, h->tk.block_ties, h->tk.ck, h->tk.ci, h->tk.cc, h->tk_rec, h->tk_pay};
+  for (void *p : tkb) if (p) cudaFree(p);
+  if (h->tk_hostpay) cudaFreeHost(h->tk_hostpay);
+  if (h->tk_hostrec) cudaFreeHost(h->tk_hostrec);
   void *qsb[] = {h->qs_keys, h->qs_keys2, h->qs_ids, h->qs_ids2, h->qs_tmp, h->qs_tile, h->qs_leader, h->qs_misc, h->qs_st, h->qs_blk, h->qs_lu,
                  h->qs_qv, h->qs_w, h->qs_x, h->qs_cub, h->qs_fs};
   for (void *p : qsb) if (p) cudaFree(p);
@@ -932,6 +944,58 @@ extern "C" int spectral_argmin_device(spectral_handle_t *h, int B, const double 
   return SPECTRAL_SUCCESS;
 }
 
+// ------------------------------------------------------------------ top-k selection (topk.cuh)
+static int ensure_topk_scratch(spectral_handle *h, cudaStream_t st) {
+  if (h->tk.cc) return SPECTRAL_SUCCESS;  // the last allocation: set only when all of them succeeded
+  const size_t hist_bytes = (size_t)TK_PASSES_MAX * TK_BINS * 4;
+  if (!h->tk.hist) CK(cudaMalloc(&h->tk.hist, hist_bytes));
+  if (!h->tk.st) CK(cudaMalloc(&h->tk.st, sizeof(TopkState)));
+  if (!h->tk.block_ties) CK(cudaMalloc(&h->tk.block_ties, TK_GRID_MAX * 4));
+  if (!h->tk.ck) CK(cudaMalloc(&h->tk.ck, TK_MAX * 8));
+  if (!h->tk.ci) CK(cudaMalloc(&h->tk.ci, TK_MAX * 8));
+  CK(cudaMemsetAsync(h->tk.hist, 0, hist_bytes, st));  // the kernels restore zero histograms, ticket and counter behind them
+  CK(cudaMemsetAsync(h->tk.st, 0, sizeof(TopkState), st));
+  CK(cudaMalloc(&h->tk.cc, TK_MAX * 8));
+  return SPECTRAL_SUCCESS;
+}
+
+// npass + 2 launches: the radix passes (6 implicit, 12 explicit), compaction, finish (ties + sort + output)
+static int topk_run(spectral_handle *h, TopkArgs a, cudaStream_t st) {
+  { const int rc = ensure_topk_scratch(h, st); if (rc) return rc; }
+  a.s = h->tk;
+  const long long per_block = (long long)TK_THREADS * TK_UNROLL;
+  const int cap = 4 * h->sm_count < TK_GRID_MAX ? 4 * h->sm_count : TK_GRID_MAX;
+  const long long want = ((long long)a.n + per_block - 1) / per_block;
+  const int grid = want < cap ? (int)want : cap;
+  const int npass = (a.total_bits + TK_BITS - 1) / TK_BITS;
+  for (int p = 0; p < npass; p++) k_topk_pass<<<grid, TK_THREADS, 0, st>>>(a, p);
+  k_topk_compact<<<grid, TK_THREADS, 0, st>>>(a);
+  k_topk_finish<<<grid, TK_FIN_THREADS, 0, st>>>(a);
+  h->launches += npass + 2;
+  CK(cudaGetLastError());
+  return SPECTRAL_SUCCESS;
+}
+
+static int topk_implicit(spectral_handle *h, int B, const double *cost, long long index_offset, int k, double *out_cost,
+                         long long *out_index, int out_stride, cudaStream_t st) {
+  TopkArgs a{};
+  a.cost = cost; a.index = nullptr; a.index_offset = index_offset; a.cost_stride = 1;
+  a.n = B; a.keff = k < B ? k : B; a.k = k; a.total_bits = 64;
+  a.out_cost = out_cost; a.out_index = out_index; a.out_stride = out_stride;
+  return topk_run(h, a, st);
+}
+
+extern "C" int spectral_topk_device(spectral_handle_t *h, int B, const double *a_cost_dev, long long index_offset, int k,
+                                    double *out_cost_dev, long long *out_index_dev, void *cuda_stream) {
+  if (!h) return SPECTRAL_ERR_INVALID;
+  if (k < 1 || k > SPECTRAL_TOPK_MAX) return fail(h, SPECTRAL_ERR_INVALID, "topk: k must be in [1, SPECTRAL_TOPK_MAX]");
+  if (B <= 0) return fail(h, SPECTRAL_ERR_INVALID, "topk: B must be positive");
+  if (index_offset < 0) return fail(h, SPECTRAL_ERR_INVALID, "topk: index_offset must be non-negative");
+  if (!a_cost_dev || !out_cost_dev || !out_index_dev) return fail(h, SPECTRAL_ERR_INVALID, "topk: NULL pointer");
+  CK(cudaSetDevice(h->device));
+  return topk_implicit(h, B, a_cost_dev, index_offset, k, out_cost_dev, out_index_dev, 1, (cudaStream_t)cuda_stream);
+}
+
 // ------------------------------------------------------------------ upstream of the path (SURVEY.md 8f row 1)
 extern "C" int spectral_bounds_device(spectral_handle_t *h, int B, int N, int M, const double *obstacles_dev, const int *n_obs_dev,
                                       const double road[4], int R_cap, double *s_bounds_dev, double *l_bounds_dev, int *n_lanes_dev,
@@ -977,6 +1041,7 @@ struct NcclApi {
   ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
   ncclResult_t (*AllGather)(const void *, void *, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
   ncclResult_t (*Broadcast)(const void *, void *, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
+  ncclResult_t (*AllReduce)(const void *, void *, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
   const char *(*GetErrorString)(ncclResult_t) = nullptr;
 };
 NcclApi *nccl_api() {
@@ -993,8 +1058,10 @@ NcclApi *nccl_api() {
       api.CommDestroy = (decltype(api.CommDestroy))dlsym(api.lib, "ncclCommDestroy");
       api.AllGather = (decltype(api.AllGather))dlsym(api.lib, "ncclAllGather");
       api.Broadcast = (decltype(api.Broadcast))dlsym(api.lib, "ncclBroadcast");
+      api.AllReduce = (decltype(api.AllReduce))dlsym(api.lib, "ncclAllReduce");
       api.GetErrorString = (decltype(api.GetErrorString))dlsym(api.lib, "ncclGetErrorString");
-      if (!api.GetUniqueId || !api.CommInitRank || !api.CommDestroy || !api.AllGather || !api.Broadcast) api.lib = nullptr;
+      if (!api.GetUniqueId || !api.CommInitRank || !api.CommDestroy || !api.AllGather || !api.Broadcast || !api.AllReduce)
+        api.lib = nullptr;
     }
   }
   return api.lib ? &api : nullptr;
@@ -1026,6 +1093,28 @@ __global__ void k_pack_winner(const WinnerRec *win, long long offset, int B, int
   for (int k = threadIdx.x; k < 32; k += blockDim.x)
     if (k < Kw && k < k_max) ps[k] = segs[(size_t)loc * k_max + k];
   for (int j = threadIdx.x; j < 12 * 32; j += blockDim.x) pc[j] = (j < 12 * Kw && j < 12 * k_max) ? ctrl[(size_t)loc * 12 * k_max + j] : 0.0;
+}
+// top-k exchange: slot j of the payload buffer gets winner j's payload from the rank that owns it (header: K, rank, 1, 0);
+// every other rank leaves the slot zero, so a byte-wise sum over ranks reproduces it exactly
+__global__ void k_pack_topk(const WinnerRec *win, int rank, long long offset, int B, int k_max, const int *K, const SpectralCube *segs,
+                            const double *ctrl, unsigned char *pay) {
+  const int j = blockIdx.x;
+  const long long idx = win[j].idx, loc = idx - offset;
+  if (idx < 0 || loc < 0 || loc >= B) return;
+  unsigned char *p = pay + (size_t)j * kPayBytes;
+  int *hdr = (int *)p;
+  const int Kw = K[loc];
+  if (threadIdx.x == 0) { hdr[0] = Kw; hdr[1] = rank; hdr[2] = 1; hdr[3] = 0; }
+  SpectralCube *ps = (SpectralCube *)(p + 16);
+  double *pc = (double *)(p + 16 + 32 * sizeof(SpectralCube));
+  for (int q = threadIdx.x; q < 32; q += blockDim.x)
+    if (q < Kw && q < k_max) ps[q] = segs[(size_t)loc * k_max + q];
+  for (int q = threadIdx.x; q < 12 * 32; q += blockDim.x) pc[q] = (q < 12 * Kw && q < 12 * k_max) ? ctrl[(size_t)loc * 12 * k_max + q] : 0.0;
+}
+// a rank without scenarios contributes k empty records (+inf, -1): ranked after every real entry by the merge
+__global__ void k_empty_records(WinnerRec *rec, int k) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j < k) { rec[j].cost = __longlong_as_double(0x7FF0000000000000LL); rec[j].idx = -1; }
 }
 }  // namespace
 
@@ -1107,6 +1196,82 @@ extern "C" int spectral_sweep_argmin(spectral_handle_t *h, int B_local, const Sp
   winner->K = hdr[0];
   memcpy(winner->segs, hostpay + 16, 32 * sizeof(SpectralCube));
   memcpy(winner->ctrl, hostpay + 16 + 32 * sizeof(SpectralCube), 12 * 32 * 8);
+  return SPECTRAL_SUCCESS;
+}
+
+extern "C" int spectral_sweep_topk(spectral_handle_t *h, int B_local, const SpectralOutputs *dev_out, long long index_offset, int k,
+                                   SpectralWinner *winners, int *n_out, void *cuda_stream) {
+  if (!h) return SPECTRAL_ERR_INVALID;
+  if (k < 1 || k > SPECTRAL_TOPK_MAX) return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: k must be in [1, SPECTRAL_TOPK_MAX]");
+  if (B_local < 0) return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: B_local must be non-negative");
+  if (index_offset < 0) return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: index_offset must be non-negative");
+  if (!dev_out || !winners || !n_out) return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: NULL pointer");
+  if (B_local > 0 && (!dev_out->a_cost || !dev_out->K || !dev_out->segs || !dev_out->ctrl))
+    return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: a_cost/K/segs/ctrl are required");
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  const bool multi = h->nranks > 1;
+  NcclApi *n = multi ? nccl_api() : nullptr;
+  if (multi && (!n || !h->comm)) return fail(h, SPECTRAL_ERR_INVALID, "spectral_comm_init has not been called on this handle");
+  const int nr = multi ? h->nranks : 1;
+  if (h->tk_cap < k || h->tk_cap_ranks < nr) {  // sized by k and the number of ranks, never by the batch
+    if (h->tk_rec) cudaFree(h->tk_rec);
+    if (h->tk_pay) cudaFree(h->tk_pay);
+    if (h->tk_hostpay) cudaFreeHost(h->tk_hostpay);
+    if (h->tk_hostrec) cudaFreeHost(h->tk_hostrec);
+    h->tk_rec = nullptr; h->tk_pay = nullptr; h->tk_hostpay = nullptr; h->tk_hostrec = nullptr; h->tk_cap = 0;
+    CK(cudaMalloc(&h->tk_rec, (size_t)(2 + nr) * k * sizeof(WinnerRec)));
+    CK(cudaMalloc(&h->tk_pay, (size_t)k * kPayBytes));
+    CK(cudaHostAlloc(&h->tk_hostpay, (size_t)k * kPayBytes, cudaHostAllocDefault));
+    CK(cudaHostAlloc(&h->tk_hostrec, (size_t)k * sizeof(WinnerRec), cudaHostAllocDefault));
+    h->tk_cap = k; h->tk_cap_ranks = nr;
+  }
+  WinnerRec *loc = (WinnerRec *)h->tk_rec, *merged = loc + k, *all = loc + 2 * k;
+  if (B_local > 0) {
+    const int rc = topk_implicit(h, B_local, dev_out->a_cost, index_offset, k, &loc->cost, &loc->idx, 2, st);
+    if (rc) return rc;
+  } else {
+    k_empty_records<<<(k + 255) / 256, 256, 0, st>>>(loc, k);
+    h->launches++;
+  }
+  const WinnerRec *win = loc;
+  if (multi) {  // phase 1: every rank's k records -> the same select over nranks x k records (explicit indices)
+    if (n->AllGather(loc, all, (size_t)k * sizeof(WinnerRec), ncclUint8, h->comm, st) != ncclSuccess) return fail(h, SPECTRAL_ERR_CUDA, "ncclAllGather");
+    TopkArgs a{};
+    a.cost = &all->cost; a.index = &all->idx; a.cost_stride = 2;
+    a.n = nr * k; a.keff = k; a.k = k; a.total_bits = 128;
+    a.out_cost = &merged->cost; a.out_index = &merged->idx; a.out_stride = 2;
+    const int rc = topk_run(h, a, st);
+    if (rc) return rc;
+    win = merged;
+  }
+  // phase 2: payloads of the winners this rank owns, summed over ranks
+  CK(cudaMemsetAsync(h->tk_pay, 0, (size_t)k * kPayBytes, st));
+  k_pack_topk<<<k, 128, 0, st>>>(win, multi ? h->rank : 0, index_offset, B_local, h->k_max, dev_out->K, dev_out->segs, dev_out->ctrl, h->tk_pay);
+  h->launches++;
+  CK(cudaGetLastError());
+  if (multi && n->AllReduce(h->tk_pay, h->tk_pay, (size_t)k * kPayBytes, ncclUint8, ncclSum, h->comm, st) != ncclSuccess)
+    return fail(h, SPECTRAL_ERR_CUDA, "ncclAllReduce");
+  WinnerRec *hrec = (WinnerRec *)h->tk_hostrec;
+  CK(cudaMemcpyAsync(hrec, win, (size_t)k * sizeof(WinnerRec), cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  int cnt = 0;
+  while (cnt < k && hrec[cnt].idx >= 0) cnt++;
+  if (cnt) {
+    CK(cudaMemcpyAsync(h->tk_hostpay, h->tk_pay, (size_t)cnt * kPayBytes, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+  }
+  for (int j = 0; j < k; j++) {
+    SpectralWinner *w = winners + j;
+    memset(w, 0, sizeof(*w));
+    if (j >= cnt) { w->cost = __builtin_huge_val(); w->index = -1; w->rank = -1; continue; }
+    const unsigned char *p = h->tk_hostpay + (size_t)j * kPayBytes;
+    const int *hdr = (const int *)p;
+    w->cost = hrec[j].cost; w->index = hrec[j].idx; w->rank = hdr[1]; w->K = hdr[0];
+    memcpy(w->segs, p + 16, 32 * sizeof(SpectralCube));
+    memcpy(w->ctrl, p + 16 + 32 * sizeof(SpectralCube), 12 * 32 * 8);
+  }
+  *n_out = cnt;
   return SPECTRAL_SUCCESS;
 }
 
