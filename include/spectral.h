@@ -19,6 +19,8 @@
  *                               and the wrapper cost (src/trp_wrapper.cpp:217-286).
  *   spectral_argmin_device()    new (the reference has no batch): best trajectory of a sweep.
  *   spectral_topk_device()      new: the k best trajectories of a sweep (spectral_sweep_topk across GPUs).
+ *   spectral_eval_device()      new: solved trajectories at caller-chosen times (the sampler of Optimize, :1351-1390, on
+ *                               any time grid, with jerk).
  *   SpectralCube                struct Cube, include/btrapz/cube_type.h:2-24 (same 112-byte layout).
  *   SpectralParams              struct Params, include/btrapz/py_cpp_.h:6-21 (same 88-byte layout).
  */
@@ -223,6 +225,31 @@ int spectral_ego_states_device(spectral_handle_t *h, int B, const double *sample
                                const double *s_offset_dev, int offset_stride, double *states_dev, void *cuda_stream);
 int spectral_frenet_to_cartesian_device(spectral_handle_t *h, long long n, const double *ref_dev, const double *s_cond_dev,
                                         const double *d_cond_dev, double *out_dev, void *cuda_stream);
+
+/* Trajectories of solved scenarios evaluated at caller-chosen times (device buffers, enqueued on cuda_stream, no
+ * synchronisation).  Works on any solve output, including a top-k winner or an earlier plan uploaded into [k] arrays.
+ *   dev_out    K, segs, ctrl and status of B scenarios, all required, in the handle's k_max layout (as spectral_sweep_argmin).
+ *   times_dev  [T] (times_stride 0: the same times for every scenario) or [B][T] (times_stride 1), seconds.
+ *   states_dev [B][T][6] = (s, ds, dds, l, dl, ddl): the layout of `samples` and of SpectralInputs.init, so with T = 1 it
+ *              is the next solve's init, and it feeds spectral_ego_states_device directly (samples_cap = npts = T).
+ *   jerk_dev   [B][T][2] = (ddds, dddl), or NULL.      horizon_dev [B] = H, or NULL.
+ * B is limited only by int (not by the handle's max_batch); B * T may exceed 2^31.
+ * Time model.  tau = 0 is the initial state.  Segment k spans [T_k, T_{k+1}], T_0 = 0, T_{k+1} = T_k + segs[k].t, summed in
+ *   double in array order (the corridor order, not beg_t: the cuboid variant leaves beg_t unsorted); H = T_K.  A time at a
+ *   joint belongs to the segment that ends there (the reference's sampler also ends each segment at u = 1).  Segments with
+ *   t_k <= 1e-9 (CorridorSplit's slivers) are never selected; a time past the last selectable segment's end evaluates it
+ *   at u = 1.  u = clamp((tau - T_k) / t_k, 0, 1), c = ctrl[6k .. 6k+6) (s axis; l axis: ctrl[6K + 6k ..]),
+ *     s = t_k sum c_i B5_i(u),  ds = 5 sum (c_{i+1} - c_i) B4_i(u),  dds = 20 sum D2c_i B3_i(u) / t_k,
+ *     ddds = 60 sum D3c_i B2_i(u) / t_k^2            (the arithmetic of the `samples` of spectral_solve_batch*)
+ *   Times in [-1e-9, H + 1e-9] are valid and clamped to [0, H], so a horizon end computed as (N - 1) delta is not lost to
+ *   the rounding of the summed durations.
+ * NaN rows of states and jerk: times outside that range or NaN (the scenario's horizon is still H); every row of a
+ *   scenario whose status is not SOLVED or SOLVED_INACCURATE or whose K is outside [1, k_max] (its horizon is NaN too)
+ *   or whose segments are all slivers (horizon H).  segs / ctrl are never read beyond K.
+ * SPECTRAL_ERR_INVALID: null handle, dev_out, K/segs/ctrl/status, times_dev or states_dev; B < 1; T < 1; times_stride
+ *   other than 0 or 1. */
+int spectral_eval_device(spectral_handle_t *h, int B, const SpectralOutputs *dev_out, int T, const double *times_dev,
+                         int times_stride, double *states_dev, double *jerk_dev, double *horizon_dev, void *cuda_stream);
 
 /* Multi-GPU sweep (SURVEY.md 8e): scenarios are sharded over ranks (one handle = one GPU = one rank); the ONLY exchange is
  * the best trajectory: local arg-min (k_argmin) -> NCCL all-gather of one 16-byte (cost, global index) record per rank ->

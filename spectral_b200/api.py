@@ -145,6 +145,8 @@ def load_library() -> ctypes.CDLL:
                                          ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
     lib.spectral_sweep_topk.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_longlong, ctypes.c_int,
                                         ctypes.c_void_p, ctypes.POINTER(ctypes.c_int), ctypes.c_void_p]
+    lib.spectral_eval_device.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(SpectralOutputs), ctypes.c_int, ctypes.c_void_p,
+                                         ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
     _lib = lib
     return lib
 
@@ -538,6 +540,46 @@ class SpectralPlanner:
                                                                   ctypes.c_void_p(d_cond.data_ptr()), ctypes.c_void_p(out.data_ptr()),
                                                                   ctypes.c_void_p(stream)))
         return out
+
+    # ---- solved trajectories at caller-chosen times (spectral_eval_device)
+    def eval_device(self, outputs: dict, times, B: Optional[int] = None, jerk: bool = False, stream: Optional[int] = None):
+        """The trajectories of `outputs` (alloc_device_outputs / solve_device: K, segs, ctrl, status) at `times`, a CUDA
+        float64 tensor [T] (every scenario) or [B, T] (per scenario).  Returns (states float64 [B, T, 6] = (s, ds, dds, l, dl,
+        ddl), jerk float64 [B, T, 2] = (ddds, dddl) or None, horizon float64 [B]), enqueued on `stream` (default: the
+        current torch stream).  NaN rows for times outside [-1e-9, H + 1e-9] and for failed scenarios (include/spectral.h)."""
+        import torch
+        B = int(outputs["K"].numel()) if B is None else int(B)
+        if B < 1:
+            raise ValueError("B must be positive")
+        self._check_tensor(outputs["K"], "K", torch.int32, B)
+        self._check_tensor(outputs["status"], "status", torch.int32, B)
+        self._check_tensor(outputs["segs"], "segs", torch.uint8, B, self.k_max * 112)
+        self._check_tensor(outputs["ctrl"], "ctrl", torch.float64, B, 12 * self.k_max)
+        if not isinstance(times, torch.Tensor) or times.dim() not in (1, 2):
+            raise ValueError("times must be a tensor of shape [T] or [B, T]")
+        T = int(times.shape[-1])
+        if T < 1:
+            raise ValueError("times is empty")
+        if times.dim() == 2:
+            self._check_tensor(times, "times", torch.float64, B, T)
+        else:
+            self._check_tensor(times, "times", torch.float64, T)
+        dev = times.device
+        states = torch.empty(B, T, 6, dtype=torch.float64, device=dev)
+        jk = torch.empty(B, T, 2, dtype=torch.float64, device=dev) if jerk else None
+        horizon = torch.empty(B, dtype=torch.float64, device=dev)
+        out = SpectralOutputs()
+        out.K = ctypes.cast(ctypes.c_void_p(outputs["K"].data_ptr()), _ip)
+        out.status = ctypes.cast(ctypes.c_void_p(outputs["status"].data_ptr()), _ip)
+        out.segs = outputs["segs"].data_ptr()
+        out.ctrl = ctypes.cast(ctypes.c_void_p(outputs["ctrl"].data_ptr()), _dp)
+        if stream is None:
+            stream = torch.cuda.current_stream(dev).cuda_stream
+        self._check(self._lib.spectral_eval_device(self._h, B, ctypes.byref(out), T, ctypes.c_void_p(times.data_ptr()),
+                                                   1 if times.dim() == 2 else 0, ctypes.c_void_p(states.data_ptr()),
+                                                   ctypes.c_void_p(jk.data_ptr()) if jk is not None else None,
+                                                   ctypes.c_void_p(horizon.data_ptr()), ctypes.c_void_p(stream)))
+        return states, jk, horizon
 
     def launch_count(self) -> int:
         return int(self._lib.spectral_launch_count(self._h))

@@ -17,6 +17,7 @@
 #include "bounds.cuh"
 #include "corridor.cuh"
 #include "downstream.cuh"
+#include "eval.cuh"
 #include "finalize.cuh"
 #include "qp.cuh"
 #include "qp_dense.cuh"
@@ -1027,6 +1028,61 @@ extern "C" int spectral_frenet_to_cartesian_device(spectral_handle_t *h, long lo
   if (!h || n <= 0 || !ref_dev || !s_cond_dev || !d_cond_dev || !out_dev) return SPECTRAL_ERR_INVALID;
   CK(cudaSetDevice(h->device));
   k_frenet_to_cartesian<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)cuda_stream>>>(ref_dev, s_cond_dev, d_cond_dev, out_dev, n);
+  h->launches++;
+  CK(cudaGetLastError());
+  return SPECTRAL_SUCCESS;
+}
+
+// ------------------------------------------------------------------ trajectories at caller-chosen times (eval.cuh)
+// Flat grid-stride loop over the B*T points, one thread per point.  A block's points are consecutive in the output, so
+// they are staged in shared memory and written back as one contiguous run (the 6- and 2-double rows would otherwise
+// be strided stores); the scenario's durations and control points are read through L1.
+#define EVAL_THREADS 256
+__global__ void __launch_bounds__(EVAL_THREADS) k_eval(const EvalArgs a, double *states, double *jerk, double *horizon) {
+  __shared__ double s_st[EVAL_THREADS * 6];
+  __shared__ double s_jk[EVAL_THREADS * 2];
+  __shared__ long long s_b0;
+  __shared__ int s_j0;
+  const long long n = (long long)a.B * a.T;
+  for (long long base = (long long)blockIdx.x * EVAL_THREADS; base < n; base += (long long)gridDim.x * EVAL_THREADS) {
+    if (threadIdx.x == 0) { s_b0 = base / a.T; s_j0 = (int)(base - s_b0 * a.T); }  // one 64-bit division per tile
+    __syncthreads();
+    const long long p = base + threadIdx.x;
+    if (p < n) {
+      const unsigned off = (unsigned)s_j0 + threadIdx.x;  // < 2^31 + EVAL_THREADS
+      const int b = (int)(s_b0 + off / (unsigned)a.T), j = (int)(off % (unsigned)a.T);
+      double st[6], jk[2];
+      const double H = eval_point(a, b, j, st, jk);
+#pragma unroll
+      for (int i = 0; i < 6; i++) s_st[6 * threadIdx.x + i] = st[i];
+      s_jk[2 * threadIdx.x] = jk[0];
+      s_jk[2 * threadIdx.x + 1] = jk[1];
+      if (horizon && j == 0) horizon[b] = H;
+    }
+    __syncthreads();
+    const int cnt = n - base < EVAL_THREADS ? (int)(n - base) : EVAL_THREADS;
+    double *so = states + 6 * base;
+    for (int i = threadIdx.x; i < 6 * cnt; i += EVAL_THREADS) so[i] = s_st[i];
+    if (jerk) {
+      double *jo = jerk + 2 * base;
+      for (int i = threadIdx.x; i < 2 * cnt; i += EVAL_THREADS) jo[i] = s_jk[i];
+    }
+    __syncthreads();
+  }
+}
+
+extern "C" int spectral_eval_device(spectral_handle_t *h, int B, const SpectralOutputs *dev_out, int T, const double *times_dev,
+                                    int times_stride, double *states_dev, double *jerk_dev, double *horizon_dev, void *cuda_stream) {
+  if (!h) return SPECTRAL_ERR_INVALID;
+  if (!dev_out || !dev_out->K || !dev_out->segs || !dev_out->ctrl || !dev_out->status)
+    return fail(h, SPECTRAL_ERR_INVALID, "eval: K/segs/ctrl/status are required");
+  if (!times_dev || !states_dev) return fail(h, SPECTRAL_ERR_INVALID, "eval: NULL times or states");
+  if (B < 1 || T < 1) return fail(h, SPECTRAL_ERR_INVALID, "eval: B and T must be positive");
+  if (times_stride != 0 && times_stride != 1) return fail(h, SPECTRAL_ERR_INVALID, "eval: times_stride must be 0 or 1");
+  CK(cudaSetDevice(h->device));
+  const EvalArgs a{B, T, h->k_max, times_stride, dev_out->K, dev_out->status, dev_out->segs, dev_out->ctrl, times_dev};
+  const long long want = ((long long)B * T + EVAL_THREADS - 1) / EVAL_THREADS, cap = 8LL * h->sm_count;
+  k_eval<<<(unsigned)(want < cap ? want : cap), EVAL_THREADS, 0, (cudaStream_t)cuda_stream>>>(a, states_dev, jerk_dev, horizon_dev);
   h->launches++;
   CK(cudaGetLastError());
   return SPECTRAL_SUCCESS;

@@ -4,6 +4,7 @@
 //   cost:     find_traj, trp_wrapper.cpp:217-286 | cub_wrapper.cpp:210-258
 #pragma once
 #include "common.cuh"
+#include "eval.cuh"
 #include "qp.cuh"
 
 struct FinalArgs {
@@ -27,13 +28,6 @@ struct FinalArgs {
 #define SP_NUM_CLASSES 5
 SP_DEV int lane_class(int K) { return K <= 8 ? 0 : (K <= 10 ? 1 : (K <= 12 ? 2 : (K <= 16 ? 3 : 4))); }
 SP_HD int class_kcap(int cls) { return cls == 0 ? 8 : (cls == 1 ? 10 : (cls == 2 ? 12 : (cls == 3 ? 16 : 32))); }
-
-SP_DEV void bernstein_powers(double u, double up[6], double vp[6]) {
-  up[0] = 1.0; vp[0] = 1.0;
-  const double v = 1 - u;
-#pragma unroll
-  for (int i = 1; i < 6; i++) { up[i] = up[i - 1] * u; vp[i] = vp[i - 1] * v; }
-}
 
 // one thread per scenario
 SP_DEV void finalize_body(const FinalArgs &a, int b) {
@@ -71,7 +65,6 @@ SP_DEV void finalize_body(const FinalArgs &a, int b) {
     int num_of_points = 1;  // solve_3d.h:114
     for (int k = 0; k < K; k++) num_of_points = (int)((double)num_of_points + segs[k].t / delta);  // int += double (:1281)
     const bool trp = a.variant == SPECTRAL_TRP;
-    const double bc0[6] = {1, 5, 10, 10, 5, 1}, bc1[5] = {1, 4, 6, 4, 1}, bc2[4] = {1, 3, 3, 1};
     double s_cost = 0.0, l_cost = 0.0, smax = 0.0, lmax = 0.0;
     double prev_dds = 0.0, prev_ddl = 0.0, l_end = 0.0;
     const int end_idx = (N - 1 < num_of_points) ? N - 1 : num_of_points - 1;
@@ -114,22 +107,10 @@ SP_DEV void finalize_body(const FinalArgs &a, int b) {
       const int linter = (int)(t / delta);  // :1351
       for (int l = 1; l <= linter; l++) {
         if (var_index >= num_of_points) { overflow = true; break; }  // x_.at() would throw
-        double up[6], vp[6];
+        double up[6], vp[6], o[6];
         bernstein_powers((double)l / linter, up, vp);
-        double x = 0, y = 0, dx = 0, dy = 0, ddx = 0, ddy = 0;
-#pragma unroll
-        for (int i = 0; i < 6; i++) { const double bb = bc0[i] * up[i] * vp[5 - i]; x += cs[i] * bb; y += cl[i] * bb; }
-#pragma unroll
-        for (int i = 0; i < 5; i++) {
-          const double bb = bc1[i] * up[i] * vp[4 - i];
-          dx += 5.0 * (cs[i + 1] - cs[i]) * bb; dy += 5.0 * (cl[i + 1] - cl[i]) * bb;
-        }
-#pragma unroll
-        for (int i = 0; i < 4; i++) {
-          const double bb = bc2[i] * up[i] * vp[3 - i];
-          ddx += 20.0 * (cs[i + 2] - 2.0 * cs[i + 1] + cs[i]) * bb; ddy += 20.0 * (cl[i + 2] - 2.0 * cl[i + 1] + cl[i]) * bb;
-        }
-        emit(x * t, dx, ddx / t, y * t, dy, ddy / t);
+        bezier_state(cs, cl, t, up, vp, o);
+        emit(o[0], o[1], o[2], o[3], o[4], o[5]);
       }
     }
     if (overflow || var_index != num_of_points) {  // CHECK_EQ(var_index, num_of_points_) -> abort (:1407)
