@@ -99,13 +99,10 @@ __global__ void __launch_bounds__(32 * WPB) k_qp(const QpArgs a) {
 }
 
 // dense-operator ADMM kernel (qp_dense.cuh): one CTA (2 TA threads) per scenario of this class
-#ifndef QPD_MINBLOCKS
-#define QPD_MINBLOCKS(KC) ((KC) <= 10 ? 2 : 1)  // CTAs per SM the register budget is capped for
-#endif
-// Persistent like k_qpa: QPD_MINBLOCKS CTAs per SM take scenarios of the class from the device-side queue (a.next) until
-// the list is drained, so a launch never holds more CTAs than the class has work for (was: B CTAs, most of them empty).
+// Persistent like k_qpa: one CTA per SM takes scenarios of the class from the device-side queue (a.next) until the list is
+// drained, so a launch never holds more CTAs than the class has work for (was: B CTAs, most of them empty).
 template <int KC>
-__global__ void __launch_bounds__(2 * QpdLayout<KC>::TA, QPD_MINBLOCKS(KC)) k_qpd(const QpArgs a) {
+__global__ void __launch_bounds__(2 * QpdLayout<KC>::TA, 1) k_qpd(const QpArgs a) {
   extern __shared__ __align__(16) double qpd_smem[];
   __shared__ int s_slot;
   for (;;) {
@@ -158,31 +155,9 @@ __global__ void k_broadcast_corridor(int *K, SpectralCube *segs, int *cstatus, i
   for (int k = 0; k < n; k++) segs[(size_t)b * k_max + k] = segs[k];
 }
 
-// k_qpa<8> with the finish deferred (qp_shared.cuh: qpa_handoff): the CTA hands the end state of each scenario to k_qps_finish,
-// which polishes 16 scenarios per SM at a time instead of one warp of a 4-warp CTA while the other three wait.
-__global__ void __launch_bounds__(2 * QpdLayout<8>::TA, 2) k_qpa8_deferred(const QpsArgs A) {
-  extern __shared__ __align__(16) double qpd_smem[];
-  __shared__ int s_slot;
-  const QpArgs &a = A.q;
-  for (;;) {
-    if (threadIdx.x == 0) s_slot = atomicAdd(a.next, 1);
-    __syncthreads();
-    const int slot = s_slot;
-    __syncthreads();
-    if (slot >= *a.count) return;
-    qpa_cta_body<8>(a, slot, threadIdx.x, qpd_smem, []() { __syncthreads(); },
-                    [](int axis) {
-                      if (axis == 0) asm volatile("bar.sync 1, %0;" ::"n"(QpdLayout<8>::TA) : "memory");
-                      else asm volatile("bar.sync 2, %0;" ::"n"(QpdLayout<8>::TA) : "memory");
-                    },
-                    true);
-    qpa_handoff(A, slot, threadIdx.x, blockDim.x, qpd_smem);
-  }
-}
-
 // ------------------------------------------------------------------ shared-KKT path (qp_shared.cuh)
 // structure key of a scenario of the K <= 8 class: (K, the bit patterns of t_k, the weights when they are per scenario)
-// `hint` (may be null): st[4 b + 3] of a first prepare pass run with the interval pre-check forced on = "this corridor is provably
+// `hint`: st[4 b + 3] of a first prepare pass run with the interval pre-check forced on = "this corridor is provably
 // empty".  It is mixed into the key, so that tiles are homogeneous in it: members that converge in a few hundred iterations no
 // longer idle in a tile until an infeasible member has burnt its 5000 (the hint decides tile membership only, never a status).
 __global__ void k_qps_keys(const int *cstatus, const int *K, const SpectralCube *segs, int k_max, const double *weights, int wstride, int B,
@@ -198,7 +173,7 @@ __global__ void k_qps_keys(const int *cstatus, const int *K, const SpectralCube 
     for (int k = 0; k < K[b]; k++) mix((unsigned long long)__double_as_longlong(segs[(size_t)b * k_max + k].t));
     if (wstride)
       for (int i = 0; i < 10; i++) mix((unsigned long long)__double_as_longlong(weights[(size_t)b * 10 + i]));
-    if (hint) mix(hint[4 * b + 3] ? 0x5bd1e995ull : 0x1b873593ull);
+    mix(hint[4 * b + 3] ? 0x5bd1e995ull : 0x1b873593ull);
     if (h == ~0ull) h = 0x1234567ull;
   }
   keys[b] = h; ids[b] = b; leader_tile[b] = -1;
@@ -229,19 +204,6 @@ __global__ void __launch_bounds__(64) k_qps_prepare(const QpsArgs A, const int *
   extern __shared__ double qp_smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   qps_prepare_body(A, leader_tile, blockIdx.x * 2 + warp, lane, qp_smem + (size_t)warp * QP_SM_DOUBLES_PER_LANE * 32);
-}
-__global__ void __launch_bounds__(64) k_qps(const QpsArgs A) {
-  extern __shared__ __align__(16) double qps_smem[];
-  __shared__ int s_tile;
-  for (;;) {
-    if (threadIdx.x == 0) s_tile = atomicAdd(A.tile_next, 1);
-    __syncthreads();
-    const int tile = s_tile;
-    __syncthreads();
-    if (tile >= *A.n_tiles) return;
-    qps_tile_body(A, tile, blockIdx.x, threadIdx.x, qps_smem, []() { __syncthreads(); });
-    __syncthreads();
-  }
 }
 // four warps per tile (qp_shared4.cuh): warp = (axis, half), one segment per thread
 __global__ void __launch_bounds__(128, 2) k_qps4(const QpsArgs A) {
@@ -414,11 +376,6 @@ struct spectral_handle {
   int tk_cap = 0, tk_cap_ranks = 0;
   int classes_timed = 0;    // solver classes launched per call (k_max dependent)
   int corridor_smem = 0;    // dynamic shared memory the corridor kernel is opted in for on this handle's device
-  bool legacy_qpd = false;  // SPECTRAL_LEGACY_QPD=1: the round-1 full-row kernels for K <= 10 (A/B measurements)
-  bool defer_finish = false; // SPECTRAL_DEFER_FINISH=1: K <= 8 class: status / polish / outputs in k_qps_finish instead of in the ADMM CTA
-  bool force_lanes = false; // SPECTRAL_FORCE_LANES=1: k_qp<8|16> (lane per segment, block-tridiagonal solve) for every class
-  bool qps_nohint = false;  // SPECTRAL_QPS_NOHINT=1: shared-KKT tiles keyed by structure only (no feasibility hint in the key)
-  bool legacy_qps = false;  // SPECTRAL_LEGACY_QPS=1: the two-warp shared-KKT tile kernel instead of the four-warp one
 };
 
 static int fail(spectral_handle *h, int code, const std::string &msg) {
@@ -454,11 +411,6 @@ extern "C" int spectral_create(int device, int max_batch, int n_max, int r_max, 
   }
   spectral_handle *h = new spectral_handle();
   h->device = device; h->max_batch = max_batch; h->n_max = n_max; h->r_max = r_max; h->k_max = k_max;
-  { const char *e = getenv("SPECTRAL_LEGACY_QPD"); h->legacy_qpd = e && e[0] == '1'; }
-  { const char *e = getenv("SPECTRAL_LEGACY_QPS"); h->legacy_qps = e && e[0] == '1'; }
-  { const char *e = getenv("SPECTRAL_QPS_NOHINT"); h->qps_nohint = e && e[0] == '1'; }
-  { const char *e = getenv("SPECTRAL_FORCE_LANES"); h->force_lanes = e && e[0] == '1'; }
-  { const char *e = getenv("SPECTRAL_DEFER_FINISH"); h->defer_finish = e && e[0] == '1'; }
   *out = h;
   CK(cudaSetDevice(device));
   cudaDeviceProp prop;
@@ -569,8 +521,7 @@ static cudaError_t launch_qpd(spectral_handle *h, const QpArgs &qa, int B, cudaS
   const size_t smem = QpdLayout<KC>::BYTES;
   cudaError_t e = cudaFuncSetAttribute(k_qpd<KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  const int cap = QPD_MINBLOCKS(KC) * h->sm_count;
-  k_qpd<KC><<<B < cap ? B : cap, 2 * QpdLayout<KC>::TA, smem, st>>>(qa);
+  k_qpd<KC><<<B < h->sm_count ? B : h->sm_count, 2 * QpdLayout<KC>::TA, smem, st>>>(qa);
   h->launches++;
   return cudaGetLastError();
 }
@@ -586,14 +537,6 @@ static cudaError_t launch_qpa(spectral_handle *h, const QpArgs &qa, int B, cudaS
   return cudaGetLastError();
 }
 
-// Shared-KKT path for the K <= 8 class: structure keys -> sort -> tiles of <= 8 scenarios -> prepare -> tile ADMM (DMMA) -> finish
-static int ensure_qps_buffers(spectral_handle *h);
-static int launch_qps_impl(spectral_handle *h, const QpArgs &qa, const int *cstatus, int B, const SpectralInputs *in, cudaStream_t st);
-static int launch_qps(spectral_handle *h, const QpArgs &qa, const int *cstatus, int B, const SpectralInputs *in, cudaStream_t st) {
-  const size_t Bm = (size_t)h->max_batch;
-  { const int rc = ensure_qps_buffers(h); if (rc) return rc; }
-  return launch_qps_impl(h, qa, cstatus, B, in, st);
-}
 static int ensure_qps_buffers(spectral_handle *h) {
   const size_t Bm = (size_t)h->max_batch, km = (size_t)h->k_max;
   if (!h->qs_keys) {
@@ -614,7 +557,9 @@ static int ensure_qps_buffers(spectral_handle *h) {
   }
   return SPECTRAL_SUCCESS;
 }
-static int launch_qps_impl(spectral_handle *h, const QpArgs &qa, const int *cstatus, int B, const SpectralInputs *in, cudaStream_t st) {
+// Shared-KKT path for the K <= 8 class: structure keys -> sort -> tiles of <= 8 scenarios -> prepare -> tile ADMM (DMMA) -> finish
+static int launch_qps(spectral_handle *h, const QpArgs &qa, const int *cstatus, int B, cudaStream_t st) {
+  { const int rc = ensure_qps_buffers(h); if (rc) return rc; }
   const size_t Bm = (size_t)h->max_batch;
   int *head = h->qs_tmp, *gstart = h->qs_tmp + Bm, *flag = h->qs_tmp + 2 * Bm, *tidx = h->qs_tmp + 3 * Bm;
   int *tile_start = h->qs_tile, *tile_count = h->qs_tile + Bm;
@@ -623,19 +568,17 @@ static int launch_qps_impl(spectral_handle *h, const QpArgs &qa, const int *csta
   const size_t sm_pf = 2 * (size_t)QP_SMEM_PER_WARP;
   const int pf_blocks = (B + 3) / 4;  // two scenarios per warp, two warps per block
   CK(cudaFuncSetAttribute(k_qps_prepare, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_pf));
-  if (!h->qps_nohint) {
-    // hint pass: the K3 assembly of every scenario of the class with the interval pre-check forced on, no tile yet (leader = -1)
-    QpsArgs Hh;
-    memset(&Hh, 0, sizeof(Hh));
-    Hh.q = qa; Hh.q.lu = h->qs_lu; Hh.q.opt.precheck = 1;
-    if (!(Hh.q.opt.precheck_margin > 0.0)) Hh.q.opt.precheck_margin = 1e-3;
-    Hh.blk = h->qs_blk; Hh.qv = h->qs_qv; Hh.wrows = h->qs_w; Hh.xout = h->qs_x; Hh.st = h->qs_st;
-    CK(cudaMemsetAsync(h->qs_leader, 0xFF, (size_t)B * 4, st));
-    k_qps_prepare<<<pf_blocks, 64, sm_pf, st>>>(Hh, h->qs_leader);
-    h->launches++;
-  }
+  // hint pass: the K3 assembly of every scenario of the class with the interval pre-check forced on, no tile yet (leader = -1)
+  QpsArgs Hh;
+  memset(&Hh, 0, sizeof(Hh));
+  Hh.q = qa; Hh.q.lu = h->qs_lu; Hh.q.opt.precheck = 1;
+  if (!(Hh.q.opt.precheck_margin > 0.0)) Hh.q.opt.precheck_margin = 1e-3;
+  Hh.blk = h->qs_blk; Hh.qv = h->qs_qv; Hh.wrows = h->qs_w; Hh.xout = h->qs_x; Hh.st = h->qs_st;
+  CK(cudaMemsetAsync(h->qs_leader, 0xFF, (size_t)B * 4, st));
+  k_qps_prepare<<<pf_blocks, 64, sm_pf, st>>>(Hh, h->qs_leader);
+  h->launches++;
   k_qps_keys<<<nb, 256, 0, st>>>(cstatus, qa.K, qa.segs, h->k_max, qa.weights, qa.wstride, B, h->qs_keys, h->qs_ids, h->qs_leader,
-                                h->qps_nohint ? nullptr : h->qs_st);
+                                h->qs_st);
   size_t tb = h->qs_cub_bytes;
   CK(cub::DeviceRadixSort::SortPairs(h->qs_cub, tb, h->qs_keys, h->qs_keys2, h->qs_ids, h->qs_ids2, B, 0, 64, st));
   k_qps_heads<<<nb, 256, 0, st>>>(h->qs_keys2, B, head);
@@ -651,40 +594,13 @@ static int launch_qps_impl(spectral_handle *h, const QpArgs &qa, const int *csta
   A.fs_scratch = h->qs_fs;
   A.blk = h->qs_blk; A.qv = h->qs_qv; A.wrows = h->qs_w; A.xout = h->qs_x; A.st = h->qs_st;
   CK(cudaFuncSetAttribute(k_qps_finish, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_pf));
-  CK(cudaFuncSetAttribute(k_qps, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QpsSmem::BYTES));
+  CK(cudaFuncSetAttribute(k_qps4, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Qps4Smem::BYTES));
   k_qps_prepare<<<pf_blocks, 64, sm_pf, st>>>(A, h->qs_leader);
-  const int tiles_max = B;
-  if (h->legacy_qps) {   // SPECTRAL_LEGACY_QPS=1: the two-warp tile layout (A/B measurements)
-    const int per_sm = 2 * (QpsSmem::BYTES + 1024 + 16) <= 227 * 1024 ? 2 : 1;
-    const int grid = tiles_max < per_sm * h->sm_count ? tiles_max : per_sm * h->sm_count;
-    k_qps<<<grid, 64, QpsSmem::BYTES, st>>>(A);
-  } else {
-    CK(cudaFuncSetAttribute(k_qps4, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Qps4Smem::BYTES));
-    const int per_sm = 2 * (Qps4Smem::BYTES + 1024 + 16) <= 227 * 1024 ? 2 : 1;
-    const int grid = tiles_max < per_sm * h->sm_count ? tiles_max : per_sm * h->sm_count;
-    k_qps4<<<grid, 128, Qps4Smem::BYTES, st>>>(A);
-  }
+  const int per_sm = 2 * (Qps4Smem::BYTES + 1024 + 16) <= 227 * 1024 ? 2 : 1;
+  const int grid = B < per_sm * h->sm_count ? B : per_sm * h->sm_count;
+  k_qps4<<<grid, 128, Qps4Smem::BYTES, st>>>(A);
   k_qps_finish<<<pf_blocks, 64, sm_pf, st>>>(A);
   h->launches += 8;
-  CK(cudaGetLastError());
-  return SPECTRAL_SUCCESS;
-}
-
-// K <= 8 class on the anchor kernel with the finish deferred to k_qps_finish (each scenario its own tile)
-static int launch_qpa8_deferred(spectral_handle *h, const QpArgs &qa, int B, cudaStream_t st) {
-  { const int rc = ensure_qps_buffers(h); if (rc) return rc; }
-  QpsArgs A;
-  memset(&A, 0, sizeof(A));
-  A.q = qa; A.q.lu = h->qs_lu;
-  A.blk = h->qs_blk; A.qv = h->qs_qv; A.wrows = h->qs_w; A.xout = h->qs_x; A.st = h->qs_st;
-  const size_t smem = QpdLayout<8>::BYTES;
-  CK(cudaFuncSetAttribute(k_qpa8_deferred, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const int grid = B < 2 * h->sm_count ? B : 2 * h->sm_count;
-  k_qpa8_deferred<<<grid, 2 * QpdLayout<8>::TA, smem, st>>>(A);
-  const size_t sm_pf = 2 * (size_t)QP_SMEM_PER_WARP;
-  CK(cudaFuncSetAttribute(k_qps_finish, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_pf));
-  k_qps_finish<<<(B + 3) / 4, 64, sm_pf, st>>>(A);
-  h->launches += 2;
   CK(cudaGetLastError());
   return SPECTRAL_SUCCESS;
 }
@@ -783,14 +699,9 @@ static int solve_device_impl(spectral_handle_t *h, int variant, int B, int N, in
     qa.list = h->lists + (size_t)cls * B; qa.count = h->counts + cls; qa.next = h->counts + SP_NUM_CLASSES + cls;
     cudaEvent_t *ec = h->ev_cls[h->timed_calls % spectral_handle::kTimingSlots][cls];
     if (tm) CK(cudaEventRecord(ec[0], cs));
-    if (h->force_lanes && cls < 4) {   // SPECTRAL_FORCE_LANES=1: lane-per-segment kernels for every class (A/B measurements)
-      if (cls == 0) CK((launch_qp<8, 2>(h, qa, B, cs)));
-      else CK((launch_qp<16, 2>(h, qa, B, cs)));
-    }
-    else if (cls == 0 && opt.shared_kkt) { const int rc = launch_qps(h, qa, h->cstatus, B, in, cs); if (rc) return rc; }
-    else if (cls == 0 && h->defer_finish && !h->legacy_qpd && out->lu == nullptr) { const int rc = launch_qpa8_deferred(h, qa, B, cs); if (rc) return rc; }
-    else if (cls == 0) CK((h->legacy_qpd ? launch_qpd<8>(h, qa, B, cs) : launch_qpa<8>(h, qa, B, cs)));
-    else if (cls == 1) CK((h->legacy_qpd ? launch_qpd<10>(h, qa, B, cs) : launch_qpa<10>(h, qa, B, cs)));
+    if (cls == 0 && opt.shared_kkt) { const int rc = launch_qps(h, qa, h->cstatus, B, cs); if (rc) return rc; }
+    else if (cls == 0) CK((launch_qpa<8>(h, qa, B, cs)));
+    else if (cls == 1) CK((launch_qpa<10>(h, qa, B, cs)));
     else if (cls == 2) CK((launch_qpd<12>(h, qa, B, cs)));
     else if (cls == 3) CK((launch_qpd<16>(h, qa, B, cs)));
     else CK((launch_qp<32, 2>(h, qa, B, cs)));

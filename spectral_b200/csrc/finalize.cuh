@@ -23,7 +23,7 @@ struct FinalArgs {
 };
 
 // solver class of a scenario by segment count:
-//   0: K <= 8  k_qpd<8>   1: K <= 10  k_qpd<10>   2: K <= 12  k_qpd<12>   3: K <= 16  k_qpd<16>   (dense kernels)
+//   0: K <= 8  k_qpa<8>   1: K <= 10  k_qpa<10>   2: K <= 12  k_qpd<12>   3: K <= 16  k_qpd<16>   (dense kernels)
 //   4: K <= 32  lane-per-segment k_qp<32>
 #define SP_NUM_CLASSES 5
 SP_DEV int lane_class(int K) { return K <= 8 ? 0 : (K <= 10 ? 1 : (K <= 12 ? 2 : (K <= 16 ? 3 : 4))); }

@@ -756,9 +756,6 @@ SP_DEV void qp_setup(const QpArgs &a, int ap, bool have, int seg, int lane, doub
 // (v = rho (2 clip(w') - w')) come from the same loads.  Same arithmetic per quantity as the general iteration of
 // qp_admm_lanes below (which handles iteration 1, the check iterations and the rho updates), so the two can be interleaved.
 // Rows are staged in groups of CH (loads, arithmetic, stores) to bound the live registers next to the factor.
-#ifndef QP_FAST_BLOCK
-#define QP_FAST_BLOCK 1
-#endif
 SP_DEV double qp_ld(const double *p) {
 #ifdef SPECTRAL_CPU_EMU
   return *p;
@@ -857,7 +854,6 @@ SP_DEV void qp_admm_lanes(const SpOptionsDev &o, double *sm, int lane, QpLane &Q
     if (sp_all(state != QP_RUNNING)) break;
     const bool run = state == QP_RUNNING;
     const bool check = (o.check_every > 0) && (it % o.check_every == 0);
-#if QP_FAST_BLOCK
     if (it > 1 && !check) {
       // the iterations up to (not including) the next check, or to max_iter: the state cannot change inside the block
       int it_end = o.max_iter + 1;
@@ -870,7 +866,6 @@ SP_DEV void qp_admm_lanes(const SpOptionsDev &o, double *sm, int lane, QpLane &Q
       it = it_end - 1;
       continue;
     }
-#endif
     double v[QP_ROWS];
     // v = rho (2 clip(w) - w)  (= rho z - y); first iteration: z = y = 0 exactly as OSQP's cold start
 #pragma unroll

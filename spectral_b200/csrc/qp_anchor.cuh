@@ -25,16 +25,8 @@
 #include "qp_dense.cuh"
 
 #define QPA_SPW 5  // segments per warp
-// tuning switches (measured on B200, profiles/r2_qpa_variants.md)
-#ifndef QPA_GRP
-#define QPA_GRP(N) (((N) % 24 == 0) ? 24 : (((N) % 20 == 0) ? 20 : 12))  // doubles of g in flight per group in S3
-#endif
-#ifndef QPA_WRAP_SHFL
-#define QPA_WRAP_SHFL 0   // 1: neighbour shuffles with wrap-around instead of shfl.up + boundary masks (measured: 86.7 k vs 87.2 k solves/s, not taken)
-#endif
-#ifndef QPA_FENCE
-#define QPA_FENCE 0   // scheduling fences between the load runs and the arithmetic (measured: 81.5 k solves/s with, 82.6 k without)
-#endif
+// doubles of g in flight per group in S3
+SP_HD constexpr int qpa_grp(int N) { return (N % 24 == 0) ? 24 : ((N % 20 == 0) ? 20 : 12); }
 
 template <int N>
 struct QpaIO {
@@ -65,16 +57,6 @@ SP_DEV void qpa_map(int ta, int &seg, int &i, bool &isvar) {
 // Arithmetic ordered as qpd_block1's S2.
 template <bool CHECK_ORDER>
 SP_DEV double qpa_gather(const double vv[5], int lane, int jsrc, double tkv, double f0, double f1, double f2, double rest) {
-#if QPA_WRAP_SHFL
-  // Neighbours by index shuffle with wrap-around: lanes 0..2 read lanes 29..31, which hold no live velocity / acceleration /
-  // jerk row (lanes 30, 31 are idle, lane 29 is control point 5 of its segment: its jerk slot does not exist), i.e. rho = 0
-  // and value 0 -- like the neighbour across any segment boundary.  No boundary masks needed.
-  const int l1 = (lane + 31) & 31, l2 = (lane + 30) & 31, l3 = (lane + 29) & 31;
-  const double g1a = sp_shfl(vv[1], l1);
-  const double g2b = sp_shfl(vv[2], l1), g2a = sp_shfl(vv[2], l2);
-  const double g3c = sp_shfl(vv[3], l1), g3b = sp_shfl(vv[3], l2), g3a = sp_shfl(vv[3], l3);
-  const double c0 = sp_shfl(vv[4], jsrc), c1 = sp_shfl(vv[4], jsrc + 1), c2 = sp_shfl(vv[4], jsrc + 2);
-#else
   const double u11 = sp_shfl_up(vv[1], 1, 32);
   const double u21 = sp_shfl_up(vv[2], 1, 32), u22 = sp_shfl_up(vv[2], 2, 32);
   const double u31 = sp_shfl_up(vv[3], 1, 32), u32 = sp_shfl_up(vv[3], 2, 32), u33 = sp_shfl_up(vv[3], 3, 32);
@@ -84,7 +66,6 @@ SP_DEV double qpa_gather(const double vv[5], int lane, int jsrc, double tkv, dou
   const double g1a = lane >= 1 ? u11 : 0.0;
   const double g2b = lane >= 1 ? u21 : 0.0, g2a = lane >= 2 ? u22 : 0.0;
   const double g3c = lane >= 1 ? u31 : 0.0, g3b = lane >= 2 ? u32 : 0.0, g3a = lane >= 3 ? u33 : 0.0;
-#endif
   if (CHECK_ORDER) {  // summation order of qpd_gather (the termination check's A' y and A' delta y)
     double g = tkv * vv[0];
     g += 5.0 * (g1a - vv[1]);
@@ -100,16 +81,13 @@ SP_DEV double qpa_gather(const double vv[5], int lane, int jsrc, double tkv, dou
   return (t01 + t2) + (t3 + tc);
 }
 
-// A block of n ADMM iterations (out of line: only the hot state is live).
-#ifndef QPA_AXIS_TMPL
-#define QPA_AXIS_TMPL 1  // 1: the axis is a template parameter of the block (barrier ids become immediates without predication)
-#endif
+// A block of n ADMM iterations (out of line: only the hot state is live).  The axis AX is a template parameter, so that the
+// barrier ids become immediates without predication.
 template <int KC, int AX, typename SyncAxisFn>
-SP_DEV_NOINLINE void qpa_block(QpaIO<6 * KC> &io, double *smx, int ta, int axis_rt, int n, double alpha, SyncAxisFn sync_axis_fn) {
-  const int axis = AX >= 0 ? AX : axis_rt;
+SP_DEV_NOINLINE void qpa_block(QpaIO<6 * KC> &io, double *smx, int ta, int n, double alpha, SyncAxisFn sync_axis_fn) {
   using L = QpdLayout<KC>;
   constexpr int N = L::N;
-  constexpr int GRP = QPA_GRP(N);
+  constexpr int GRP = qpa_grp(N);
   static_assert(N % GRP == 0 && GRP % 4 == 0, "g in whole groups");
   int seg, i;
   bool isvar;
@@ -144,7 +122,7 @@ SP_DEV_NOINLINE void qpa_block(QpaIO<6 * KC> &io, double *smx, int ta, int axis_
       const double g = qpa_gather<false>(vv, lane, jsrc, tkv, f0, f1, f2, sigv * xv - qv);
       if (isvar) *gvp = g;
     }
-    sync_axis_fn(axis);
+    sync_axis_fn(AX);
     double xt;
     {  // S3
       double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
@@ -153,7 +131,6 @@ SP_DEV_NOINLINE void qpa_block(QpaIO<6 * KC> &io, double *smx, int ta, int axis_
         double gl[GRP];
 #pragma unroll
         for (int e = 0; e < GRP; e += 2) qpd_lds2(gv + g0 + e, gl[e], gl[e + 1]);
-        qpd_sched_fence_if<QPA_FENCE>();
 #pragma unroll
         for (int e = 0; e < GRP; e += 4) {
           a0 += G[g0 + e] * gl[e]; a1 += G[g0 + e + 1] * gl[e + 1]; a2 += G[g0 + e + 2] * gl[e + 2]; a3 += G[g0 + e + 3] * gl[e + 3];
@@ -165,11 +142,10 @@ SP_DEV_NOINLINE void qpa_block(QpaIO<6 * KC> &io, double *smx, int ta, int axis_
         *cxp = xt;
       }
     }
-    sync_axis_fn(axis);
+    sync_axis_fn(AX);
     {  // S1
       const double c1 = cxp[1], c2 = cxp[2], c3 = cxp[3];
       const double j0 = cpj[0], j1 = cpj[1], j2 = cpj[2], j3 = cpj[3], j4 = cpj[4], j5 = cpj[5];
-      qpd_sched_fence_if<QPA_FENCE>();
       const double c0 = xt;
       const double d1 = c1 - c0, e1 = c2 - c1, f1_ = c3 - c2;
       const double d2 = e1 - d1, e2 = f1_ - e1;
@@ -327,10 +303,8 @@ SP_DEV_NOINLINE int qpa_check(const QpArgs &a, int slot, int tid, double *smem, 
 
 // slot: index of the scenario in this class' list.  tid in [0, 2 TA).  smem: QpdLayout<KC>::BYTES, 16-byte aligned.
 // sync_axis(axis) synchronises the TA threads of one axis.
-// defer: leave the final status / polish / outputs (qpd_control_finish) to a later kernel: the scalars it needs are published
-// in red[0..3] = (c_scale, rhobar, state, iterations), everything else already sits in the control slots of shared memory.
 template <int KC, typename SyncFn, typename SyncAxisFn>
-SP_DEV void qpa_cta_body(const QpArgs &a, int slot, int tid, double *smem, SyncFn sync_cta, SyncAxisFn sync_axis_fn, bool defer = false) {
+SP_DEV void qpa_cta_body(const QpArgs &a, int slot, int tid, double *smem, SyncFn sync_cta, SyncAxisFn sync_axis_fn) {
   using L = QpdLayout<KC>;
   static_assert(L::ROWFULL && L::TA == 32 * ((KC + QPA_SPW - 1) / QPA_SPW), "anchor layout: five segments per warp, whole rows of G");
   constexpr int N = L::N, LPA = L::LPA, STR = L::STR, TA = L::TA;
@@ -413,12 +387,8 @@ SP_DEV void qpa_cta_body(const QpArgs &a, int slot, int tid, double *smem, SyncF
       it_end = nxt < it_end ? nxt : it_end;
     }
     const bool check = (o.check_every > 0) && (it_end % o.check_every == 0);
-#if QPA_AXIS_TMPL
-    if (axis == 0) qpa_block<KC, 0>(io, smx, ta, 0, it_end - it + 1, o.alpha, sync_axis_fn);
-    else qpa_block<KC, 1>(io, smx, ta, 1, it_end - it + 1, o.alpha, sync_axis_fn);
-#else
-    qpa_block<KC, -1>(io, smx, ta, axis, it_end - it + 1, o.alpha, sync_axis_fn);
-#endif
+    if (axis == 0) qpa_block<KC, 0>(io, smx, ta, it_end - it + 1, o.alpha, sync_axis_fn);
+    else qpa_block<KC, 1>(io, smx, ta, it_end - it + 1, o.alpha, sync_axis_fn);
     iters = it_end;
     it = it_end + 1;
     if (!check) continue;
@@ -442,11 +412,6 @@ SP_DEV void qpa_cta_body(const QpArgs &a, int slot, int tid, double *smem, SyncF
       ctlw[QP_SM_RHO * STR + ooff] = io.rho[s];
     }
     if (isvar) smx[L::O_XR + QPD_CP + v] = io.xv;
-  }
-  if (defer) {
-    if (tid == 0) { red[0] = c_scale; red[1] = rhobar; red[2] = (double)state; red[3] = (double)iters; }
-    sync_cta();
-    return;
   }
   sync_cta();
   if (warp != 0) return;

@@ -2,7 +2,8 @@
 //
 // Replaces the iteration that the reference delegates to OSQP (osqp_solve, called at solve_3d.cc:1249 |
 // cuboid_3d.cc:1108 with the settings of solve_3d.cc:1235-1243,1446-1462) for scenarios with at most
-// KC <= 16 Bezier segments (instantiated for KC = 8, 10, 12, 16).  One CTA = one scenario = both axis problems (s and l), solved as ONE OSQP
+// KC <= 16 Bezier segments (k_qpd is instantiated for KC = 12, 16; the KC <= 10 classes run the anchor layout of qp_anchor.cuh,
+// which shares this file's setup, layout and check code).  One CTA = one scenario = both axis problems (s and l), solved as ONE OSQP
 // instance like the reference does: one cost scaling c, one rho, joint termination and infeasibility norms.
 //
 // Why this form.  The lane-per-segment loop of qp.cuh (block-tridiagonal Cholesky, one lane per segment)
@@ -19,9 +20,11 @@
 //   KC = 12       row pairs (below): 2 chunks per row of G, 160 threads per axis, 168 registers, staged loads  qpd_block
 //   KC = 8, 10    full rows: one thread per variable holds its whole row of G, 64 threads per axis, 255
 //                 registers, four generic row slots per thread                                              qpd_block1
+//                 (replaced by the anchor layout of qp_anchor.cuh; kept as its bit-exact reference in the emulator tests)
 //   KC = 16       quarter rows: 4 chunks per row, one constraint row per thread, 384 threads per axis        qpd_block4
 //                 (KC = 12 ran this layout at 7.7 ms; as staged row pairs, one CTA per SM at 320 threads: 6.4 ms)
-// (QPD_VMAJOR / qpd_block5 is a fourth, measured slower and kept off.)
+// (A v-major layout, chunk index uniform per warp and partial sums through shared memory, measured slower for K <= 8: 14.6
+// against 11.6 ms, profiles/r1_qpd_staging.md.)
 //
 // Thread map of the row-pair layout (per axis TA = 2n threads rounded up to whole warps: 96 for KC = 8; CTA = 2 TA):
 //   thread (v, h) = ta >> 1, ta & 1 : half row h of G (n/2 doubles in registers); the h = 0 thread also owns the
@@ -52,40 +55,28 @@
 #define QPD_LS 24         // doubles of lane state per segment: t, tp, tn, q[6], sig[6], cD[6]
 #define QPD_NRED 10
 
-// Chunks per row of G (= threads per variable).  Measured on B200 (profiles/r1_qpd_nch.md): 2 chunks beat 4 for the
-// common K <= 8 class -- with 4, the warps run the variable gather with a quarter of their lanes and the total
-// instruction / shared-memory wavefront count per iteration rises 59 % / 69 %.  4 chunks (a quarter row of G and at
-// most one constraint row per thread) are kept where 2 would not fit the register file (KC >= 12).
-// V-major layout (QPD_VMAJOR): 4 chunks per row of G with the chunk index h UNIFORM PER WARP (thread t = h N + v), so
-// that the broadcast load of the g chunk costs one shared-memory wavefront per LDS.128 instead of one per distinct
-// address (with the chunk lanes adjacent: 4); the four partial sums of a variable meet in shared memory (one more
-// barrier), the gather and the partial-sum reduction run on the h = 0 warps only, every thread owns one constraint row.
-// Measured on B200 for K <= 8 (profiles/r1_qpd_staging.md): 14.6 ms against 11.6 ms of the row-pair layout -- 29 % more
-// instructions, a fourth barrier over 12 warps and no room for staged loads at 80 registers outweigh the cheaper
-// broadcast.  Kept behind the switch (off) as the measured alternative.
-#ifndef QPD_VMAJOR
-#define QPD_VMAJOR(KC) 0
-#endif
-// Full-row layout (QPD_ROWFULL): ONE thread per variable holds its whole row of G (n doubles) -- 64 threads per axis,
-// 128 per CTA, up to 255 registers, still two CTAs per SM.  No chunk reduction (no shuffles), the g vector is read with
-// every lane on the same address (one wavefront per LDS.128), the gather runs on all variable lanes, and every thread
-// carries ceil(21 KC / 64) constraint rows whose loads and updates interleave (ILP instead of TLP: the kernel is
-// latency-bound and every wider layout tried lost to its extra barriers and instructions, profiles/r1_qpd_staging.md).
-// Measured (profiles/r1_qpd_staging.md): K <= 10: 9.95 ms (row pairs at 128 registers) -> 7.85 ms; K <= 8: 10.0 ms against 10.6 ms
-// of the staged row-pair layout at 168 registers (same box), once g is staged in groups of 24 doubles.
-#ifndef QPD_ROWFULL
-#define QPD_ROWFULL(KC) ((KC) <= 10)
-#endif
-#ifndef QPD_NCH
-#define QPD_NCH(KC) (QPD_ROWFULL(KC) ? 1 : (((KC) >= 16 || QPD_VMAJOR(KC)) ? 4 : 2))
-#endif
-SP_HD constexpr int qpd_nch(int KC) { return QPD_NCH(KC); }
-
 template <int KC>
 struct QpdLayout {
-  static constexpr int NCH = qpd_nch(KC);      // threads per variable (chunks per row of G)
-  static constexpr bool VMAJOR = QPD_VMAJOR(KC); // thread t = h N + v (chunk index uniform per warp) instead of t = v NCH + h
-  static constexpr bool ROWFULL = QPD_ROWFULL(KC); // thread t = variable t, whole row of G, NSLOT generic row slots
+  // Full-row layout: ONE thread per variable holds its whole row of G (n doubles) -- 64 threads per axis, 128 per CTA, up to
+  // 255 registers, still two CTAs per SM.  No chunk reduction (no shuffles), the g vector is read with every lane on the same
+  // address (one wavefront per LDS.128), the gather runs on all variable lanes, and every thread carries ceil(21 KC / 64)
+  // constraint rows whose loads and updates interleave (ILP instead of TLP: the kernel is latency-bound and every wider layout
+  // tried lost to its extra barriers and instructions, profiles/r1_qpd_staging.md).
+  // Measured (profiles/r1_qpd_staging.md): K <= 10: 9.95 ms (row pairs at 128 registers) -> 7.85 ms; K <= 8: 10.0 ms against
+  // 10.6 ms of the staged row-pair layout at 168 registers (same box), once g is staged in groups of 24 doubles.
+  static constexpr bool ROWFULL = KC <= 10;    // thread t = variable t, whole row of G, NSLOT generic row slots
+  // Chunks per row of G (= threads per variable).  Measured on B200 (profiles/r1_qpd_nch.md): 2 chunks beat 4 for the
+  // common K <= 8 class -- with 4, the warps run the variable gather with a quarter of their lanes and the total
+  // instruction / shared-memory wavefront count per iteration rises 59 % / 69 %.  4 chunks (a quarter row of G and at
+  // most one constraint row per thread) are kept where 2 would not fit the register file (KC >= 12).
+  static constexpr int NCH = ROWFULL ? 1 : (KC >= 16 ? 4 : 2);  // threads per variable (chunks per row of G)
+  // Staged loads (a run of loads, a fence, then the arithmetic) need temporaries for everything in flight: they pay where
+  // the register budget has room (KC <= 8: 168 registers, measured 14.9 -> 12.5 ms) and spill where it has not (KC = 10 at
+  // 128 registers: 9.5 -> 12.2 ms, in groups of 10 doubles: 9.65 -> 10.2 ms; KC >= 12 at 96 / 80: 8.0 -> 8.9 ms) --
+  // profiles/r1_qpd_staging.md.
+  static constexpr bool STAGE = KC <= 8 || KC == 12;       // S3: the whole g chunk in flight (CH doubles of temporaries)
+  static constexpr bool LU_REG = KC <= 8 || KC == 12;      // (l, u) of the row slots in registers instead of one LDS.128 per slot and iteration
+  static constexpr bool STAGE_ROWS = KC <= 8 || KC == 12;  // S2 / S1: 13 - 18 doubles of temporaries (KC = 10 at 128 registers: 9.5 -> 10.6 ms)
   static_assert(KC % NCH == 0, "the chunks of a row of G split the segments evenly");
   static constexpr int N = 6 * KC;             // variables per axis
   static constexpr int CH = N / NCH;           // columns of G per thread
@@ -101,7 +92,7 @@ struct QpdLayout {
   static constexpr bool TWO_SLOTS = NCH == 2;
   static constexpr int T0 = TWO_SLOTS ? ((NJ + 31) / 32) * 32 : 0;
   static constexpr int TN = TA - T0;
-  // row slots per thread.  Legacy layouts: 3 (difference rows A, B and one continuity row J).  Full-row layout: NDS slots of
+  // row slots per thread.  Chunked layouts (NCH = 2, 4): 3 (difference rows A, B and one continuity row J).  Full-row layout: NDS slots of
   // difference rows and NJS slots of continuity / init rows, so that every slot is one kind of row on all threads.
   static constexpr int NDS = (NN + TA - 1) / TA;   // full-row layout: slots of difference rows (slot s = row s TA + t) ...
   static constexpr int NJS = (NJ + TA - 1) / TA;   // ... followed by slots of continuity / initial-state rows
@@ -120,8 +111,7 @@ struct QpdLayout {
   static constexpr int O_CE = O_XR + N + 8;                          // continuity row coefficients [3KC][6]
   static constexpr int O_VCF = O_CE + 18 * KC;                       // continuity gather coefficients [N][3]
   static constexpr int O_LU = ((O_VCF + 3 * N + 1) / 2) * 2;         // (l, u) of the row slots [NSLOT][TA] pairs (16-byte aligned)
-  static constexpr int O_PS = O_LU + 2 * NSLOT * TA;                 // v-major layout: partial sums of x~ [NCH][N]
-  static constexpr int O_V2 = O_PS + (VMAJOR ? ((NCH * N + 1) / 2) * 2 : 0);  // second row-value array (checks: y next to delta y)
+  static constexpr int O_V2 = O_LU + 2 * NSLOT * TA;                 // second row-value array (checks: y next to delta y)
   static constexpr int AXIS = O_V2 + ((QPD_VB * (KC + 1) + 1) / 2) * 2;       // doubles per axis (even)
   // per-CTA tail: reduction scratch [NWARPS][QPD_NRED], eqmask ints [2][LPA]
   static constexpr int O_RED = 2 * AXIS;
@@ -144,21 +134,6 @@ SP_DEV void qpd_lds2(const double *p, double &a, double &b) {
   asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(a), "=d"(b) : "r"((unsigned)__cvta_generic_to_shared(p)));
 #endif
 }
-// Staged loads (a run of loads, a fence, then the arithmetic) need temporaries for everything in flight: they pay where
-// the register budget has room (KC <= 8: 168 registers, measured 14.9 -> 12.5 ms) and spill where it has not (KC = 10 at
-// 128 registers: 9.5 -> 12.2 ms; KC >= 12 at 96 / 80: 8.0 -> 8.9 ms) -- profiles/r1_qpd_staging.md.
-#ifndef QPD_STAGE
-#define QPD_STAGE(KC) ((KC) <= 8 || (KC) == 12)      // S3: the whole g chunk in flight (CH doubles of temporaries)
-#endif
-#ifndef QPD_STAGE_GROUP
-#define QPD_STAGE_GROUP(KC) 0  // S3 in groups of this many doubles where the whole chunk does not fit (0: unstaged; KC = 10 in groups of 10: 9.65 -> 10.2 ms)
-#endif
-#ifndef QPD_LU_REG
-#define QPD_LU_REG(KC) ((KC) <= 8 || (KC) == 12)   // (l, u) of the row slots in registers instead of one LDS.128 per slot and iteration
-#endif
-#ifndef QPD_STAGE_ROWS
-#define QPD_STAGE_ROWS(KC) ((KC) <= 8 || (KC) == 12)   // S2 / S1: 13 - 18 doubles of temporaries (KC = 10 at 128 registers: 9.5 -> 10.6 ms)
-#endif
 template <bool ON>
 SP_DEV void qpd_sched_fence_if() {
 #ifndef SPECTRAL_CPU_EMU
@@ -274,50 +249,7 @@ SP_DEV void qpd_inverse_chunk(const double *fs, int v, int h, double *g) {
 // thread -> (variable v, chunk h) of the G layout; threads beyond NCH N hold nothing (v = N)
 template <int KC>
 SP_DEV void qpd_map(int ta, int &v, int &h) {
-  using L = QpdLayout<KC>;
-  if (L::VMAJOR) { h = ta / L::N; v = ta - h * L::N; if (h >= L::NCH) { h = 0; v = L::N; } }
-  else { v = ta / L::NCH; h = ta % L::NCH; }
-}
-
-// V-major layout: chunk h of row v of G = S^-1 by ONE thread (the chunk lanes are not adjacent, so there is no carry to
-// hand over): the whole block forward / backward substitution on e_v with the intermediate vector in local memory,
-// keeping the KC / NCH segments of the chunk.  Runs at setup and after adaptive-rho updates only.
-template <int KC>
-SP_DEV void qpd_inverse_row_chunk(const double *fs, int v, int h, double *g) {
-  constexpr int KB = QpdLayout<KC>::KB, N = QpdLayout<KC>::N;
-  const int kv = v / 6, iv = v - 6 * kv;
-  const int kbase = h * KB;
-  double Y[N];
-  double c3 = 0.0, c4 = 0.0, c5 = 0.0;  // y_{k-1}[3..5]
-  for (int k = 0; k < KC; k++) {
-    const double *F = fs + 57 * k;
-#pragma unroll
-    for (int a = 0; a < 6; a++) {
-      double y = 0.0;
-      if (k == kv && a >= iv) y = F[LT(a, 0) + iv];
-      y -= F[21 + a * 3 + 0] * c3 + F[21 + a * 3 + 1] * c4 + F[21 + a * 3 + 2] * c5;  // C_0 = 0
-      Y[6 * k + a] = y;
-    }
-    c3 = Y[6 * k + 3]; c4 = Y[6 * k + 4]; c5 = Y[6 * k + 5];
-  }
-  double n0 = 0.0, n1 = 0.0, n2 = 0.0;  // x_{k+1}[0..2]
-  for (int k = KC - 1; k >= kbase; k--) {
-    const double *F = fs + 57 * k;
-    double x[6];
-#pragma unroll
-    for (int i = 0; i < 6; i++) {
-      double xx = 0.0;
-#pragma unroll
-      for (int a = i; a < 6; a++) xx += F[LT(a, i)] * Y[6 * k + a];
-      xx -= F[39 + i * 3 + 0] * n0 + F[39 + i * 3 + 1] * n1 + F[39 + i * 3 + 2] * n2;  // E of the last segment = 0
-      x[i] = xx;
-    }
-    n0 = x[0]; n1 = x[1]; n2 = x[2];
-    if (k < kbase + KB) {
-#pragma unroll
-      for (int i = 0; i < 6; i++) g[6 * (k - kbase) + i] = x[i];
-    }
-  }
+  v = ta / QpdLayout<KC>::NCH; h = ta % QpdLayout<KC>::NCH;
 }
 
 // CTA-wide reduction of QPD_NRED values: slots 0..8 max (of non-negative norms), slot 9 sum.  All threads return the
@@ -485,13 +417,7 @@ SP_DEV void qpd_decode_diff(int e, int &order, int &k, int &i) {
 template <int KC>
 SP_DEV_NOINLINE void qpd_build_g(const double *fs, int v, int h, bool isg, double *out) {
   double g[QpdLayout<KC>::CH];
-  if constexpr (QpdLayout<KC>::VMAJOR) {
-#pragma unroll
-    for (int e = 0; e < QpdLayout<KC>::CH; e++) g[e] = 0.0;
-    if (isg) qpd_inverse_row_chunk<KC>(fs, v, h, g);
-  } else {
-    qpd_inverse_chunk<KC>(fs, v, h, g);
-  }
+  qpd_inverse_chunk<KC>(fs, v, h, g);
 #pragma unroll
   for (int e = 0; e < QpdLayout<KC>::CH; e++) out[e] = isg ? g[e] : 0.0;
 }
@@ -611,7 +537,7 @@ SP_DEV double qpd_row_update(QpdRow &r, const QpdLU &b, double zt, double alpha)
 template <int CHN, int NS = 3>
 struct QpdIOT {
   double G[CHN];    // this thread's chunk of its row of G = S^-1
-  QpdRow rows[NS];  // row slots (legacy layouts: difference rows A, B and continuity row J); unused ones have meta bit 3 clear
+  QpdRow rows[NS];  // row slots (chunked layouts: difference rows A, B and continuity row J); unused ones have meta bit 3 clear
   double yo[NS];    // multipliers before the check iteration's update
   double xv, sigv, qv, tkv;  // variable thread: relaxed iterate, sigma, q, segment duration
   double c_scale, rhobar;
@@ -655,7 +581,7 @@ SP_DEV_NOINLINE void qpd_block(QpdIOT<QpdLayout<KC>::CH, QpdLayout<KC>::NSLOT> &
 #pragma unroll
   for (int e = 0; e < CH; e++) G[e] = io.G[e];
   // where the register budget allows, the (l, u) pairs of both slots stay in registers for the whole block
-  constexpr bool LU_REG = QPD_LU_REG(KC);
+  constexpr bool LU_REG = L::LU_REG;
   const QpdLU la_r = lua[0], l2_r = lu2[0];
   double yoa = 0.0, yo2 = 0.0;
   for (int i = 0; i < n; i++) {
@@ -666,7 +592,7 @@ SP_DEV_NOINLINE void qpd_block(QpdIOT<QpdLayout<KC>::CH, QpdLayout<KC>::NSLOT> &
       const double g3a = vb[QPD_V3 + vj - 3], g3b = vb[QPD_V3 + vj - 2], g3c = vb[QPD_V3 + vj - 1], g3d = vb[QPD_V3 + vj];
       const double c0 = vkk[QPD_VC], c1 = vkk[QPD_VC + 1], c2 = vkk[QPD_VC + 2];
       const double f0 = vcf[0], f1 = vcf[1], f2 = vcf[2];  // (hoisting these into registers too costs more than it saves: 10.5 -> 11.4 ms)
-      qpd_sched_fence_if<QPD_STAGE_ROWS(KC)>();
+      qpd_sched_fence_if<L::STAGE_ROWS>();
       double g = tkv * g0;
       g += 5.0 * (g1a - g1b);
       g += 20.0 * ((g2a - g2b) - (g2b - g2c));
@@ -677,25 +603,16 @@ SP_DEV_NOINLINE void qpd_block(QpdIOT<QpdLayout<KC>::CH, QpdLayout<KC>::NSLOT> &
     sync_cta();
     {
       double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
-      static_assert(CH % 2 == 0, "g chunks are loaded in 16-byte pairs");
-      // the g chunk in groups of GRP doubles: a run of loads, a scheduling fence, the FMAs (ptxas otherwise consumes each
-      // load before issuing the next); GRP = the whole chunk where the register budget allows
-      constexpr int GRP = QPD_STAGE(KC) ? CH : (QPD_STAGE_GROUP(KC) > 0 ? QPD_STAGE_GROUP(KC) : CH);
-      static_assert(GRP % 2 == 0, "groups of 16-byte pairs");
+      static_assert(CH % 4 == 0, "g chunks are loaded in 16-byte pairs and summed in four chains");
+      // the g chunk: a run of loads, a scheduling fence where the register budget allows (L::STAGE), the FMAs (ptxas
+      // otherwise consumes each load before issuing the next)
+      double gl[CH];
 #pragma unroll
-      for (int g0 = 0; g0 < CH; g0 += GRP) {
-        double gl[GRP];
+      for (int e = 0; e < CH; e += 2) qpd_lds2(gvh + e, gl[e], gl[e + 1]);
+      qpd_sched_fence_if<L::STAGE>();
 #pragma unroll
-        for (int e = 0; e < GRP; e += 2)
-          if (g0 + e < CH) qpd_lds2(gvh + g0 + e, gl[e], gl[e + 1]);
-        qpd_sched_fence_if<QPD_STAGE(KC) || (QPD_STAGE_GROUP(KC) > 0)>();
-#pragma unroll
-        for (int e = 0; e < GRP; e += 2) {
-          if (g0 + e < CH) {
-            if ((e >> 1) & 1) { a2 += G[g0 + e] * gl[e]; a3 += G[g0 + e + 1] * gl[e + 1]; }
-            else { a0 += G[g0 + e] * gl[e]; a1 += G[g0 + e + 1] * gl[e + 1]; }
-          }
-        }
+      for (int e = 0; e < CH; e += 4) {
+        a0 += G[e] * gl[e]; a1 += G[e + 1] * gl[e + 1]; a2 += G[e + 2] * gl[e + 2]; a3 += G[e + 3] * gl[e + 3];
       }
       double xt = (a0 + a1) + (a2 + a3);
       xt += sp_shfl_xor(xt, 1);
@@ -713,7 +630,7 @@ SP_DEV_NOINLINE void qpd_block(QpdIOT<QpdLayout<KC>::CH, QpdLayout<KC>::NSLOT> &
       const double a0 = cpa[0], a1 = cpa[1], a2 = cpa[2], a3 = cpa[3];
       const double b0 = cp2[0], b1 = cp2[1], b2 = cp2[2], b3 = cp2[3];
       const QpdLU la = LU_REG ? la_r : lua[0], lb = LU_REG ? l2_r : lu2[0];
-      qpd_sched_fence_if<QPD_STAGE_ROWS(KC)>();
+      qpd_sched_fence_if<L::STAGE_ROWS>();
       const double wa[4] = {a0, a1, a2, a3}, wb[4] = {b0, b1, b2, b3};
       const double za = qpd_diff_row(wa, oa, ra.scale), zb = qpd_diff_row(wb, ob, r2.scale);
       const double ua = qpd_row_update(ra, la, za, alpha), ub = qpd_row_update(r2, lb, zb, alpha);
@@ -724,7 +641,7 @@ SP_DEV_NOINLINE void qpd_block(QpdIOT<QpdLayout<KC>::CH, QpdLayout<KC>::NSLOT> &
       const double j0 = cp2[0], j1 = cp2[1], j2 = cp2[2], j3 = cp2[3], j4 = cp2[4], j5 = cp2[5];
       const double e0 = cej[0], e1 = cej[1], e2 = cej[2], e3 = cej[3], e4 = cej[4], e5 = cej[5];
       const QpdLU la = LU_REG ? la_r : lua[0], lj = LU_REG ? l2_r : lu2[0];
-      qpd_sched_fence_if<QPD_STAGE_ROWS(KC)>();
+      qpd_sched_fence_if<L::STAGE_ROWS>();
       const double wa[4] = {a0, a1, a2, a3};
       const double za = qpd_diff_row(wa, oa, ra.scale);
       const double zj = (e0 * j0 + e1 * j1) + (e2 * j2 + e3 * j3) + (e4 * j4 + e5 * j5);
@@ -829,77 +746,7 @@ SP_DEV_NOINLINE void qpd_block4(QpdIOT<QpdLayout<KC>::CH, QpdLayout<KC>::NSLOT> 
   io.xv = xv;
 }
 
-// The v-major form of the block (QPD_VMAJOR): thread t = h N + v.  Four barriers per iteration:
-//   S2  (h = 0 warps) g_v = (A' V)_v + sigma x - q        the whole 13-load gather per variable thread
-//   S3  (all)         partial_h[v] = G[v][chunk h] . g[chunk h]   g chunk by warp-uniform LDS.128 (one wavefront each)
-//   S3b (h = 0 warps) x~_v = sum_h partial_h[v], x = alpha x~ + (1 - alpha) x
-//   S1  (all)         one constraint row per thread: z~ = (A x~)_row, w += alpha (z~ - clip(w)), next v -> V
-template <int KC, typename SyncFn>
-SP_DEV_NOINLINE void qpd_block5(QpdIOT<QpdLayout<KC>::CH, QpdLayout<KC>::NSLOT> &io, double *smx, int ta, int n, double alpha, SyncFn sync_cta) {
-  using L = QpdLayout<KC>;
-  constexpr int N = L::N, CH = L::CH, TA = L::TA;
-  static_assert(L::VMAJOR && L::NCH == 4 && !L::TWO_SLOTS && CH % 4 == 0, "v-major layout");
-  int v, h;
-  qpd_map<KC>(ta, v, h);
-  const bool isg = v < N;
-  const bool isvar = isg && h == 0;
-  const int vk = isg ? v / 6 : 0, vj = isg ? v - 6 * vk : 0;
-  const double *vb = smx + L::O_V + QPD_VB * vk;
-  const double *vkk = smx + L::O_V + QPD_VB * (vj < 3 ? vk : vk + 1);
-  const double *vcf = smx + L::O_VCF + 3 * (isg ? v : 0);  // continuity gather coefficients (zero for unused segments)
-  double *gvp = smx + L::O_GV + (isg ? v : 0);
-  const double *gvh = smx + L::O_GV + CH * h;
-  double *psp = smx + L::O_PS + h * N + (isg ? v : 0);
-  const double *ps0 = smx + L::O_PS + (isg ? v : 0);
-  double *cxp = smx + L::O_C + QPD_CP + (isg ? v : 0);
-  // the thread's row
-  const bool isj = io.rows[2].meta & 8;
-  const int ri = isj ? 2 : 0;
-  QpdRow r = io.rows[ri];
-  const bool rvalid = r.meta & 8;
-  const int order = r.meta & 3;
-  const double *cp = smx + L::O_C + r.coff;
-  double *vp = smx + L::O_V + r.voff;
-  const QpdLU *lu = (const QpdLU *)(smx + L::O_LU) + ta + (isj ? 2 * TA : 0);
-  const double *cej = smx + L::O_CE + 6 * (isj ? 3 * ((r.meta >> 8) & 0xff) + ((r.meta >> 16) - 18) : 0);
-  double xv = io.xv;
-  const double sigv = io.sigv, qv = io.qv, tkv = io.tkv;
-  double G[CH];
-#pragma unroll
-  for (int e = 0; e < CH; e++) G[e] = io.G[e];
-  double yo = 0.0;
-  for (int i = 0; i < n; i++) {
-    if (i == n - 1) yo = r.rho * (r.w - r.p);
-    if (isvar) *gvp = qpd_gather(vb, vkk, vj, tkv, vcf[0], vcf[1], vcf[2]) + sigv * xv - qv;  // S2
-    sync_cta();
-    {  // S3
-      double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
-#pragma unroll
-      for (int e = 0; e < CH; e += 4) {
-        a0 += G[e] * gvh[e]; a1 += G[e + 1] * gvh[e + 1]; a2 += G[e + 2] * gvh[e + 2]; a3 += G[e + 3] * gvh[e + 3];
-      }
-      if (isg) *psp = (a0 + a1) + (a2 + a3);
-    }
-    sync_cta();
-    if (isvar) {  // S3b
-      const double xt = (ps0[0] + ps0[N]) + (ps0[2 * N] + ps0[3 * N]);
-      xv = alpha * xt + (1.0 - alpha) * xv;
-      *cxp = xt;
-    }
-    sync_cta();
-    if (rvalid) {  // S1
-      const QpdLU b = lu[0];
-      const double zt = isj ? qpd_join_row(cp, cej) : qpd_diff_row(cp, order, r.scale);
-      *vp = qpd_row_update(r, b, zt, alpha);
-    }
-    sync_cta();
-  }
-  io.rows[ri].w = r.w; io.rows[ri].p = r.p;
-  io.yo[0] = 0.0; io.yo[1] = 0.0; io.yo[2] = 0.0; io.yo[ri] = yo;
-  io.xv = xv;
-}
-
-// The full-row form of the block (QPD_ROWFULL): thread t < N is variable t and holds ROW t of G entirely; every thread
+// The full-row form of the block (QpdLayout::ROWFULL): thread t < N is variable t and holds ROW t of G entirely; every thread
 // carries NSLOT constraint rows (slot s = row s TA + t of the unified numbering).  Three barriers per iteration:
 //   S2  g_t = (A' V)_t + sigma x - q          13 loads in one run, then the arithmetic
 //   S3  x~_t = G[t][:] . g                     g read by every lane from the same address (one wavefront per LDS.128),
@@ -1211,7 +1058,6 @@ SP_DEV void qpd_cta_body(const QpArgs &a, int slot, int tid, double *smem, SyncF
     // one out-of-line call per check interval; before its LAST iteration the block captures the multipliers
     // y = rho (w - clip(w)) of the thread's rows (io.yo) for the delta y of the check
     if constexpr (L::ROWFULL) qpd_block1<KC>(io, smx, ta, it_end - it + 1, o.alpha, sync_cta);
-    else if constexpr (L::VMAJOR) qpd_block5<KC>(io, smx, ta, it_end - it + 1, o.alpha, sync_cta);
     else if constexpr (L::NCH == 4) qpd_block4<KC>(io, smx, ta, it_end - it + 1, o.alpha, sync_cta);
     else qpd_block<KC>(io, smx, ta, it_end - it + 1, o.alpha, sync_cta);
     iters = it_end;

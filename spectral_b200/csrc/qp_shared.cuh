@@ -6,15 +6,13 @@
 // depends on the structure and rho only, so ONE copy of G serves a TILE of 8 scenarios, and the per-iteration solve
 // X~ = G [g_1 .. g_8] becomes a dense multi-RHS contraction on mma.sync.m8n8k4.f64 (DMMA).
 //
-// Layout.  One CTA = one tile = two warps (warp 0: the s-axis problems, warp 1: the l-axis problems of the same 8 scenarios).
-// In a warp, lane = 4 n + q: scenario slot n = 0..7, quad lane q owns segments 2q and 2q+1 of that scenario: their 12 control
-// points (registers), their 42 constraint rows (w, l, u in shared memory, lane-interleaved) -- the stencils A x and A' v of a
-// segment are thread-local (apply_A / apply_AT of qp.cuh), only the three continuity rows at a thread boundary travel, by
-// quad shuffle.  The DMMA computes X~' = [g]' G with the 8 scenarios as the M dimension:
-//     A fragment (8 x 4)  a = g_n[12 q + s]                       k-step s = 0..11: the thread's own 12 gather values
-//     B fragment (4 x 8)  G[12 (lane & 3) + s][12 (r >> 1) + 2 nt + (r & 1)], r = lane >> 2, from shared memory (fragment order)
-//     C fragment (8 x 8)  x~_n[12 q + 2 nt + {0, 1}]              n-tile nt = 0..5: the thread's own 12 outputs
-// i.e. 72 DMMAs per iteration and axis, no data movement between the gather, the contraction and the row update.
+// This header holds the parts of the path around the tile kernel (k_qps4, qp_shared4.cuh, which describes its thread map and
+// its DMMA fragments): the structure keys that group scenarios into tiles (k_qps_keys / heads / flags / emit in capi.cu sort
+// the class by key and cut runs of equal keys into tiles of at most QPS_TILE), the per-tile structure block (QpsTileBlk) and
+// the kernel arguments (QpsArgs), the DMMA and shared-memory load primitives, and the bodies of the two kernels that bracket
+// the tile kernel:
+//   k_qps_prepare  K3 assembly of every member (l, u, q), and for a tile's first scenario the tile's scaling, rho and P
+//   k_qps_finish   status at max_iter, polish and outputs of every member (qp_finish of qp.cuh) in the tile scaling
 //
 // What differs from the per-scenario kernels (qp_anchor.cuh / qp_dense.cuh), and why it is a separate, opt-in path
 // (SpectralOptions::shared_kkt): a shared G needs ONE scaling and ONE rho for the tile.  The Ruiz scaling (D, E, c) is taken
@@ -29,15 +27,15 @@
 #define QPS_KC 8
 #define QPS_N 48
 #define QPS_TILE 8
-#define QPS_ROWSZ (21 * 32)             // one (slot, segl) plane of the row arrays: [row][lane]
-#define QPS_NFRAG 72                    // B fragments of G per axis: [nt 0..5][s 0..11]
+#define QPS_ROWSZ (21 * 32)             // one (slot, half) plane of the row arrays: [row][lane]
+#define QPS_NFRAG 72                    // B fragments of G per axis: [half][36]
 // The tile's structure slots are addressed like qp.cuh's lane slots (slot * 8 + segment) through a base pointer shifted so
 // that QP_SM_P is the first slot stored: P at QP_SM_P, rho at QPS_RHO, the row scalings E_r at QPS_ER.
 #define QPS_RHO (QP_SM_P + 21)
 #define QPS_ER (QP_SM_P + 42)
 #define QPS_FS_DOUBLES (2 * 57 * 8)     // factor store of one tile CTA (global scratch: read only when G is rebuilt)
 
-// per tile and axis; written by k_qps_prepare from the tile's first scenario, read by k_qps / k_qps_finish
+// per tile and axis; written by k_qps_prepare from the tile's first scenario, read by k_qps4 / k_qps_finish
 struct QpsTileBlk {
   double t[8], tp[8], tn[8];
   double rho[21][8];   // [row][segment]: the RHO slots of qp.cuh with stride 8
@@ -69,28 +67,6 @@ SP_DEV void qps_dmma(double a, double b, double &c0, double &c1) {
 #endif
 }
 
-// position of element (v, c) of G in the fragment array: B fragment of (n-tile, k-step) at lane
-SP_DEV int qps_frag_index(int v, int c) {
-  const int qv = v / 12, s = v - 12 * qv;
-  const int cq = c / 12, cr = c - 12 * cq;
-  const int nt = cr >> 1, r = 2 * cq + (cr & 1);
-  return (nt * 12 + s) * 32 + r * 4 + qv;
-}
-
-// shared memory of one tile CTA (doubles)
-struct QpsSmem {
-  static constexpr int O_ROWS = 0;                          // [axis][slot W/L/U][segl][21][32]
-  static constexpr int ROWS_AXIS = 3 * 2 * QPS_ROWSZ;
-  static constexpr int O_GF = O_ROWS + 2 * ROWS_AXIS;       // [axis][72][32]
-  static constexpr int O_CTL = O_GF + 2 * QPS_NFRAG * 32;   // [axis][63][8]: P, RHO and E_r slots, stride 8 (see QPS_RHO / QPS_ER)
-  static constexpr int CTL_AXIS = 63 * 8;
-  static constexpr int O_SEG = O_CTL + 2 * CTL_AXIS;        // [axis][8][16]: t, tp, tn, pad, sig[6], cD[6]
-  static constexpr int O_XCH = O_SEG + 2 * 8 * 16;          // [axis][8][QPD_NRED] cross-axis exchange of the check
-  static constexpr int O_FLAG = O_XCH + 2 * 8 * QPD_NRED;   // [2] cross-axis flags (bad pivot)
-  static constexpr int TOTAL = O_FLAG + 8;
-  static constexpr int BYTES = TOTAL * 8;
-};
-
 SP_DEV double qps_lds(const double *p) {
 #ifdef SPECTRAL_CPU_EMU
   return *p;
@@ -99,435 +75,6 @@ SP_DEV double qps_lds(const double *p) {
   asm volatile("ld.shared.f64 %0, [%1];" : "=d"(a) : "r"((unsigned)__cvta_generic_to_shared(p)));
   return a;
 #endif
-}
-
-// One ADMM row pass over the thread's segment `segl` (0 / 1): w += alpha (z~ - clip(w)), v = rho (2 clip(w) - w) of the new w.
-// Loads are staged in groups of 7 rows (ordered loads, then the arithmetic, then the stores) so that their latencies
-// overlap; the update is branch-free (a finished member runs it with alpha = 0).  CHECK: also the multiplier step
-// dy = y_new - y_old and its norm terms.
-template <bool CHECK, int RB, int RE, int CH>
-SP_DEV void qps_row_pass(double *__restrict__ rw, const double *__restrict__ rl, const double *__restrict__ ru, const double *__restrict__ rho,
-                         const double z[QP_ROWS], int lane, double alpha_eff, double v[QP_ROWS], double dy[QP_ROWS],
-                         const double *__restrict__ er_c, double c_scale, double &nd, double &lhs) {
-  static_assert((RE - RB) % CH == 0, "whole groups");
-#pragma unroll
-  for (int r0 = RB; r0 < RE; r0 += CH) {
-    double w[CH], l[CH], u[CH], rh[CH];
-#pragma unroll
-    for (int j = 0; j < CH; j++) {
-      w[j] = qps_lds(rw + (r0 + j) * 32 + lane); l[j] = qps_lds(rl + (r0 + j) * 32 + lane); u[j] = qps_lds(ru + (r0 + j) * 32 + lane);
-      rh[j] = qps_lds(rho + (r0 + j) * 8);
-    }
-#pragma unroll
-    for (int j = 0; j < CH; j++) {
-      const int r = r0 + j;
-      const double p = qpd_clip(w[j], l[j], u[j]);
-      const double wn = w[j] + alpha_eff * (z[r] - p);
-      const double pn = qpd_clip(wn, l[j], u[j]);
-      v[r] = rh[j] * (2.0 * pn - wn);
-      if (CHECK) {
-        const double d = rh[j] * (wn - pn) - rh[j] * (w[j] - p);
-        dy[r] = d;
-        const double live = rh[j] > 0.0 ? 1.0 : 0.0;
-        nd = qpd_max(nd, live * fabs(c_scale * d / er_c[r * 8]));
-        lhs += live * (c_scale * (u[j] * qpd_max(d, 0.0) + l[j] * (d < 0.0 ? d : 0.0)));
-      }
-      w[j] = wn;
-    }
-#pragma unroll
-    for (int j = 0; j < CH; j++) rw[(r0 + j) * 32 + lane] = w[j];
-  }
-}
-
-// warp: (re)factorise S for the RHO slots in ctl and rebuild the B fragments of G = S^-1 (setup and tile-rho updates)
-SP_DEV int qps_build_g(const double *ctl, double *fs, double *gf, const double *segc, int lane, int K) {
-  const int seg = lane & 7;
-  const double *sc = segc + 16 * seg;
-  double sig[6];
-#pragma unroll
-  for (int j = 0; j < 6; j++) sig[j] = sc[4 + j];
-  QpFactor F;
-  int bad = qp_factorize<8, 8>(ctl, seg, QPS_RHO, sig, sc[0], sc[1], sc[2], seg == 0, seg == K - 1, seg < K, seg, K, 0u, 0u, 0.0, F);
-  bad = sp_group_or(bad, 8);
-  if (lane < 8) {
-    double *dst = fs + 57 * seg;
-#pragma unroll
-    for (int e = 0; e < 21; e++) dst[e] = F.Linv[e];
-#pragma unroll
-    for (int e = 0; e < 18; e++) { dst[21 + e] = F.C[e]; dst[39 + e] = F.E[e]; }
-  }
-  sp_syncwarp();
-  for (int v = lane; v < 64; v += 32) {
-    double g[QPS_N];
-    qpd_inverse_chunk<QPS_KC>(fs, v < QPS_N ? v : 0, 0, g);
-    if (v < QPS_N) {
-#pragma unroll
-      for (int c = 0; c < QPS_N; c++) gf[qps_frag_index(v, c)] = g[c];
-    }
-  }
-  sp_syncwarp();
-  return bad;
-}
-
-// The tile body: `tid` in [0, 64).
-template <typename SyncFn>
-SP_DEV void qps_tile_body(const QpsArgs &A, int tile, int cta, int tid, double *smem, SyncFn sync_cta) {
-  using S = QpsSmem;
-  const QpArgs &a = A.q;
-  const SpOptionsDev &o = a.opt;
-  const int axis = tid >> 5, lane = tid & 31;
-  const int n = lane >> 2, q = lane & 3;
-  const int cnt = A.tile_count[tile];
-  const int b = A.sorted[A.tile_start[tile] + (n < cnt ? n : 0)];
-  const bool have = n < cnt;
-  double *rows = smem + S::O_ROWS + axis * S::ROWS_AXIS;
-  double *gf = smem + S::O_GF + axis * QPS_NFRAG * 32;
-  double *ctl = smem + S::O_CTL + axis * S::CTL_AXIS - QP_SM_P * 8;  // virtual base (see QPS_RHO)
-  double *fs = A.fs_scratch + ((size_t)cta * 2 + axis) * 57 * 8;
-  double *segc = smem + S::O_SEG + axis * 8 * 16;
-  double *xch = smem + S::O_XCH;
-  const QpsTileBlk &B = A.blk[2 * tile + axis];
-  const int K = B.K;
-  const double c_scale = B.c;
-  double rhobar = B.rhobar;
-
-  // ---------------- load the tile structure and the members' rows ----------------
-  for (int e = lane; e < 21 * 8; e += 32) {
-    ctl[QPS_RHO * 8 + e] = (&B.rho[0][0])[e];
-    ctl[QP_SM_P * 8 + e] = (&B.P[0][0])[e];
-  }
-  if (lane < 8) {
-    double *sc = segc + 16 * lane;
-    sc[0] = B.t[lane]; sc[1] = B.tp[lane]; sc[2] = B.tn[lane]; sc[3] = 0.0;
-#pragma unroll
-    for (int j = 0; j < 6; j++) { sc[4 + j] = B.sig[lane][j]; sc[10 + j] = B.cD[lane][j]; }
-  }
-  double qv[12], x[12], xt[12];
-#pragma unroll
-  for (int segl = 0; segl < 2; segl++) {
-    const int seg = 2 * q + segl;
-    const bool act = have && seg < K;
-    const double *lu = a.lu + (((size_t)b * 2 + axis) * a.k_max + seg) * QP_ROWS * 2;
-    const double *qs = A.qv + (((size_t)b * 2 + axis) * 8 + seg) * 6;
-    double *rw = rows + (0 * 2 + segl) * QPS_ROWSZ, *rl = rows + (1 * 2 + segl) * QPS_ROWSZ, *ru = rows + (2 * 2 + segl) * QPS_ROWSZ;
-#pragma unroll
-    for (int r = 0; r < QP_ROWS; r++) {
-      rw[r * 32 + lane] = 0.0;
-      rl[r * 32 + lane] = act ? lu[2 * r] : -1.0;
-      ru[r * 32 + lane] = act ? lu[2 * r + 1] : 1.0;
-    }
-#pragma unroll
-    for (int j = 0; j < 6; j++) { qv[6 * segl + j] = act ? qs[j] : 0.0; x[6 * segl + j] = 0.0; xt[6 * segl + j] = 0.0; }
-  }
-  sp_syncwarp();
-  // E_r of the tile scaling (invariant under rho updates): [row][seg]
-  for (int e = lane; e < 21 * 8; e += 32) {
-    const int r = e >> 3, seg = e & 7;
-    const int eq = (B.eqmask[seg] >> r) & 1;
-    const double rh = ctl[QPS_RHO * 8 + e];
-    ctl[QPS_ER * 8 + e] = (seg < K && rh > 0.0) ? sqrt(rh * (c_scale / rhobar) * (eq ? 1e-3 : 1.0)) : 1.0;
-  }
-  sp_syncwarp();
-  int bad = qps_build_g(ctl, fs, gf, segc, lane, K);
-  {  // a failed factorisation on either axis fails the tile on both (the two warps must hold the same states)
-    double *flag = smem + S::O_FLAG;
-    if (lane == 0) flag[axis] = (double)bad;
-    sync_cta();
-    bad = (flag[0] != 0.0 || flag[1] != 0.0) ? 1 : 0;
-    sync_cta();
-  }
-
-  // per-thread segment constants
-  double tS[2], tpS[2], tnS[2];
-  bool firstS[2], lastS[2], actS[2];
-#pragma unroll
-  for (int segl = 0; segl < 2; segl++) {
-    const int seg = 2 * q + segl;
-    tS[segl] = segc[16 * seg]; tpS[segl] = segc[16 * seg + 1]; tnS[segl] = segc[16 * seg + 2];
-    firstS[segl] = seg == 0; lastS[segl] = seg == K - 1; actS[segl] = seg < K;
-  }
-  int state = (have && K > 0) ? QP_RUNNING : QP_ST_MAXITER;
-  if (have && (bad || A.st[4 * b + 3])) state = QP_ST_INFEASIBLE;
-  int iters = 0;
-  const double alpha = o.alpha;
-
-  // g of the cold start: w = 0 -> v = 0 -> g = -q
-  double g[12];
-#pragma unroll
-  for (int j = 0; j < 12; j++) g[j] = -qv[j];
-
-  for (int it = 1; it <= o.max_iter; it++) {
-    const bool run = state == QP_RUNNING;
-    if (!sp_any(run)) break;   // (the two axis warps hold the same states: both leave together)
-    const bool check = (o.check_every > 0) && (it % o.check_every == 0);
-    // ---- S3: X~' = g' G on the FP64 tensor pipe (72 DMMAs, B fragments streamed from shared memory)
-#pragma unroll
-    for (int j = 0; j < 12; j++) xt[j] = 0.0;
-#pragma unroll
-    for (int s = 0; s < 12; s++) {
-      double bf[6];
-#pragma unroll
-      for (int nt = 0; nt < 6; nt++) bf[nt] = qps_lds(gf + (nt * 12 + s) * 32 + lane);
-#pragma unroll
-      for (int nt = 0; nt < 6; nt++) qps_dmma(g[s], bf[nt], xt[2 * nt], xt[2 * nt + 1]);
-    }
-    if (run) {
-#pragma unroll
-      for (int j = 0; j < 12; j++) x[j] = alpha * xt[j] + (1.0 - alpha) * x[j];
-      iters = it;
-    }
-    // ---- S1 + S2 fused: rows of segment 2q+1 then 2q; gathers
-    const double alpha_eff = run ? alpha : 0.0;  // a finished member keeps its state
-    double v0[QP_ROWS], v1[QP_ROWS], dy0[QP_ROWS], dy1[QP_ROWS];
-    double nd = 0.0, lhs = 0.0;
-    double *rw0 = rows + (0 * 2 + 0) * QPS_ROWSZ, *rw1 = rows + (0 * 2 + 1) * QPS_ROWSZ;
-    const double *rl0 = rows + (1 * 2 + 0) * QPS_ROWSZ, *rl1 = rows + (1 * 2 + 1) * QPS_ROWSZ;
-    const double *ru0 = rows + (2 * 2 + 0) * QPS_ROWSZ, *ru1 = rows + (2 * 2 + 1) * QPS_ROWSZ;
-    const double *rho0 = ctl + QPS_RHO * 8 + 2 * q, *rho1 = rho0 + 1, *er0 = ctl + QPS_ER * 8 + 2 * q, *er1 = er0 + 1;
-    // Order: (1) the three continuity rows of segment 2q -- the quad neighbour needs their values for its gather; (2) all rows
-    // of segment 2q+1 and its gather (v1 is dead after it); (3) the difference rows of segment 2q and its gather.  One v[21] live.
-    double z0[QP_ROWS];
-    {
-      const double p3 = sp_shfl_up(xt[9], 1, 4), p4 = sp_shfl_up(xt[10], 1, 4), p5 = sp_shfl_up(xt[11], 1, 4);
-      apply_A(xt, p3, p4, p5, tS[0], tpS[0], firstS[0], z0);
-    }
-    if (check) qps_row_pass<true, 18, 21, 3>(rw0, rl0, ru0, rho0, z0, lane, alpha_eff, v0, dy0, er0, c_scale, nd, lhs);
-    else qps_row_pass<false, 18, 21, 3>(rw0, rl0, ru0, rho0, z0, lane, alpha_eff, v0, dy0, nullptr, c_scale, nd, lhs);
-    double n18 = sp_shfl_down(v0[18], 1, 4), n19 = sp_shfl_down(v0[19], 1, 4), n20 = sp_shfl_down(v0[20], 1, 4);
-    if (lastS[1] || !actS[1] || q == 3) { n18 = 0.0; n19 = 0.0; n20 = 0.0; }
-    {
-      double z[QP_ROWS];
-      apply_A(xt + 6, xt[3], xt[4], xt[5], tS[1], tpS[1], false, z);
-      if (check) qps_row_pass<true, 0, 21, 7>(rw1, rl1, ru1, rho1, z, lane, alpha_eff, v1, dy1, er1, c_scale, nd, lhs);
-      else qps_row_pass<false, 0, 21, 7>(rw1, rl1, ru1, rho1, z, lane, alpha_eff, v1, dy1, nullptr, c_scale, nd, lhs);
-    }
-    apply_AT(v1, n18, n19, n20, tS[1], tpS[1], tnS[1], false, g + 6);
-    double m18 = v1[18], m19 = v1[19], m20 = v1[20];
-    if (lastS[0] || !actS[0]) { m18 = 0.0; m19 = 0.0; m20 = 0.0; }
-    if (check) qps_row_pass<true, 0, 18, 6>(rw0, rl0, ru0, rho0, z0, lane, alpha_eff, v0, dy0, er0, c_scale, nd, lhs);
-    else qps_row_pass<false, 0, 18, 6>(rw0, rl0, ru0, rho0, z0, lane, alpha_eff, v0, dy0, nullptr, c_scale, nd, lhs);
-    apply_AT(v0, m18, m19, m20, tS[0], tpS[0], tnS[0], firstS[0], g);
-    {
-      const double *sg0 = segc + 16 * (2 * q) + 4, *sg1 = segc + 16 * (2 * q + 1) + 4;
-#pragma unroll
-      for (int j = 0; j < 6; j++) { g[j] += sg0[j] * x[j] - qv[j]; g[6 + j] += sg1[j] * x[6 + j] - qv[6 + j]; }
-    }
-    if (!check) continue;
-
-    // ---- termination check (OSQP's test in the tile scaling), joint over the two axes of each scenario
-    double red_v[QPD_NRED];
-#pragma unroll
-    for (int i = 0; i < QPD_NRED; i++) red_v[i] = 0.0;
-    red_v[7] = nd; red_v[9] = lhs;
-    {
-      // A x (relaxed x), A' y, A' dy, P x per segment
-      double ax0[QP_ROWS], ax1[QP_ROWS];
-      apply_A(x + 6, x[3], x[4], x[5], tS[1], tpS[1], false, ax1);
-      const double p3 = sp_shfl_up(x[9], 1, 4), p4 = sp_shfl_up(x[10], 1, 4), p5 = sp_shfl_up(x[11], 1, 4);
-      apply_A(x, p3, p4, p5, tS[0], tpS[0], firstS[0], ax0);
-      double y0[QP_ROWS], y1[QP_ROWS];
-#pragma unroll
-      for (int segl = 0; segl < 2; segl++) {
-        const double *rw = rows + (0 * 2 + segl) * QPS_ROWSZ, *rl = rows + (1 * 2 + segl) * QPS_ROWSZ, *ru = rows + (2 * 2 + segl) * QPS_ROWSZ;
-        const double *rho = ctl + QPS_RHO * 8 + 2 * q + segl, *er = ctl + QPS_ER * 8 + 2 * q + segl;
-        const double *ax = segl ? ax1 : ax0;
-        double *y = segl ? y1 : y0;
-#pragma unroll
-        for (int r = 0; r < QP_ROWS; r++) {
-          const double w = rw[r * 32 + lane], p = qpd_clip(w, rl[r * 32 + lane], ru[r * 32 + lane]);
-          const double rh = rho[r * 8];
-          y[r] = rh * (w - p);
-          if (rh > 0.0 && actS[segl]) {
-            const double E = er[r * 8];
-            red_v[0] = qpd_max(red_v[0], E * fabs(ax[r] - p));
-            red_v[2] = qpd_max(red_v[2], E * fabs(p));
-            red_v[3] = qpd_max(red_v[3], E * fabs(ax[r]));
-          }
-        }
-      }
-      double aty[12], atd[12];
-      {
-        double n18 = sp_shfl_down(y0[18], 1, 4), n19 = sp_shfl_down(y0[19], 1, 4), n20 = sp_shfl_down(y0[20], 1, 4);
-        if (lastS[1] || !actS[1] || q == 3) { n18 = 0.0; n19 = 0.0; n20 = 0.0; }
-        double m18 = y1[18], m19 = y1[19], m20 = y1[20];
-        if (lastS[0] || !actS[0]) { m18 = 0.0; m19 = 0.0; m20 = 0.0; }
-        apply_AT(y0, m18, m19, m20, tS[0], tpS[0], tnS[0], firstS[0], aty);
-        apply_AT(y1, n18, n19, n20, tS[1], tpS[1], tnS[1], false, aty + 6);
-      }
-      {
-        double n18 = sp_shfl_down(dy0[18], 1, 4), n19 = sp_shfl_down(dy0[19], 1, 4), n20 = sp_shfl_down(dy0[20], 1, 4);
-        if (lastS[1] || !actS[1] || q == 3) { n18 = 0.0; n19 = 0.0; n20 = 0.0; }
-        double m18 = dy1[18], m19 = dy1[19], m20 = dy1[20];
-        if (lastS[0] || !actS[0]) { m18 = 0.0; m19 = 0.0; m20 = 0.0; }
-        apply_AT(dy0, m18, m19, m20, tS[0], tpS[0], tnS[0], firstS[0], atd);
-        apply_AT(dy1, n18, n19, n20, tS[1], tpS[1], tnS[1], false, atd + 6);
-      }
-#pragma unroll
-      for (int segl = 0; segl < 2; segl++) {
-        if (!actS[segl]) continue;
-        const int seg = 2 * q + segl;
-        double px[6];
-        apply_P<8>(ctl, seg, x + 6 * segl, px);
-        const double *cD = segc + 16 * seg + 10;
-#pragma unroll
-        for (int j = 0; j < 6; j++) {
-          const int jj = 6 * segl + j;
-          red_v[8] = qpd_max(red_v[8], fabs(cD[j] * atd[jj]));
-          red_v[1] = qpd_max(red_v[1], cD[j] * fabs(px[j] + qv[jj] + aty[jj]));
-          red_v[4] = qpd_max(red_v[4], cD[j] * fabs(qv[jj]));
-          red_v[5] = qpd_max(red_v[5], cD[j] * fabs(px[j]));
-          red_v[6] = qpd_max(red_v[6], cD[j] * fabs(aty[jj]));
-        }
-      }
-    }
-    // reduce over the quad, then across the two axis warps
-#pragma unroll
-    for (int i = 0; i < QPD_NRED - 1; i++) {
-      red_v[i] = qpd_max(red_v[i], sp_shfl_xor(red_v[i], 1));
-      red_v[i] = qpd_max(red_v[i], sp_shfl_xor(red_v[i], 2));
-    }
-    red_v[9] += sp_shfl_xor(red_v[9], 1);
-    red_v[9] += sp_shfl_xor(red_v[9], 2);
-    if (q == 0) {
-#pragma unroll
-      for (int i = 0; i < QPD_NRED; i++) xch[(axis * 8 + n) * QPD_NRED + i] = red_v[i];
-    }
-    sync_cta();
-    {
-      const double *o0 = xch + (0 * 8 + n) * QPD_NRED, *o1 = xch + (1 * 8 + n) * QPD_NRED;
-#pragma unroll
-      for (int i = 0; i < QPD_NRED - 1; i++) red_v[i] = qpd_max(o0[i], o1[i]);
-      red_v[9] = o0[9] + o1[9];
-    }
-    sync_cta();
-    const double pri = red_v[0], dua = red_v[1], nz = red_v[2], nax = red_v[3], nq = red_v[4], npx = red_v[5], naty = red_v[6];
-    const double ndn = red_v[7], na = red_v[8], lh = red_v[9];
-    const double eps_p = o.eps_abs + o.eps_rel * fmax(nz, nax);
-    const double eps_d = o.eps_abs + o.eps_rel * fmax(nq, fmax(npx, naty));
-    if (run) {
-      if (pri < eps_p && dua < eps_d) state = QP_ST_SOLVED;
-      else if (!(pri < eps_p) && ndn > o.eps_pinf && lh < -o.eps_pinf * ndn && na < o.eps_pinf * ndn) state = QP_ST_INFEASIBLE;
-    }
-    // ---- tile rho: OSQP's estimate per member, geometric mean over the members still running
-    if (o.adapt_every > 0 && (it % o.adapt_every == 0)) {
-      const bool still = state == QP_RUNNING;
-      const double pr = pri / (fmax(nz, nax) + 1e-10);
-      const double dr = dua / (fmax(nq, fmax(npx, naty)) + 1e-10);
-      double est = rhobar * sqrt(pr / (dr + 1e-10));
-      est = fmin(fmax(est, 1e-6), 1e6);
-      double ls = (still && q == 0) ? log(est) : 0.0, lc = (still && q == 0) ? 1.0 : 0.0;
-#pragma unroll
-      for (int m = 16; m > 0; m >>= 1) { ls += sp_shfl_xor(ls, m); lc += sp_shfl_xor(lc, m); }
-      if (lc > 0.0) {
-        const double tile_est = exp(ls / lc);
-        if (tile_est > rhobar * o.adapt_tol || tile_est < rhobar / o.adapt_tol) {
-          const double ratio = tile_est / rhobar;
-#pragma unroll
-          for (int segl = 0; segl < 2; segl++) {
-            double *rw = rows + (0 * 2 + segl) * QPS_ROWSZ;
-            const double *rl = rows + (1 * 2 + segl) * QPS_ROWSZ, *ru = rows + (2 * 2 + segl) * QPS_ROWSZ;
-#pragma unroll
-            for (int r = 0; r < QP_ROWS; r++) {
-              const double w = rw[r * 32 + lane], p = qpd_clip(w, rl[r * 32 + lane], ru[r * 32 + lane]);
-              rw[r * 32 + lane] = p + (w - p) / ratio;  // keep (z, y): w' = z + y / rho'
-            }
-          }
-          sp_syncwarp();
-          for (int e = lane; e < 21 * 8; e += 32) ctl[QPS_RHO * 8 + e] *= ratio;
-          rhobar = tile_est;
-          sp_syncwarp();
-          int b2 = qps_build_g(ctl, fs, gf, segc, lane, K);
-          {
-            double *flag = smem + S::O_FLAG;
-            if (lane == 0) flag[axis] = (double)b2;
-            sync_cta();
-            b2 = (flag[0] != 0.0 || flag[1] != 0.0) ? 1 : 0;
-            sync_cta();
-          }
-          if (b2 && state == QP_RUNNING) state = QP_ST_INFEASIBLE;
-          // v and g of the rescaled rows
-#pragma unroll
-          for (int segl = 0; segl < 2; segl++) {
-            const double *rw = rows + (0 * 2 + segl) * QPS_ROWSZ, *rl = rows + (1 * 2 + segl) * QPS_ROWSZ, *ru = rows + (2 * 2 + segl) * QPS_ROWSZ;
-            const double *rho = ctl + QPS_RHO * 8 + 2 * q + segl;
-            double *v = segl ? v1 : v0;
-#pragma unroll
-            for (int r = 0; r < QP_ROWS; r++) {
-              const double w = rw[r * 32 + lane], p = qpd_clip(w, rl[r * 32 + lane], ru[r * 32 + lane]);
-              v[r] = rho[r * 8] * (2.0 * p - w);
-            }
-          }
-          double n18 = sp_shfl_down(v0[18], 1, 4), n19 = sp_shfl_down(v0[19], 1, 4), n20 = sp_shfl_down(v0[20], 1, 4);
-          if (lastS[1] || !actS[1] || q == 3) { n18 = 0.0; n19 = 0.0; n20 = 0.0; }
-          double m18 = v1[18], m19 = v1[19], m20 = v1[20];
-          if (lastS[0] || !actS[0]) { m18 = 0.0; m19 = 0.0; m20 = 0.0; }
-          apply_AT(v0, m18, m19, m20, tS[0], tpS[0], tnS[0], firstS[0], g);
-          apply_AT(v1, n18, n19, n20, tS[1], tpS[1], tnS[1], false, g + 6);
-          const double *sg0 = segc + 16 * (2 * q) + 4, *sg1 = segc + 16 * (2 * q + 1) + 4;
-#pragma unroll
-          for (int j = 0; j < 6; j++) { g[j] += sg0[j] * x[j] - qv[j]; g[6 + j] += sg1[j] * x[6 + j] - qv[6 + j]; }
-        }
-      }
-    }
-  }
-
-  // ---------------- hand off to k_qps_finish: w rows, relaxed x, state, iterations; the tile's final rho ----------------
-  if (have) {
-#pragma unroll
-    for (int segl = 0; segl < 2; segl++) {
-      const int seg = 2 * q + segl;
-      const double *rw = rows + (0 * 2 + segl) * QPS_ROWSZ;
-      double *dw = A.wrows + (((size_t)b * 2 + axis) * 8 + seg) * QP_ROWS;
-#pragma unroll
-      for (int r = 0; r < QP_ROWS; r++) dw[r] = rw[r * 32 + lane];
-      double *dx = A.xout + ((size_t)b * 2 + axis) * QPS_N + 6 * seg;
-#pragma unroll
-      for (int j = 0; j < 6; j++) dx[j] = x[6 * segl + j];
-    }
-    if (q == 0 && axis == 0) { A.st[4 * b + 0] = state; A.st[4 * b + 1] = iters; A.st[4 * b + 2] = tile; }
-  }
-  sp_syncwarp();
-  QpsTileBlk &Bw = A.blk[2 * tile + axis];
-  for (int e = lane; e < 21 * 8; e += 32) (&Bw.rho[0][0])[e] = ctl[QPS_RHO * 8 + e];
-  if (lane == 0) Bw.rhobar = rhobar;
-}
-
-// Deferred finish of the per-scenario anchor kernel (K <= 8 class): the CTA that ran the ADMM loop of one scenario hands its end
-// state to k_qps_finish in the formats of the shared-KKT path -- the scenario is its own "tile" (tile id = its slot in the class
-// list): structure block, (l, u) rows, q, w rows, relaxed x, state.  All of it sits in the control slots of the CTA's shared
-// memory (QpdLayout<8>: slots [slot][segment] with stride 8, lane store, XR) when the loop ends.
-SP_DEV void qpa_handoff(const QpsArgs &A, int slot, int tid, int nthreads, const double *smem) {
-  using L = QpdLayout<QPS_KC>;
-  static_assert(L::STR == 8 && L::LPA == 8, "control slots of the K <= 8 layout");
-  const QpArgs &a = A.q;
-  const int b = a.list[slot];
-  const double *red = smem + L::O_RED;
-  const int *eqm = (const int *)(smem + L::O_EQ);
-  for (int e = tid; e < 2 * 8 * QP_ROWS; e += nthreads) {
-    const int axis = e / (8 * QP_ROWS), rem = e - axis * 8 * QP_ROWS, seg = rem / QP_ROWS, r = rem - seg * QP_ROWS;
-    const double *ctl = smem + axis * L::AXIS + L::O_CTRL;
-    QpsTileBlk &Bk = A.blk[2 * slot + axis];
-    Bk.rho[r][seg] = ctl[(QP_SM_RHO + r) * 8 + seg];
-    Bk.P[r][seg] = ctl[(QP_SM_P + r) * 8 + seg];
-    double *lu = a.lu + ((((size_t)b * 2 + axis) * a.k_max + seg) * QP_ROWS + r) * 2;
-    lu[0] = ctl[(QP_SM_L + r) * 8 + seg];
-    lu[1] = ctl[(QP_SM_U + r) * 8 + seg];
-    A.wrows[(((size_t)b * 2 + axis) * 8 + seg) * QP_ROWS + r] = ctl[(QP_SM_W + r) * 8 + seg];
-  }
-  for (int e = tid; e < 2 * 8; e += nthreads) {
-    const int axis = e >> 3, seg = e & 7;
-    const double *d = smem + axis * L::AXIS + L::O_LS + QPD_LS * seg;
-    const double *xr = smem + axis * L::AXIS + L::O_XR + QPD_CP + 6 * seg;
-    QpsTileBlk &Bk = A.blk[2 * slot + axis];
-    Bk.t[seg] = d[0]; Bk.tp[seg] = d[1]; Bk.tn[seg] = d[2];
-    double *qs = A.qv + (((size_t)b * 2 + axis) * 8 + seg) * 6;
-    double *dx = A.xout + ((size_t)b * 2 + axis) * QPS_N + 6 * seg;
-#pragma unroll
-    for (int j = 0; j < 6; j++) { qs[j] = d[3 + j]; Bk.sig[seg][j] = d[9 + j]; Bk.cD[seg][j] = d[15 + j]; dx[j] = xr[j]; }
-    Bk.eqmask[seg] = eqm[axis * 8 + seg];
-    if (seg == 0) { Bk.c = red[0]; Bk.rhobar = red[1]; Bk.K = a.K[b]; Bk.pad = 0; }
-  }
-  if (tid == 0) { A.st[4 * b + 0] = (int)red[2]; A.st[4 * b + 1] = (int)red[3]; A.st[4 * b + 2] = slot; A.st[4 * b + 3] = 0; }
 }
 
 // k_qps_prepare body: one warp = two scenarios of the K <= 8 class (16 lanes each: 8 segment lanes per axis).  K3 assembly

@@ -1,15 +1,20 @@
-// spectral_b200/csrc/qp_shared4.cuh -- K4a, second layout: the shared-KKT tile kernel with FOUR warps per tile.
+// spectral_b200/csrc/qp_shared4.cuh -- K4a: the shared-KKT tile kernel k_qps4, four warps per tile.
 //
-// Same algorithm, same tile builder and the same prepare / finish kernels as qp_shared.cuh (read that header first); only the
-// thread map of the tile body changes (and with it where the w rows live: registers here, shared memory there).  The two-warp layout (one warp per axis, two
-// segments per thread) is bound by shared-memory CAPACITY, not by any pipe: 110 KB per tile -> two tiles = four warps per SM,
-// one warp per scheduler, every dependent-instruction latency exposed (profiles/r2_qps_full.md: sm__warps_active 5.6 %,
-// stall "wait" 2.2 per issue).  Here one tile = 4 warps = (axis, half): lane 4n + q of warp (axis, h) owns ONE segment,
-// seg = 4h + q, of scenario n -- twice the warps per byte of shared memory, half the serial work per thread.
+// The tile structure, the keys, and the prepare / finish kernels around this one are in qp_shared.cuh (read that header first).
+// Layout.  One CTA = one tile = 4 warps = (axis, half): lane 4n + q of warp (axis, h) owns ONE segment, seg = 4h + q, of
+// scenario n = 0..7: its 6 control points and its 21 constraint rows (w in registers, l, u in shared memory, lane-interleaved).
+// The stencils A x and A' v of a segment are thread-local (apply_A / apply_AT of qp.cuh); only the three continuity rows at a
+// segment boundary travel, by quad shuffle inside a warp.  The DMMA (mma.sync.m8n8k4.f64) computes X~' = [g]' G with the 8
+// scenarios of the tile as the M dimension: the A fragments are the threads' own gather values, the B fragments G from shared
+// memory, the C fragments the threads' own outputs x~ -- no data movement between the gather, the contraction and the row update.
+// Why four warps: the two-warp layout measured in round 2 (one warp per axis, two segments per thread, w rows in shared memory)
+// was bound by shared-memory CAPACITY, not by any pipe: 110 KB per tile -> two tiles = four warps per SM, one warp per
+// scheduler, every dependent-instruction latency exposed (profiles/r2_qps_full.md: sm__warps_active 5.6 %, stall "wait" 2.2 per
+// issue).  Here there are twice the warps per byte of shared memory and half the serial work per thread.
 //
 // DMMA split.  The k dimension of X~' = [g]' G (48 variables of an axis) is split between the two warps of the axis: warp h
 // contracts its own 24 gather values (6 k-steps x 4 quad lanes) against ALL 48 columns (6 n-tiles) -- 36 DMMAs per warp,
-// 72 per axis as before.  The column order of its B fragments puts its OWN segments' outputs in n-tiles 0..2 and the OTHER
+// 72 per axis.  The column order of its B fragments puts its OWN segments' outputs in n-tiles 0..2 and the OTHER
 // warp's in n-tiles 3..5, so that thread (n, q) holds the partial sums of exactly its own six outputs and of the six outputs
 // of thread (n, q) of the other warp: one 6-double store, one named barrier over the 64 threads of the axis, one 6-double
 // load complete x~.  The continuity rows couple segment 3 (warp 0, q = 3) with segment 4 (warp 1, q = 0): x~ of segment 3's
@@ -21,8 +26,8 @@
 #define QPS4_EXT (2 * 3 * 32)       // [axis][j][lane]: warp 0's own partial sums of control points 3..5 (for segment 4's join rows)
 #define QPS4_NXT (2 * 3 * 8)        // [axis][row 18..20][scenario]: join-row values of segment 4 (for segment 3's gather)
 
-// shared memory of one four-warp tile CTA (doubles).  The w rows live in REGISTERS here (21 per thread: one segment), which
-// frees a third of the row arrays for the exchange buffers and keeps two tiles per SM.
+// shared memory of one four-warp tile CTA (doubles).  The w rows live in REGISTERS (21 per thread: one segment), so the row
+// arrays hold only l and u, which leaves room for the exchange buffers at two tiles per SM.
 struct Qps4Smem {
   static constexpr int O_ROWS = 0;                          // [axis][slot L/U][h][21][32]
   static constexpr int ROWS_AXIS = 2 * 2 * QPS_ROWSZ;
@@ -41,7 +46,7 @@ struct Qps4Smem {
 
 // One ADMM row pass over the thread's segment, rows [RB, RE), with the w rows in registers: w += alpha (z~ - clip(w)),
 // v = rho (2 clip(w) - w) of the new w.  Loads (l, u, rho) staged in groups of CH rows.  CHECK: also the multiplier step
-// dy = y_new - y_old and its norm terms.  Same arithmetic as qps_row_pass.
+// dy = y_new - y_old and its norm terms.  The update is branch-free: a finished member runs it with alpha = 0.
 template <bool CHECK, int RB, int RE, int CH>
 SP_DEV void qps4_row_pass(double w[QP_ROWS], const double *__restrict__ rl, const double *__restrict__ ru, const double *__restrict__ rho,
                           const double z[QP_ROWS], int lane, double alpha_eff, double v[QP_ROWS], double dy[QP_ROWS],

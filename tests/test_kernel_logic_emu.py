@@ -60,7 +60,7 @@ def _subset(batch, idx):
 
 
 def test_emu_dense_kernel_tracks_reference_osqp():
-    """The dense-operator ADMM loop (qp_dense.cuh, k_qpd<8> and k_qpd<10>) solves both axes of a scenario as ONE
+    """The dense-operator ADMM loop (qp_anchor.cuh, k_qpa<8> and k_qpa<10>) solves both axes of a scenario as ONE
     OSQP instance like the reference: on scenarios that converge quickly the ITERATION COUNT equals that of the
     reference-settings oracle, infeasible ones are certified at the same check, and the polished control
     points match the converged oracle.  Scenarios: K = 9 (#779), K = 10 (#508: 1200 iterations), an early
@@ -82,7 +82,7 @@ def test_emu_anchor_layout_equals_fullrow(monkeypatch):
     from spectral_b200.scenarios import GOLDEN_W_CUB
     batch = _subset(config2(1024), [779, 914])
     new = H.emu_solve("cub", batch, GOLDEN_W_CUB)
-    monkeypatch.setenv("SPECTRAL_LEGACY_QPD", "1")
+    monkeypatch.setenv("SPECTRAL_EMU_FULLROW", "1")
     old = H.emu_solve("cub", batch, GOLDEN_W_CUB)
     assert list(new.K) == [9, 4]
     assert np.array_equal(new.iters, old.iters) and np.array_equal(new.status, old.status) and np.array_equal(new.flags, old.flags)
@@ -102,8 +102,9 @@ def test_emu_many_segments_joint_solve():
 
 
 def test_emu_lane_kernel_matches_dense_kernel(monkeypatch):
-    """The lane-per-segment loop (qp.cuh, used above the dense kernel's capacity) and the dense loop are the
-    same OSQP iteration: same iteration count, same status, same polished optimum."""
+    """The lane-per-segment body of k_qp<32,2> (qp.cuh, the product's kernel above the dense kernels' capacity, K > 16),
+    run here at K <= 16, and the dense loop are the same OSQP iteration: same iteration count, same status, same polished
+    optimum."""
     batch = ScenarioBatch.from_scenarios([load_fixture("c4_2")])
     dense = H.emu_solve("trp", batch, WEIGHTS_FILE)
     monkeypatch.setenv("SPECTRAL_EMU_LANES", "1")

@@ -50,8 +50,8 @@ extern "C" int emu_solve_batch(int variant, int B, int N, int R, double delta, c
                                const SpectralOptions *opt, int *K, SpectralCube *segs, double *ctrl,
                                double *obj, double *a_cost, int *status, int *iters, int *flags, int *npts,
                                double *samples, int samples_cap, double *lu) {
-  const bool force_lanes = getenv("SPECTRAL_EMU_LANES") != nullptr;  // run the lane-per-segment loop for every class
-  const bool legacy_qpd = getenv("SPECTRAL_LEGACY_QPD") != nullptr;   // the full-row loop instead of the anchor layout (K <= 10)
+  const bool force_lanes = getenv("SPECTRAL_EMU_LANES") != nullptr;  // run the lane-per-segment body of k_qp<32, 2> for every class
+  const bool fullrow = getenv("SPECTRAL_EMU_FULLROW") != nullptr;     // K <= 10: the full-row loop, the anchor layout's reference
   std::vector<int> cstatus(B, 0);
   // ---- corridor kernel: one CTA per scenario, R warps
   CorridorArgs ca{B, N, R, variant, k_max, delta, s_bounds, l_bounds, s_ref, l_ref, segs, K, cstatus.data()};
@@ -106,8 +106,8 @@ extern "C" int emu_solve_batch(int variant, int B, int N, int R, double delta, c
         run_warps(nwarps, [&](int w, int l, pthread_barrier_t *cta) {
           auto sync = [cta]() { pthread_barrier_wait(cta); };
           auto sync_axis = [&axbar](int axis) { pthread_barrier_wait(&axbar[axis]); };
-          if (cls == 0 && !legacy_qpd) qpa_cta_body<8>(qa, slot, 32 * w + l, base, sync, sync_axis);
-          else if (cls == 1 && !legacy_qpd) qpa_cta_body<10>(qa, slot, 32 * w + l, base, sync, sync_axis);
+          if (cls == 0 && !fullrow) qpa_cta_body<8>(qa, slot, 32 * w + l, base, sync, sync_axis);
+          else if (cls == 1 && !fullrow) qpa_cta_body<10>(qa, slot, 32 * w + l, base, sync, sync_axis);
           else if (cls == 0) qpd_cta_body<8>(qa, slot, 32 * w + l, base, sync);
           else if (cls == 1) qpd_cta_body<10>(qa, slot, 32 * w + l, base, sync);
           else if (cls == 2) qpd_cta_body<12>(qa, slot, 32 * w + l, base, sync);
@@ -117,24 +117,12 @@ extern "C" int emu_solve_batch(int variant, int B, int N, int R, double delta, c
       }
       continue;
     }
-    const int lpa = cls <= 0 ? 8 : (cls <= 3 ? 16 : 32);
-    if (lpa == 32) {  // k_qp<32, 2>: one CTA of two warps per scenario (s-axis warp, l-axis warp, joint reductions)
-      for (int slot = 0; slot < cnt; slot++) {
-        std::vector<double> sm(2 * QP_SM_DOUBLES_PER_LANE * 32 + QP_XCH_DOUBLES);
-        run_warps(2, [&](int w, int l, pthread_barrier_t *) {
-          qp_warp_body<32, 64>(qa, 2 * slot + w, l, sm.data() + (size_t)w * QP_SM_DOUBLES_PER_LANE * 32,
-                               sm.data() + 2 * QP_SM_DOUBLES_PER_LANE * 32);
-        });
-      }
-      continue;
-    }
-    const int G = 32 / lpa;
-    const int nw = (2 * cnt + G - 1) / G;
-    for (int w = 0; w < nw; w++) {
-      std::vector<double> sm(QP_SM_DOUBLES_PER_LANE * 32);
-      run_warps(1, [&](int, int l, pthread_barrier_t *) {
-        if (lpa == 8) qp_warp_body<8, 16>(qa, w, l, sm.data(), nullptr);
-        else qp_warp_body<16, 32>(qa, w, l, sm.data(), nullptr);
+    // k_qp<32, 2>: one CTA of two warps per scenario (s-axis warp, l-axis warp, joint reductions)
+    for (int slot = 0; slot < cnt; slot++) {
+      std::vector<double> sm(2 * QP_SM_DOUBLES_PER_LANE * 32 + QP_XCH_DOUBLES);
+      run_warps(2, [&](int w, int l, pthread_barrier_t *) {
+        qp_warp_body<32, 64>(qa, 2 * slot + w, l, sm.data() + (size_t)w * QP_SM_DOUBLES_PER_LANE * 32,
+                             sm.data() + 2 * QP_SM_DOUBLES_PER_LANE * 32);
       });
     }
   }
