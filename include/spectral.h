@@ -48,7 +48,11 @@ extern "C" {
 #define SPECTRAL_FAIL_NO_CORRIDOR 2  /* CollisionCheck selected nothing (reference: UB, solve_3d.cc:617) */
 #define SPECTRAL_FAIL_SOLVER 3       /* Optimize() == false -> find_traj returns 1e11 (trp_wrapper.cpp:199) */
 #define SPECTRAL_FAIL_POINTS_CHECK 4 /* CHECK_EQ(var_index, num_of_points_) would abort (solve_3d.cc:1407) */
-#define SPECTRAL_FAIL_TOO_MANY 5     /* more cubes/segments than the handle's capacity */
+/* SPECTRAL_FAIL_TOO_MANY: the corridor exceeds a capacity.  K[] is then
+ *   0        when a region holds more than 64 cubes before the split (64 or more slope breaks) or after it,
+ *   0        when CollisionCheck selects more than 64 distinct cubes (the CPU oracle reports their count here),
+ *   the true segment count K when K > k_max. */
+#define SPECTRAL_FAIL_TOO_MANY 5
 
 /* per-scenario flags[] bits */
 #define SPECTRAL_FLAG_POLISHED_S 1 /* s-axis control points come from an accepted polish step */

@@ -7,7 +7,7 @@
 // Mapping: one CTA per scenario, one warp per lateral region ("corridor face set").  Each warp
 // stages its region's s/l bound slabs (2 x 16N bytes) into shared memory with a 1-D bulk async
 // copy (TMA, cp.async.bulk + mbarrier), finds the slope breaks with ballot votes, splits its
-// cubes (one lane per pre-split cube) and counts the reference-trajectory points inside each
+// cubes (lane j % 32 holds pre-split cube j) and counts the reference-trajectory points inside each
 // cube (lanes over knots, popc of ballots).  Warp 0 then replays the selection / dedupe / sort /
 // swap / de-overlap logic, whose O(K^2) sequential parts run on lane 0 exactly as written in the
 // reference (including libstdc++'s std::sort algorithm, whose result on equal keys is
@@ -250,9 +250,11 @@ SP_DEV int corridor_generate_region(int variant, int N, double delta, const doub
 #define XHI(i) xb[2 * (i) + 1]
 #define YLO(i) yb[2 * (i)]
 #define YHI(i) yb[2 * (i) + 1]
-  // pre-split cube j lives in the registers of lane j
-  SpectralCube mine;
-  cube_defaults(mine);
+  // pre-split cube j lives in the registers of lane j % 32, slot j / 32: up to SP_REGION_CAP = 64 cubes, the oracle's cap.
+  // Slots are only ever indexed with constants (both branches written out), which keeps them in registers.
+  SpectralCube mine[2];
+  cube_defaults(mine[0]);
+  cube_defaults(mine[1]);
   int j = 0;
   // backward slopes of every knot, once (:355-356; the forward slope at a break knot i, :380-384, is the backward slope
   // of knot i + 1: same operands, same operation).  The break search below then only compares.
@@ -265,14 +267,15 @@ SP_DEV int corridor_generate_region(int variant, int N, double delta, const doub
   double cur_down = dsk[1];  // :332
   double cur_up = usk[1];    // :334
   if (lane == 0) {
-    mine.beg_t = 0;
-    mine.down_skew = cur_down; mine.down_bias = XLO(0);
-    mine.upp_skew = cur_up; mine.upp_bias = XHI(0);
+    SpectralCube &c = mine[0];
+    c.beg_t = 0;
+    c.down_skew = cur_down; c.down_bias = XLO(0);
+    c.upp_skew = cur_up; c.upp_bias = XHI(0);
     if (variant == SPECTRAL_TRP) {  // :338-341
-      mine.l_down_skew = slope_div(YLO(1) - YLO(0), delta); mine.l_down_bias = YLO(0);
-      mine.l_upp_skew = slope_div(YHI(1) - YHI(0), delta); mine.l_upp_bias = YHI(0);
+      c.l_down_skew = slope_div(YLO(1) - YLO(0), delta); c.l_down_bias = YLO(0);
+      c.l_upp_skew = slope_div(YHI(1) - YHI(0), delta); c.l_upp_bias = YHI(0);
     }
-    mine.beg_l = YLO(0); mine.end_l = YHI(0);
+    c.beg_l = YLO(0); c.end_l = YHI(0);
   }
   j = 1;
   int i0 = 2;
@@ -288,47 +291,68 @@ SP_DEV int corridor_generate_region(int variant, int N, double delta, const doub
       if (m) { found = base + sp_ffs(m) - 1; break; }
     }
     if (found < 0) break;
-    if (j >= 32) { overflow = 1; break; }
+    if (j >= SP_REGION_CAP) { overflow = 1; break; }
     const int i = found;
-    if (lane == j - 1) mine.end_t = i;  // :376
+    if (lane == ((j - 1) & 31)) {  // :376
+      if (j - 1 < 32) mine[0].end_t = i;
+      else mine[1].end_t = i;
+    }
     cur_down = dsk[i + 1];  // :380
     cur_up = usk[i + 1];    // :384
-    if (lane == j) {
-      mine.beg_t = i;
-      mine.down_skew = cur_down; mine.down_bias = XLO(i);
-      mine.upp_skew = cur_up; mine.upp_bias = XHI(i);
+    if (lane == (j & 31)) {
+      SpectralCube c;
+      cube_defaults(c);
+      c.beg_t = i;
+      c.down_skew = cur_down; c.down_bias = XLO(i);
+      c.upp_skew = cur_up; c.upp_bias = XHI(i);
       if (variant == SPECTRAL_TRP) {  // :360-367, backward differences at the break knot
-        mine.l_down_bias = YLO(i); mine.l_upp_bias = YHI(i);
-        mine.l_down_skew = slope_div(YLO(i) - YLO(i - 1), delta);
-        mine.l_upp_skew = slope_div(YHI(i) - YHI(i - 1), delta);
+        c.l_down_bias = YLO(i); c.l_upp_bias = YHI(i);
+        c.l_down_skew = slope_div(YLO(i) - YLO(i - 1), delta);
+        c.l_upp_skew = slope_div(YHI(i) - YHI(i - 1), delta);
       }
-      mine.beg_l = YLO(i); mine.end_l = YHI(i);  // :388-389
+      c.beg_l = YLO(i); c.end_l = YHI(i);  // :388-389
+      if (j < 32) mine[0] = c;
+      else mine[1] = c;
     }
     j++;
     i0 = i + 1;
   }
   if (overflow) return -1;
-  if (lane == j - 1) mine.end_t = N - 1;  // :461
-  mine.t = (mine.end_t - mine.beg_t) * delta;  // :465  (int -> double, then * delta)
+  if (lane == ((j - 1) & 31)) {  // :461
+    if (j - 1 < 32) mine[0].end_t = N - 1;
+    else mine[1].end_t = N - 1;
+  }
+  const int nslot = j > 32 ? 2 : 1;
 
-  // CorridorSplit (:729-772): lane j peels 1.0 s / 10-knot pieces off the front of its cube
-  int pieces = 0;
-  if (lane < j) {
-    double t = mine.t;
-    while (t > 1) { t = t - 1; pieces++; }
+  // CorridorSplit (:729-772): each pre-split cube peels 1.0 s / 10-knot pieces off its front; cube j's pieces are written
+  // after those of cubes 0 .. j-1 (a prefix sum over slot 0, then over slot 1)
+  int pieces[2] = {0, 0}, pos[2] = {0, 0};
+  int total = 0;
+#pragma unroll
+  for (int s = 0; s < 2; s++) {
+    if (s >= nslot) break;
+    const bool have = 32 * s + lane < j;
+    mine[s].t = (mine[s].end_t - mine[s].beg_t) * delta;  // :465  (int -> double, then * delta)
+    if (have) {
+      double t = mine[s].t;
+      while (t > 1) { t = t - 1; pieces[s]++; }
+    }
+    const int mycount = have ? pieces[s] + 1 : 0;
+    int incl = mycount;
+    for (int d = 1; d < 32; d <<= 1) {
+      int o = sp_shfl_up_i(incl, d, 32);
+      if (lane >= d) incl += o;
+    }
+    pos[s] = total + incl - mycount;
+    total += sp_shfl_i(incl, 31);
   }
-  const int mycount = (lane < j) ? pieces + 1 : 0;
-  int incl = mycount;
-  for (int d = 1; d < 32; d <<= 1) {
-    int o = sp_shfl_up_i(incl, d, 32);
-    if (lane >= d) incl += o;
-  }
-  const int total = sp_shfl_i(incl, 31);
   if (total > SP_REGION_CAP) return -1;
-  if (lane < j) {
-    int pos = incl - mycount;
-    SpectralCube rest = mine;
-    for (int p = 0; p < pieces; p++) {
+#pragma unroll
+  for (int s = 0; s < 2; s++) {
+    if (32 * s + lane >= j) continue;
+    int p_out = pos[s];
+    SpectralCube rest = mine[s];
+    for (int p = 0; p < pieces[s]; p++) {
       rest.t = rest.t - 1;  // :737
       SpectralCube m;
       cube_defaults(m);
@@ -343,9 +367,9 @@ SP_DEV int corridor_generate_region(int variant, int N, double delta, const doub
       if (variant == SPECTRAL_TRP) { m.l_upp_skew = rest.l_upp_skew; m.l_upp_bias = rest.l_upp_bias; }
       m.beg_l = rest.beg_l; m.end_l = rest.end_l;
       rest.upp_bias = m.upp_bias + 1.0 * m.upp_skew;  // :764
-      out[pos++] = m;
+      out[p_out++] = m;
     }
-    out[pos] = rest;
+    out[p_out] = rest;
   }
   return total;
 #undef XLO

@@ -179,6 +179,83 @@ def zigzag_breaks(base: Scenario, B: int, seed: int = 4242, s_max: float = 100.0
                          batch.l_ref, batch.init, batch.scalars)
 
 
+def slope_wiggle(n_knots: int, breaks: Sequence[int], delta_t: float = 0.1) -> np.ndarray:
+    """Upper s-bound over `n_knots` knots: 200 m plus a ramp whose slope toggles between 0 and 0.5 m/s at each knot of
+    `breaks` (the backward slope of knot i is the new one from i in `breaks` on).  Each toggle differs from the current
+    cube's slope by more than CorridorGeneration's 0.2 threshold (solve_3d.cc:372), so each one starts a new pre-split cube
+    as long as consecutive breaks are at least two knots apart and lie in [2, n_knots - 2]."""
+    slope = np.zeros(n_knots)
+    cur = 0.0
+    at = set(int(i) for i in breaks)
+    for i in range(1, n_knots):
+        if i in at:
+            cur = 0.5 - cur
+        slope[i] = cur
+    return 200.0 + np.cumsum(slope * delta_t)
+
+
+def ladder_shape(K: int):
+    """(n_knots, break knots) of `segment_ladder` for K segments (see there)."""
+    if K < 1:
+        raise ValueError("K >= 1")
+    if K <= 25:
+        return 10 * K + 1, []
+    return 256, [15 * (m + 1) for m in range(2 * (K - 26))]
+
+
+def wiggle_batch(n_knots: int, breaks, B: int, seed: int = 20231021, regions=None) -> ScenarioBatch:
+    """B scenarios on a free road (one region, delta_t = 0.1 s, lateral bounds [1, 4], c2's derivative bounds and scalars)
+    whose upper s-bound is `slope_wiggle(n_knots, breaks)`; `breaks` is one list for all scenarios or one list per scenario.
+    The reference line is s_ref = 5 m/s * t, l_ref = 2 m, from the initial state (0, 5, 0, 2, 0, 0).  Per scenario, only
+    values that cannot move a slope break vary (scenario 0 is the unperturbed base): s_ref (after knot 0) by an offset in
+    [0, 1) m, l_ref by [-0.5, 0.5) m, the initial ds by [-0.5, 0.5) m/s and dl by [0, 0.1) m/s (the
+    dl bounds are [0, 2.5]), the lateral bounds by [-0.3, 0.3) m each.  `regions`: extra regions appended after region 0, as a list of (s_upper [N], l_lo, l_hi)."""
+    c2 = load_fixture("c2")
+    N, d = n_knots, 0.1
+    per = [list(breaks)] * B if len(breaks) == 0 or np.ndim(breaks[0]) == 0 else [list(b) for b in breaks]
+    if len(per) != B:
+        raise ValueError("one break list per scenario")
+    extra = list(regions or [])
+    R = 1 + len(extra)
+    rng = np.random.Generator(np.random.Philox(key=seed))
+    u = rng.random((B, 6))
+    u[0] = 0.5
+    u[0, 0] = u[0, 3] = 0.0
+    sb = np.zeros((B, R, N, 2))
+    lb = np.zeros((B, R, N, 2))
+    for b in range(B):
+        sb[b, 0, :, 1] = slope_wiggle(N, per[b], d)
+    lb[:, 0, :, 0] = (1.0 + np.round(0.6 * u[:, 4] - 0.3, 2))[:, None]
+    lb[:, 0, :, 1] = (4.0 + np.round(0.6 * u[:, 5] - 0.3, 2))[:, None]
+    for r, (s_up, l_lo, l_hi) in enumerate(extra, start=1):
+        sb[:, r, :, 1] = np.asarray(s_up)[None, :]
+        lb[:, r, :, 0], lb[:, r, :, 1] = l_lo, l_hi
+    t = np.arange(N) * d
+    s_ref = np.tile(5.0 * t, (B, 1))
+    s_ref[:, 1:] += np.round(u[:, 0], 2)[:, None]
+    l_ref = np.tile(2.0 + np.round(u[:, 1] - 0.5, 2)[:, None], (1, N))
+    init = np.tile(np.array([0.0, 5.0, 0.0, 2.0, 0.0, 0.0]), (B, 1))
+    init[:, 1] += u[:, 2] - 0.5
+    init[:, 4] += 0.1 * u[:, 3]
+    rep = lambda a: np.ascontiguousarray(np.broadcast_to(a, (B,) + a.shape))  # noqa: E731
+    return ScenarioBatch(N, R, d, sb, lb, rep(np.tile([0.0, 10.0], (N, 1))), rep(np.tile([0.0, 2.5], (N, 1))), s_ref, l_ref,
+                         init, rep(c2.scalars))
+
+
+def segment_ladder(K: int, B: int, seed: int = 20231021) -> ScenarioBatch:
+    """B scenarios that all have exactly K corridor segments, for every K from 1 to 34 (K <= 32 solvable with k_max = 32,
+    K >= 33 reported as too many segments), in both variants; they share one KKT structure (same K, same segment
+    durations) and differ in values only (see `wiggle_batch`).
+      K <= 25:  N = 10 K + 1 knots and no slope break: one pre-split cube of K seconds, split into K one-second segments.
+      K >= 26:  N = 256 (without breaks: 25 one-second segments and a 0.5 s one) and 2 (K - 26) slope breaks at knots 15,
+                30, 45, ...: each pair of breaks cuts 3 s of road into two 1.5 s cubes, split into 1.0 + 0.5 s each, i.e.
+                four segments where there were three.
+    Segments are never shorter than 0.5 s: closely spaced breaks give ill-conditioned QPs whose solved / failed class the
+    reference does not pin (helpers.decided_classes)."""
+    N, breaks = ladder_shape(K)
+    return wiggle_batch(N, breaks, B, seed=seed + K)
+
+
 def random_obstacles(B: int, max_obs: int = 3, seed: int = 20230606):
     """Obstacle sets for the upstream bound generator (spectral_bounds_device): [B, max_obs, 6] = (s, l, t0, vel_s, vel_l,
     horizon) and n_obs [B], with the value ranges of the reference's two-car scene (src/cart_frenet.py:1536-1546): lateral

@@ -349,6 +349,7 @@ def assert_batch_parity(got, ref, label="", need_verified_frac=0.0, ref0=None, m
 
     # ---- scenarios both sides solve but without a KKT proof on one side: the raw ADMM iterates must agree
     compared_iter = 0
+    compared_any = both.copy()
     if got0 is not None and have_ref0:
         assert np.array_equal(got0.K, got.K) and np.array_equal(got0.iters, got.iters), "%s: polish changed the iteration" % label
         same = got0.ok() & ok_ref & ~corridor_fail & (got0.iters == ref0["iters"]) & (ref0["iters"] < cap)
@@ -362,10 +363,12 @@ def assert_batch_parity(got, ref, label="", need_verified_frac=0.0, ref0=None, m
             if e > 1.0:
                 bad.append(int(b))
         compared_iter = int(same.sum())
+        compared_any |= same
         stats.update(compared_iterate=compared_iter, iterate_max_err_in_tol_units=worst, iterate_outliers=len(bad))
         assert len(bad) <= max(1, int(0.01 * compared_iter)), "%s: ADMM iterate differs from the reference-settings oracle's at %s" % (label, bad[:8])
     both_solved = got.ok() & (ref["status"] <= 1) & ok_ref
     stats["both_solved"] = int(both_solved.sum())
+    stats["compared_any"] = int(compared_any.sum())  # distinct scenarios compared numerically, by optimum, by iterate or both
     if both_solved.any():
         assert both.sum() + compared_iter > 0, "%s: %d scenarios solved on both sides and none compared numerically" % (label, both_solved.sum())
     fail = ~got.ok()
