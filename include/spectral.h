@@ -21,6 +21,9 @@
  *   spectral_topk_device()      new: the k best trajectories of a sweep (spectral_sweep_topk across GPUs).
  *   spectral_eval_device()      new: solved trajectories at caller-chosen times (the sampler of Optimize, :1351-1390, on
  *                               any time grid, with jerk).
+ *   spectral_certify_device()   new: how far each returned trajectory is from satisfying the constraint rows of its QP
+ *                               (the rows of CalculateAffineConstraint, :779-1129), and its cost with uncertified
+ *                               scenarios set to the failure sentinel.
  *   SpectralCube                struct Cube, include/btrapz/cube_type.h:2-24 (same 112-byte layout).
  *   SpectralParams              struct Params, include/btrapz/py_cpp_.h:6-21 (same 88-byte layout).
  */
@@ -254,6 +257,44 @@ int spectral_frenet_to_cartesian_device(spectral_handle_t *h, long long n, const
  *   other than 0 or 1. */
 int spectral_eval_device(spectral_handle_t *h, int B, const SpectralOutputs *dev_out, int T, const double *times_dev,
                          int times_stride, double *states_dev, double *jerk_dev, double *horizon_dev, void *cuda_stream);
+
+/* Feasibility certificate of solved trajectories (device buffers, enqueued on cuda_stream, no synchronisation, no handle
+ * scratch, one kernel launch).  It certifies PRIMAL FEASIBILITY of the returned control points for the QP they were solved
+ * for, to within tol: every row l <= A x <= u of that QP, assembled by the solver's own code.  It does not certify
+ * optimality.  Why it is needed: the ranking entry points (argmin, top-k, sweep) rank on a_cost alone, and a scenario with
+ * status SOLVED_INACCURATE (accepted as the reference does, solve_3d.cc:1253) may carry a trajectory that leaves its
+ * corridor -- on infeasible problems OSQP can stop "solved inaccurate" at max_iter.
+ *   dev_in        ds_bounds, dl_bounds, init and scalars are required; the other fields are ignored and may be NULL (no row
+ *                 depends on the weights or the references).  inputs_stride 1: B scenarios in the layout of
+ *                 spectral_solve_batch*; 0: one scenario for every b (the layout of spectral_solve_weights*).
+ *   dev_out       K, segs, ctrl and status of B scenarios, in the handle's k_max layout; a_cost too when cost_dev is given.
+ *   tol           host array, one acceptable violation per row family, each >= 0.
+ *   viol_dev      [B][2][SPECTRAL_CERT_FAMILIES] (axis s = 0, l = 1; family): the largest max(l - Ax, Ax - u, 0) over the
+ *                 axis' rows of that family, or NULL.
+ *   cost_dev      [B]: a_cost[b] when every entry of viol is <= tol[family] (a NaN entry never is), else SPECTRAL_FAIL_COST;
+ *                 or NULL (not both outputs).  Feed it to spectral_argmin_device / spectral_topk_device, or point
+ *                 dev_out.a_cost at it for spectral_sweep_argmin / spectral_sweep_topk: the best FEASIBLE trajectories.
+ * Row families, in the QP's own row units (these are the rows as assembled, not SI units: dividing by t_k or t_k^2 would be
+ * meaningless on CorridorSplit's slivers, t_k ~ 1e-15 s).  Segment k of duration t_k, control points c_0..c_5 of one axis:
+ *   position      t_k c_i in the corridor (6 rows); the initial position t_0 c_0 = s(0), and the joints
+ *                 t_k c_{k,0} - t_{k-1} c_{k-1,5} = 0
+ *   velocity      5 (c_{i+1} - c_i) in [ds_lo, ds_hi] over the segment's knots (s) / dl_bounds (l) (5 rows); the initial
+ *                 velocity and the velocity joints
+ *   acceleration  20 D2c_i = acc x t_k in [lo t_k, hi t_k] (4 rows); the initial acceleration x t_0, and the joints
+ *                 t_k D2c_{k-1,3} - t_{k-1} D2c_{k,0} = 0 (acc x t_{k-1} t_k / 20)
+ *   jerk          60 D3c_i = jerk x t_k^2 in [lo t_k^2, hi t_k^2] (3 rows)
+ * NaN entries and SPECTRAL_FAIL_COST: a scenario that is not certifiable -- status other than SOLVED / SOLVED_INACCURATE,
+ *   K outside [1, k_max], or a segment with beg_t / end_t outside [0, N - 1] or beg_t > end_t (checked before any read of
+ *   ds_bounds, since segs may come from the caller).  A NaN or infinite control point makes its axis' entries NaN.
+ * The l-axis velocity rows read dl_bounds at knots 0..4 (by control index, as the reference does, solve_3d.cc:1003), so for
+ *   N < 5 they read past the scenario's [N][2] slab, as the solver does.
+ * B is limited only by int (not by the handle's max_batch).
+ * SPECTRAL_ERR_INVALID: null handle; variant; a required pointer NULL; both outputs NULL; B < 1; N outside [3, n_max];
+ *   inputs_stride other than 0 or 1; tol NULL, or an entry negative or NaN. */
+#define SPECTRAL_CERT_FAMILIES 4 /* position, velocity, acceleration, jerk (rows as assembled, see above) */
+int spectral_certify_device(spectral_handle_t *h, int variant, int B, int N, const SpectralInputs *dev_in, int inputs_stride,
+                            const SpectralOutputs *dev_out, const double tol[SPECTRAL_CERT_FAMILIES], double *viol_dev,
+                            double *cost_dev, void *cuda_stream);
 
 /* Multi-GPU sweep (SURVEY.md 8e): scenarios are sharded over ranks (one handle = one GPU = one rank); the ONLY exchange is
  * the best trajectory: local arg-min (k_argmin) -> NCCL all-gather of one 16-byte (cost, global index) record per rank ->

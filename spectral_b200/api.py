@@ -35,6 +35,7 @@ NUM_KERNELS = 6
 NUM_CLASSES = 5
 NUM_WORK = 12
 TOPK_MAX = 1024   # SPECTRAL_TOPK_MAX
+CERT_FAMILIES = ("position", "velocity", "acceleration", "jerk")   # SPECTRAL_CERT_FAMILIES, the last axis of certify_device's viol
 KERNEL_NAMES = ("tables", "corridor", "classify", "qp", "finalize", "argmin")
 
 CUBE_DTYPE = np.dtype([
@@ -147,6 +148,9 @@ def load_library() -> ctypes.CDLL:
                                         ctypes.c_void_p, ctypes.POINTER(ctypes.c_int), ctypes.c_void_p]
     lib.spectral_eval_device.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(SpectralOutputs), ctypes.c_int, ctypes.c_void_p,
                                          ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
+    lib.spectral_certify_device.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.POINTER(SpectralInputs),
+                                            ctypes.c_int, ctypes.POINTER(SpectralOutputs), _dp, ctypes.c_void_p, ctypes.c_void_p,
+                                            ctypes.c_void_p]
     _lib = lib
     return lib
 
@@ -580,6 +584,54 @@ class SpectralPlanner:
                                                    ctypes.c_void_p(jk.data_ptr()) if jk is not None else None,
                                                    ctypes.c_void_p(horizon.data_ptr()), ctypes.c_void_p(stream)))
         return states, jk, horizon
+
+    # ---- feasibility certificate of solved trajectories (spectral_certify_device)
+    def certify_device(self, variant, n_knots: int, inputs: dict, outputs: dict, tol, shared_inputs: bool = False,
+                       B: Optional[int] = None, stream: Optional[int] = None):
+        """How far each trajectory of `outputs` (K, segs, ctrl, status, a_cost) is from satisfying the constraint rows of the
+        QP it was solved for, from `inputs` (ds_bounds, dl_bounds, init, scalars: the solve's inputs; shared_inputs=True: the
+        one scenario of a solve_weights run).  `tol`: the acceptable violation, one float or one per row family (CERT_FAMILIES),
+        in the QP's row units (include/spectral.h); there is no default.  Returns (viol float64 [B, 2, 4]: the largest violation
+        per axis (s, l) and family, NaN for scenarios that cannot be certified; cost float64 [B]: a_cost where every entry is
+        <= tol, FAIL_COST elsewhere), enqueued on `stream` (default: the current torch stream).  Primal feasibility only, not
+        optimality.  `cost` feeds topk_device / argmin_device, or sweep_topk / sweep_argmin as outputs["a_cost"]."""
+        import torch
+        B = int(outputs["K"].numel()) if B is None else int(B)
+        if B < 1:
+            raise ValueError("B must be positive")
+        n_knots = int(n_knots)
+        if not 3 <= n_knots <= self.n_max:
+            raise ValueError("n_knots must be in [3, %d]" % self.n_max)
+        tol = np.broadcast_to(np.asarray(tol, dtype=np.float64), (len(CERT_FAMILIES),)).copy()
+        if not (tol >= 0.0).all():
+            raise ValueError("tol must be non-negative, got %s" % tol)
+        self._check_tensor(outputs["K"], "K", torch.int32, B)
+        self._check_tensor(outputs["status"], "status", torch.int32, B)
+        self._check_tensor(outputs["segs"], "segs", torch.uint8, B, self.k_max * 112)
+        self._check_tensor(outputs["ctrl"], "ctrl", torch.float64, B, 12 * self.k_max)
+        self._check_tensor(outputs["a_cost"], "a_cost", torch.float64, B)
+        Bi = 1 if shared_inputs else B
+        for name, row in (("ds_bounds", 2 * n_knots), ("dl_bounds", 2 * n_knots), ("init", 6), ("scalars", 10)):
+            self._check_tensor(inputs[name], name, torch.float64, Bi, row)
+        dev = outputs["ctrl"].device
+        viol = torch.empty(B, 2, len(CERT_FAMILIES), dtype=torch.float64, device=dev)
+        cost = torch.empty(B, dtype=torch.float64, device=dev)
+        inp = SpectralInputs()
+        for name in ("ds_bounds", "dl_bounds", "init", "scalars"):
+            setattr(inp, name, ctypes.cast(ctypes.c_void_p(inputs[name].data_ptr()), _dp))
+        out = SpectralOutputs()
+        out.K = ctypes.cast(ctypes.c_void_p(outputs["K"].data_ptr()), _ip)
+        out.status = ctypes.cast(ctypes.c_void_p(outputs["status"].data_ptr()), _ip)
+        out.segs = outputs["segs"].data_ptr()
+        out.ctrl = ctypes.cast(ctypes.c_void_p(outputs["ctrl"].data_ptr()), _dp)
+        out.a_cost = ctypes.cast(ctypes.c_void_p(outputs["a_cost"].data_ptr()), _dp)
+        if stream is None:
+            stream = torch.cuda.current_stream(dev).cuda_stream
+        self._check(self._lib.spectral_certify_device(self._h, VARIANT_ID[variant], B, n_knots, ctypes.byref(inp),
+                                                      0 if shared_inputs else 1, ctypes.byref(out), _d(tol),
+                                                      ctypes.c_void_p(viol.data_ptr()), ctypes.c_void_p(cost.data_ptr()),
+                                                      ctypes.c_void_p(stream)))
+        return viol, cost
 
     def launch_count(self) -> int:
         return int(self._lib.spectral_launch_count(self._h))

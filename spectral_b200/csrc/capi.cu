@@ -15,6 +15,7 @@
 
 #include "common.cuh"
 #include "bounds.cuh"
+#include "certify.cuh"
 #include "corridor.cuh"
 #include "downstream.cuh"
 #include "eval.cuh"
@@ -994,6 +995,45 @@ extern "C" int spectral_eval_device(spectral_handle_t *h, int B, const SpectralO
   const EvalArgs a{B, T, h->k_max, times_stride, dev_out->K, dev_out->status, dev_out->segs, dev_out->ctrl, times_dev};
   const long long want = ((long long)B * T + EVAL_THREADS - 1) / EVAL_THREADS, cap = 8LL * h->sm_count;
   k_eval<<<(unsigned)(want < cap ? want : cap), EVAL_THREADS, 0, (cudaStream_t)cuda_stream>>>(a, states_dev, jerk_dev, horizon_dev);
+  h->launches++;
+  CK(cudaGetLastError());
+  return SPECTRAL_SUCCESS;
+}
+
+// ------------------------------------------------------------------ feasibility certificate (certify.cuh)
+// One warp per scenario, grid-stride over B.
+#define CERT_WARPS 8
+__global__ void __launch_bounds__(32 * CERT_WARPS) k_certify(const CertArgs a) {
+  const int lane = threadIdx.x & 31;
+  const long long stride = (long long)gridDim.x * CERT_WARPS;
+  for (long long b = (long long)blockIdx.x * CERT_WARPS + (threadIdx.x >> 5); b < a.B; b += stride) certify_warp(a, (int)b, lane);
+}
+
+extern "C" int spectral_certify_device(spectral_handle_t *h, int variant, int B, int N, const SpectralInputs *dev_in, int inputs_stride,
+                                       const SpectralOutputs *dev_out, const double tol[SPECTRAL_CERT_FAMILIES], double *viol_dev,
+                                       double *cost_dev, void *cuda_stream) {
+  if (!h) return SPECTRAL_ERR_INVALID;
+  if (variant != SPECTRAL_TRP && variant != SPECTRAL_CUB) return fail(h, SPECTRAL_ERR_INVALID, "certify: variant");
+  if (!dev_in || !dev_in->ds_bounds || !dev_in->dl_bounds || !dev_in->init || !dev_in->scalars)
+    return fail(h, SPECTRAL_ERR_INVALID, "certify: ds_bounds/dl_bounds/init/scalars are required");
+  if (!dev_out || !dev_out->K || !dev_out->segs || !dev_out->ctrl || !dev_out->status)
+    return fail(h, SPECTRAL_ERR_INVALID, "certify: K/segs/ctrl/status are required");
+  if (!viol_dev && !cost_dev) return fail(h, SPECTRAL_ERR_INVALID, "certify: viol and cost are both NULL");
+  if (cost_dev && !dev_out->a_cost) return fail(h, SPECTRAL_ERR_INVALID, "certify: cost needs a_cost");
+  if (B < 1) return fail(h, SPECTRAL_ERR_INVALID, "certify: B must be positive");
+  if (N < 3 || N > h->n_max) return fail(h, SPECTRAL_ERR_INVALID, "certify: N outside [3, n_max]");
+  if (inputs_stride != 0 && inputs_stride != 1) return fail(h, SPECTRAL_ERR_INVALID, "certify: inputs_stride must be 0 or 1");
+  if (!tol) return fail(h, SPECTRAL_ERR_INVALID, "certify: NULL tol");
+  static_assert(SPECTRAL_CERT_FAMILIES == SP_CERT_FAMILIES, "include/spectral.h");
+  CertArgs a{B, N, h->k_max, variant, inputs_stride, dev_in->ds_bounds, dev_in->dl_bounds, dev_in->init, dev_in->scalars,
+             dev_out->K, dev_out->status, dev_out->segs, dev_out->ctrl, dev_out->a_cost, {}, viol_dev, cost_dev};
+  for (int f = 0; f < SP_CERT_FAMILIES; f++) {
+    if (!(tol[f] >= 0.0)) return fail(h, SPECTRAL_ERR_INVALID, "certify: tol must be non-negative (and not NaN)");
+    a.tol[f] = tol[f];
+  }
+  CK(cudaSetDevice(h->device));
+  const long long want = ((long long)B + CERT_WARPS - 1) / CERT_WARPS, cap = 8LL * h->sm_count;
+  k_certify<<<(unsigned)(want < cap ? want : cap), 32 * CERT_WARPS, 0, (cudaStream_t)cuda_stream>>>(a);
   h->launches++;
   CK(cudaGetLastError());
   return SPECTRAL_SUCCESS;

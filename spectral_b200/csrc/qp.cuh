@@ -468,36 +468,20 @@ struct QpLane {
   int pre;  // interval pre-check: the scenario's corridor is provably empty (SpectralOptions::infeasibility_precheck)
 };
 
-// K3 + Ruiz equilibration + per-row rho: fills the shared-memory slots L, U, W (= 0), P, RHO of this
-// lane and the lane state.  `lane` is the shared-memory column of this lane (slot * STR + lane).
-template <int LPA, int STR, int JW>
-SP_DEV void qp_setup(const QpArgs &a, int ap, bool have, int seg, int lane, double *sm, QpLane &Q, double *xch = nullptr) {
-  const int b = have ? a.list[ap >> 1] : 0;
-  const int axis = ap & 1;
-  const int K = have ? a.K[b] : 0;
-  const bool active = have && seg < K;
-  const bool first = seg == 0, last = seg == K - 1;
-  const int kmaxw = sp_group_max_i(K, 32);
-  const SpOptionsDev &o = a.opt;
-  const int N = a.N;
-  const double delta = a.delta;
-
-  // ---------------- K3: assemble this lane's rows ----------------
-  SpectralCube cube;
-  if (active) cube = a.segs[(size_t)b * a.k_max + seg];
-  else { cube.beg_t = 0; cube.end_t = 0; cube.t = 1.0; cube.beg_l = 0; cube.end_l = 0; cube.upp_skew = 0; cube.upp_bias = 0;
-         cube.down_skew = 0; cube.down_bias = 0; cube.l_upp_skew = 0; cube.l_upp_bias = 0; cube.l_down_skew = 0; cube.l_down_bias = 0; }
-  const double t = cube.t;
-  double tp = sp_shfl_up(t, 1, LPA), tn = sp_shfl_down(t, 1, LPA);
-  if (first) tp = 1.0;
-  if (last || !active) tn = 1.0;
-  const size_t bi = (size_t)b * a.in_stride;  // input scenario of this lane
-  const double *sc = a.scalars + 10 * bi;
-  const double *wv = a.weights + (size_t)(a.wstride ? b : 0) * 10;
-  const double *ref = (axis == 0 ? a.s_ref : a.l_ref) + bi * N;
-  const double *ini = a.init + 6 * bi + 3 * axis;
+// K3 rows: the bounds lo <= A x <= hi of the 21 rows of segment `cube` (row_coef / apply_A give A), in the QP's own row
+// units -- the one assembly of the QP's rows, shared by the solver (qp_setup) and the certificate (certify.cuh).
+//   rows  0..5   position: t c_i                           rows  6..10  velocity: 5 (c_{i+1} - c_i)
+//   rows 11..14  acceleration x t: 20 D2c_i               rows 15..17  jerk x t^2: 60 D3c_i
+//   rows 18..20  first segment: initial (s, ds, dds t) equalities; later segments: continuity of position, velocity and
+//                acceleration with the previous segment (equalities = 0)
+// `a` (QpArgs, CertArgs) gives variant, ds_bounds and dl_bounds; bi is the input scenario, t = cube.t, sc its scalars[10],
+// ini its init + 3 axis.  The s axis reads ds_bounds[bi][beg_t .. end_t] of an active segment; the l axis reads
+// dl_bounds[bi] at knots 0..4 (control index, :1003) whatever N is.  (The arguments keep the solver's loads where they
+// were before this function was split out of qp_setup, so the solver kernels compile to the same code.)
+template <class Args>
+SP_DEV void qp_rows(const Args &a, int axis, bool active, bool first, const SpectralCube &cube, double t, size_t bi, int N,
+                    const double *sc, const double *ini, double lo[QP_ROWS], double hi[QP_ROWS]) {
   const double invm[6] = {SP_INVM1_0, SP_INVM1_1, SP_INVM1_2, SP_INVM1_3, SP_INVM1_4, SP_INVM1_5};
-  double lo[QP_ROWS], hi[QP_ROWS];
   // containment rows (solve_3d.cc:823-832, :961-977; cuboid_3d.cc:677-697, :826-827)
   if (axis == 0) {
     if (a.variant == SPECTRAL_CUB) {
@@ -565,6 +549,38 @@ SP_DEV void qp_setup(const QpArgs &a, int ap, bool have, int seg, int lane, doub
   } else {
     lo[18] = hi[18] = 0.0; lo[19] = hi[19] = 0.0; lo[20] = hi[20] = 0.0;
   }
+}
+
+// K3 + Ruiz equilibration + per-row rho: fills the shared-memory slots L, U, W (= 0), P, RHO of this
+// lane and the lane state.  `lane` is the shared-memory column of this lane (slot * STR + lane).
+template <int LPA, int STR, int JW>
+SP_DEV void qp_setup(const QpArgs &a, int ap, bool have, int seg, int lane, double *sm, QpLane &Q, double *xch = nullptr) {
+  const int b = have ? a.list[ap >> 1] : 0;
+  const int axis = ap & 1;
+  const int K = have ? a.K[b] : 0;
+  const bool active = have && seg < K;
+  const bool first = seg == 0, last = seg == K - 1;
+  const int kmaxw = sp_group_max_i(K, 32);
+  const SpOptionsDev &o = a.opt;
+  const int N = a.N;
+  const double delta = a.delta;
+
+  // ---------------- K3: assemble this lane's rows ----------------
+  SpectralCube cube;
+  if (active) cube = a.segs[(size_t)b * a.k_max + seg];
+  else { cube.beg_t = 0; cube.end_t = 0; cube.t = 1.0; cube.beg_l = 0; cube.end_l = 0; cube.upp_skew = 0; cube.upp_bias = 0;
+         cube.down_skew = 0; cube.down_bias = 0; cube.l_upp_skew = 0; cube.l_upp_bias = 0; cube.l_down_skew = 0; cube.l_down_bias = 0; }
+  const double t = cube.t;
+  double tp = sp_shfl_up(t, 1, LPA), tn = sp_shfl_down(t, 1, LPA);
+  if (first) tp = 1.0;
+  if (last || !active) tn = 1.0;
+  const size_t bi = (size_t)b * a.in_stride;  // input scenario of this lane
+  const double *sc = a.scalars + 10 * bi;
+  const double *wv = a.weights + (size_t)(a.wstride ? b : 0) * 10;
+  const double *ref = (axis == 0 ? a.s_ref : a.l_ref) + bi * N;
+  const double *ini = a.init + 6 * bi + 3 * axis;
+  double lo[QP_ROWS], hi[QP_ROWS];
+  qp_rows(a, axis, active, first, cube, t, bi, N, sc, ini, lo, hi);
   // optional interval pre-check (include/spectral.h: infeasibility_precheck): necessary conditions of feasibility on the
   // raw rows -- no row with l > u; the position intervals of consecutive segments meet at their joint (row 5 of segment
   // k - 1 and row 0 of segment k bound the same quantity, t_{k-1} c_{k-1,5} = t_k c_{k,0}); the initial state lies inside
