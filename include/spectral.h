@@ -160,7 +160,9 @@ typedef struct spectral_handle spectral_handle_t;
 
 void spectral_default_options(SpectralOptions *opt);
 
-/* device: CUDA ordinal.  Capacities: scenarios per call, knots, regions, segments (k_max <= 32). */
+/* device: CUDA ordinal.  Capacities: scenarios per call, knots, regions, segments (k_max <= 32).
+ * A failed spectral_create may leave a handle in *out, so that spectral_last_error can explain the failure; that handle
+ * must then be passed to spectral_destroy. */
 int spectral_create(int device, int max_batch, int n_max, int r_max, int k_max, spectral_handle_t **out);
 int spectral_destroy(spectral_handle_t *h);
 const char *spectral_last_error(const spectral_handle_t *h);
@@ -297,12 +299,17 @@ int spectral_certify_device(spectral_handle_t *h, int variant, int B, int N, con
                             double *cost_dev, void *cuda_stream);
 
 /* Multi-GPU sweep (SURVEY.md 8e): scenarios are sharded over ranks (one handle = one GPU = one rank); the ONLY exchange is
- * the best trajectory: local arg-min (k_argmin) -> NCCL all-gather of one 16-byte (cost, global index) record per rank ->
- * NCCL broadcast of the winner's (K, segments, control points) from the rank that owns it.  Ties -> lowest global index;
- * failed scenarios carry 1e11 (the reference's sentinel, trp_wrapper.cpp:199).  The library loads libnccl.so.2 at run time.
+ * the best trajectory.  spectral_sweep_argmin is spectral_sweep_topk (below) with k = 1: local top-1 -> NCCL all-gather of one
+ * 16-byte (cost, global index) record per rank -> the same select over those records -> the owning rank packs the winner's
+ * (K, segments, control points) into a zeroed buffer, which one NCCL all-reduce hands to every rank.  Ties -> lowest global
+ * index; failed scenarios carry 1e11 (the reference's sentinel, trp_wrapper.cpp:199).  The library loads libnccl.so.2 at run
+ * time.
  *   spectral_comm_unique_id  rank 0 makes the id (ncclGetUniqueId); the caller ships it to the other ranks by any means
  *   spectral_comm_init       every rank, same id (ncclCommInitRank on the handle's device); nranks = 1 needs no NCCL
- *   spectral_sweep_argmin    collective over all ranks; enqueued on cuda_stream, synchronises it, fills *winner on EVERY rank */
+ *   spectral_sweep_argmin    collective over all ranks; enqueued on cuda_stream, synchronises it, fills *winner on EVERY rank.
+ *                            B_local >= 1; a negative index_offset is rejected (SPECTRAL_ERR_INVALID).  A sweep whose every
+ *                            cost is above 1e300 or NaN returns its first entry in top-k order: a real index, with its own
+ *                            K, segments and control points.  segs and ctrl beyond K are zero. */
 typedef struct {
   double cost;         /* a_cost of the best scenario (1e11: every scenario of the sweep failed) */
   long long index;     /* its global index = index_offset of the owning rank + local index */
@@ -332,7 +339,7 @@ int spectral_sweep_argmin(spectral_handle_t *h, int B_local, const SpectralOutpu
  *                       <= k selected entries and one sort of those (DESIGN.md 3.4).  Scratch belongs to the handle, is
  *                       allocated on first use and does not grow with B; as for spectral_argmin_device, calls on one handle
  *                       must not overlap in time (one stream at a time, or ordered by events).
- * spectral_sweep_topk   collective, like spectral_sweep_argmin: local top-k -> NCCL all-gather of k 16-byte (cost, global index)
+ * spectral_sweep_topk   collective over all ranks: local top-k -> NCCL all-gather of k 16-byte (cost, global index)
  *                       records per rank -> the same select over the nranks x k records -> each rank packs the payloads
  *                       (K, segments, control points) of the winners it owns into a zeroed [k] buffer, which one NCCL
  *                       all-reduce (sum over bytes: exactly one rank writes each byte) hands to every rank.  Fills

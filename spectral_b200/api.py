@@ -204,6 +204,8 @@ class SpectralPlanner:
         rc = self._lib.spectral_create(device, max_batch, n_max, r_max, k_max, ctypes.byref(self._h))
         if rc != 0:
             msg = self._lib.spectral_last_error(self._h).decode() if self._h else "no CUDA device"
+            if self._h:
+                self._lib.spectral_destroy(self._h)
             self._h = ctypes.c_void_p()
             raise RuntimeError("spectral_create failed (rc=%d): %s -- libspectral has no CPU path" % (rc, msg))
 

@@ -11,6 +11,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <string>
 
 #include "common.cuh"
@@ -323,9 +324,53 @@ __global__ void k_fp64_peak(double *out, int iters) {
 }
 
 // ------------------------------------------------------------------ handle
-struct DevBuf {
-  void *p = nullptr;
-  size_t bytes = 0;
+// Every device and page-locked buffer of a handle has one owner; kernels and launch helpers get .get().
+struct CudaFree { void operator()(void *p) const { cudaFree(p); } };
+struct CudaFreeHost { void operator()(void *p) const { cudaFreeHost(p); } };
+template <typename T> using DevPtr = std::unique_ptr<T, CudaFree>;
+template <typename T> using HostPtr = std::unique_ptr<T, CudaFreeHost>;
+
+// `p` owns the new buffer only when the allocation succeeded (it is empty otherwise)
+template <typename T> static cudaError_t cuda_alloc(DevPtr<T> &p, size_t bytes) {
+  void *raw = nullptr;
+  const cudaError_t e = cudaMalloc(&raw, bytes);
+  p.reset(e == cudaSuccess ? static_cast<T *>(raw) : nullptr);
+  return e;
+}
+template <typename T> static cudaError_t cuda_alloc(HostPtr<T> &p, size_t bytes) {
+  void *raw = nullptr;
+  const cudaError_t e = cudaHostAlloc(&raw, bytes, cudaHostAllocDefault);
+  p.reset(e == cudaSuccess ? static_cast<T *>(raw) : nullptr);
+  return e;
+}
+
+// Buffers allocated on first use come in groups.  A group is built in a local and moved into the handle in one step once
+// every allocation in it has succeeded, so a handle never holds part of a group: any one owner of it tells whether it is there.
+struct QpsBuffers {  // shared-KKT path
+  DevPtr<unsigned long long> keys, keys2;
+  DevPtr<int> ids, ids2, tmp /* head, gstart, flag, tidx: 4 x B */, tile /* start, count: 2 x B */, leader, misc /* n_tiles, tile_next */, st;
+  DevPtr<QpsTileBlk> blk;
+  DevPtr<double> lu, qv, w, x, fs;
+  DevPtr<unsigned char> cub;
+  size_t cub_bytes = 0;
+};
+struct TopkBuffers {  // select scratch (topk.cuh), independent of B
+  DevPtr<unsigned> hist, block_ties;
+  DevPtr<TopkState> st;
+  DevPtr<tk_u64> ck, ci;
+  DevPtr<double> cc;
+};
+struct SweepBuffers {  // sweep exchange, sized by k and the number of ranks, never by the batch
+  DevPtr<double> rec;                // (2 + ranks) x cap 16-byte records: local, merged, gathered
+  DevPtr<unsigned char> pay;         // [cap][kPayBytes] winner payloads
+  HostPtr<unsigned char> host_pay;   // the same, page-locked host copy
+  HostPtr<double> host_rec;          // [cap] merged records, page-locked host copy
+  int cap = 0, ranks = 0;
+};
+struct HostPathBuffers {  // device mirrors of the host-buffer entry point's outputs, [max_batch]
+  DevPtr<int> K, status, iters, flags, npts;
+  DevPtr<SpectralCube> segs;
+  DevPtr<double> ctrl, obj, cost;
 };
 
 struct spectral_handle {
@@ -340,41 +385,22 @@ struct spectral_handle {
   cudaEvent_t ev[kTimingSlots][SPECTRAL_NUM_KERNELS + 1] = {};
   cudaEvent_t ev_cls[kTimingSlots][SP_NUM_CLASSES][2] = {};  // around each solver class' kernel, on that class' stream
   long long timed_calls = 0;
-  double *work = nullptr;  // device counters, see k_finalize
+  DevPtr<double> work;  // device counters, see k_finalize
   // intermediates
-  int *cstatus = nullptr, *lists = nullptr, *counts = nullptr, *axis_status = nullptr, *axis_iters = nullptr,
-      *axis_polished = nullptr;
-  double *axis_obj = nullptr, *mqm = nullptr;
-  ArgminPair *partial = nullptr;
-  unsigned *ticket = nullptr;
-  // device mirrors for the host-buffer entry point
-  double *d_in[9] = {};
-  size_t d_in_bytes[9] = {};
-  int *d_K = nullptr, *d_status = nullptr, *d_iters = nullptr, *d_flags = nullptr, *d_npts = nullptr;
-  SpectralCube *d_segs = nullptr;
-  double *d_ctrl = nullptr, *d_obj = nullptr, *d_cost = nullptr, *d_samples = nullptr, *d_lu = nullptr;
-  size_t d_samples_bytes = 0, d_lu_bytes = 0;
-  bool qp_attr_set = false;
-  // shared-KKT path (allocated on first use)
-  unsigned long long *qs_keys = nullptr, *qs_keys2 = nullptr;
-  int *qs_ids = nullptr, *qs_ids2 = nullptr, *qs_tmp = nullptr /* head, gstart, flag, tidx: 4 x B */, *qs_tile = nullptr /* start, count: 2 x B */,
-      *qs_leader = nullptr, *qs_misc = nullptr /* n_tiles, tile_next */, *qs_st = nullptr;
-  QpsTileBlk *qs_blk = nullptr;
-  double *qs_lu = nullptr, *qs_qv = nullptr, *qs_w = nullptr, *qs_x = nullptr, *qs_fs = nullptr;
-  void *qs_cub = nullptr;
-  size_t qs_cub_bytes = 0;
-  // multi-GPU exchange (spectral_comm_* / spectral_sweep_argmin)
+  DevPtr<int> cstatus, lists, counts, axis_status, axis_iters, axis_polished;
+  DevPtr<double> axis_obj, mqm;
+  DevPtr<ArgminPair> partial;
+  DevPtr<unsigned> ticket;
+  // device mirrors for the host-buffer entry point: inputs, samples and lu grow to the largest call so far
+  HostPathBuffers d_out;
+  DevPtr<double> d_in[9], d_samples, d_lu;
+  size_t d_in_bytes[9] = {}, d_samples_bytes = 0, d_lu_bytes = 0;
+  QpsBuffers qs;
+  // multi-GPU exchange (spectral_comm_* / spectral_sweep_argmin / spectral_sweep_topk)
   ncclComm_t comm = nullptr;
   int nranks = 1, rank = 0;
-  double *xg_rec = nullptr;        // [1 + nranks] (cost, index) records, 16 bytes each
-  unsigned char *xg_pay = nullptr; // winner payload
-  // top-k selection (topk.cuh), allocated on first use: select scratch (independent of B), then the sweep_topk exchange
-  TopkScratch tk{};
-  double *tk_rec = nullptr;             // (2 + nranks) x k_cap 16-byte records: local, merged, gathered
-  unsigned char *tk_pay = nullptr;      // [k_cap][kPayBytes] winner payloads (device)
-  unsigned char *tk_hostpay = nullptr;  // the same, page-locked host copy
-  double *tk_hostrec = nullptr;         // [k_cap] merged records, page-locked host copy
-  int tk_cap = 0, tk_cap_ranks = 0;
+  TopkBuffers tk;
+  SweepBuffers sw;
   int classes_timed = 0;    // solver classes launched per call (k_max dependent)
   int corridor_smem = 0;    // dynamic shared memory the corridor kernel is opted in for on this handle's device
 };
@@ -422,19 +448,19 @@ extern "C" int spectral_create(int device, int max_batch, int n_max, int r_max, 
   CK(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
   for (auto &e : h->ev_join) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
   const size_t B = (size_t)max_batch;
-  CK(cudaMalloc(&h->cstatus, B * 4));
-  CK(cudaMalloc(&h->lists, SP_NUM_CLASSES * B * 4));
-  CK(cudaMalloc(&h->counts, 4 * 2 * SP_NUM_CLASSES));  // [0, NC): list lengths, [NC, 2 NC): queue heads of the persistent kernels
-  CK(cudaMalloc(&h->axis_status, 2 * B * 4));
-  CK(cudaMalloc(&h->axis_iters, 2 * B * 4));
-  CK(cudaMalloc(&h->axis_polished, 2 * B * 4));
-  CK(cudaMalloc(&h->axis_obj, 2 * B * 8));
-  CK(cudaMalloc(&h->mqm, B * 2 * 84 * 8));
-  CK(cudaMalloc(&h->partial, 1024 * sizeof(ArgminPair)));
-  CK(cudaMalloc(&h->ticket, 4));
-  CK(cudaMemset(h->ticket, 0, 4));
-  CK(cudaMalloc(&h->work, SPECTRAL_NUM_WORK * 8));
-  CK(cudaMemset(h->work, 0, SPECTRAL_NUM_WORK * 8));
+  CK(cuda_alloc(h->cstatus, B * 4));
+  CK(cuda_alloc(h->lists, SP_NUM_CLASSES * B * 4));
+  CK(cuda_alloc(h->counts, 4 * 2 * SP_NUM_CLASSES));  // [0, NC): list lengths, [NC, 2 NC): queue heads of the persistent kernels
+  CK(cuda_alloc(h->axis_status, 2 * B * 4));
+  CK(cuda_alloc(h->axis_iters, 2 * B * 4));
+  CK(cuda_alloc(h->axis_polished, 2 * B * 4));
+  CK(cuda_alloc(h->axis_obj, 2 * B * 8));
+  CK(cuda_alloc(h->mqm, B * 2 * 84 * 8));
+  CK(cuda_alloc(h->partial, 1024 * sizeof(ArgminPair)));
+  CK(cuda_alloc(h->ticket, 4));
+  CK(cudaMemset(h->ticket.get(), 0, 4));
+  CK(cuda_alloc(h->work, SPECTRAL_NUM_WORK * 8));
+  CK(cudaMemset(h->work.get(), 0, SPECTRAL_NUM_WORK * 8));
   for (auto &slot : h->ev)
     for (auto &e : slot) CK(cudaEventCreate(&e));
   for (auto &slot : h->ev_cls)
@@ -446,20 +472,6 @@ extern "C" int spectral_destroy(spectral_handle_t *h) {
   if (!h) return SPECTRAL_ERR_INVALID;
   cudaSetDevice(h->device);
   if (h->comm) spectral_comm_destroy(h);
-  if (h->xg_rec) cudaFree(h->xg_rec);
-  if (h->xg_pay) cudaFree(h->xg_pay);
-  void *tkb[] = {h->tk.hist, h->tk.st, h->tk.block_ties, h->tk.ck, h->tk.ci, h->tk.cc, h->tk_rec, h->tk_pay};
-  for (void *p : tkb) if (p) cudaFree(p);
-  if (h->tk_hostpay) cudaFreeHost(h->tk_hostpay);
-  if (h->tk_hostrec) cudaFreeHost(h->tk_hostrec);
-  void *qsb[] = {h->qs_keys, h->qs_keys2, h->qs_ids, h->qs_ids2, h->qs_tmp, h->qs_tile, h->qs_leader, h->qs_misc, h->qs_st, h->qs_blk, h->qs_lu,
-                 h->qs_qv, h->qs_w, h->qs_x, h->qs_cub, h->qs_fs};
-  for (void *p : qsb) if (p) cudaFree(p);
-  void *bufs[] = {h->cstatus, h->lists, h->counts, h->axis_status, h->axis_iters, h->axis_polished, h->axis_obj, h->mqm,
-                  h->partial, h->ticket, h->work, h->d_K, h->d_status, h->d_iters, h->d_flags, h->d_npts, h->d_segs, h->d_ctrl,
-                  h->d_obj, h->d_cost, h->d_samples, h->d_lu};
-  for (void *p : bufs) if (p) cudaFree(p);
-  for (auto p : h->d_in) if (p) cudaFree(p);
   for (auto &slot : h->ev)
     for (auto &e : slot) if (e) cudaEventDestroy(e);
   for (auto &slot : h->ev_cls)
@@ -468,7 +480,7 @@ extern "C" int spectral_destroy(spectral_handle_t *h) {
   for (auto &s : h->side) if (s) cudaStreamDestroy(s);
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
   for (auto &e : h->ev_join) if (e) cudaEventDestroy(e);
-  delete h;
+  delete h;  // frees the buffers (their owners)
   return SPECTRAL_SUCCESS;
 }
 
@@ -512,8 +524,8 @@ extern "C" int spectral_get_work(spectral_handle_t *h, double work[SPECTRAL_NUM_
   if (!h || !work) return SPECTRAL_ERR_INVALID;
   CK(cudaSetDevice(h->device));
   CK(cudaDeviceSynchronize());
-  CK(cudaMemcpy(work, h->work, SPECTRAL_NUM_WORK * 8, cudaMemcpyDeviceToHost));
-  if (reset) CK(cudaMemset(h->work, 0, SPECTRAL_NUM_WORK * 8));
+  CK(cudaMemcpy(work, h->work.get(), SPECTRAL_NUM_WORK * 8, cudaMemcpyDeviceToHost));
+  if (reset) CK(cudaMemset(h->work.get(), 0, SPECTRAL_NUM_WORK * 8));
   return SPECTRAL_SUCCESS;
 }
 
@@ -539,64 +551,66 @@ static cudaError_t launch_qpa(spectral_handle *h, const QpArgs &qa, int B, cudaS
 }
 
 static int ensure_qps_buffers(spectral_handle *h) {
+  if (h->qs.keys) return SPECTRAL_SUCCESS;
   const size_t Bm = (size_t)h->max_batch, km = (size_t)h->k_max;
-  if (!h->qs_keys) {
-    CK(cudaMalloc(&h->qs_keys, Bm * 8)); CK(cudaMalloc(&h->qs_keys2, Bm * 8));
-    CK(cudaMalloc(&h->qs_ids, Bm * 4)); CK(cudaMalloc(&h->qs_ids2, Bm * 4));
-    CK(cudaMalloc(&h->qs_tmp, 4 * Bm * 4)); CK(cudaMalloc(&h->qs_tile, 2 * Bm * 4));
-    CK(cudaMalloc(&h->qs_leader, Bm * 4)); CK(cudaMalloc(&h->qs_misc, 2 * 4)); CK(cudaMalloc(&h->qs_st, 4 * Bm * 4));
-    CK(cudaMalloc(&h->qs_blk, 2 * Bm * sizeof(QpsTileBlk)));
-    CK(cudaMalloc(&h->qs_lu, Bm * 2 * km * QP_ROWS * 2 * 8));
-    CK(cudaMalloc(&h->qs_fs, (size_t)2 * h->sm_count * QPS_FS_DOUBLES * 8));
-    CK(cudaMalloc(&h->qs_qv, Bm * 2 * 8 * 6 * 8)); CK(cudaMalloc(&h->qs_w, Bm * 2 * 8 * QP_ROWS * 8)); CK(cudaMalloc(&h->qs_x, Bm * 2 * QPS_N * 8));
-    size_t t1 = 0, t2 = 0, t3 = 0;
-    cub::DeviceRadixSort::SortPairs(nullptr, t1, h->qs_keys, h->qs_keys2, h->qs_ids, h->qs_ids2, h->max_batch);
-    cub::DeviceScan::InclusiveScan(nullptr, t2, h->qs_tmp, h->qs_tmp, cub::Max(), h->max_batch);
-    cub::DeviceScan::ExclusiveSum(nullptr, t3, h->qs_tmp, h->qs_tmp, h->max_batch);
-    h->qs_cub_bytes = t1 > t2 ? (t1 > t3 ? t1 : t3) : (t2 > t3 ? t2 : t3);
-    CK(cudaMalloc(&h->qs_cub, h->qs_cub_bytes));
-  }
+  QpsBuffers q;
+  CK(cuda_alloc(q.keys, Bm * 8)); CK(cuda_alloc(q.keys2, Bm * 8));
+  CK(cuda_alloc(q.ids, Bm * 4)); CK(cuda_alloc(q.ids2, Bm * 4));
+  CK(cuda_alloc(q.tmp, 4 * Bm * 4)); CK(cuda_alloc(q.tile, 2 * Bm * 4));
+  CK(cuda_alloc(q.leader, Bm * 4)); CK(cuda_alloc(q.misc, 2 * 4)); CK(cuda_alloc(q.st, 4 * Bm * 4));
+  CK(cuda_alloc(q.blk, 2 * Bm * sizeof(QpsTileBlk)));
+  CK(cuda_alloc(q.lu, Bm * 2 * km * QP_ROWS * 2 * 8));
+  CK(cuda_alloc(q.fs, (size_t)2 * h->sm_count * QPS_FS_DOUBLES * 8));
+  CK(cuda_alloc(q.qv, Bm * 2 * 8 * 6 * 8)); CK(cuda_alloc(q.w, Bm * 2 * 8 * QP_ROWS * 8)); CK(cuda_alloc(q.x, Bm * 2 * QPS_N * 8));
+  size_t t1 = 0, t2 = 0, t3 = 0;
+  cub::DeviceRadixSort::SortPairs(nullptr, t1, q.keys.get(), q.keys2.get(), q.ids.get(), q.ids2.get(), h->max_batch);
+  cub::DeviceScan::InclusiveScan(nullptr, t2, q.tmp.get(), q.tmp.get(), cub::Max(), h->max_batch);
+  cub::DeviceScan::ExclusiveSum(nullptr, t3, q.tmp.get(), q.tmp.get(), h->max_batch);
+  q.cub_bytes = t1 > t2 ? (t1 > t3 ? t1 : t3) : (t2 > t3 ? t2 : t3);
+  CK(cuda_alloc(q.cub, q.cub_bytes));
+  h->qs = std::move(q);
   return SPECTRAL_SUCCESS;
 }
 // Shared-KKT path for the K <= 8 class: structure keys -> sort -> tiles of <= 8 scenarios -> prepare -> tile ADMM (DMMA) -> finish
 static int launch_qps(spectral_handle *h, const QpArgs &qa, const int *cstatus, int B, cudaStream_t st) {
   { const int rc = ensure_qps_buffers(h); if (rc) return rc; }
+  const QpsBuffers &q = h->qs;
   const size_t Bm = (size_t)h->max_batch;
-  int *head = h->qs_tmp, *gstart = h->qs_tmp + Bm, *flag = h->qs_tmp + 2 * Bm, *tidx = h->qs_tmp + 3 * Bm;
-  int *tile_start = h->qs_tile, *tile_count = h->qs_tile + Bm;
+  int *head = q.tmp.get(), *gstart = head + Bm, *flag = head + 2 * Bm, *tidx = head + 3 * Bm;
+  int *tile_start = q.tile.get(), *tile_count = tile_start + Bm;
   const int nb = (B + 255) / 256;
-  CK(cudaMemsetAsync(h->qs_misc, 0, 8, st));
+  CK(cudaMemsetAsync(q.misc.get(), 0, 8, st));
   const size_t sm_pf = 2 * (size_t)QP_SMEM_PER_WARP;
   const int pf_blocks = (B + 3) / 4;  // two scenarios per warp, two warps per block
   CK(cudaFuncSetAttribute(k_qps_prepare, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_pf));
   // hint pass: the K3 assembly of every scenario of the class with the interval pre-check forced on, no tile yet (leader = -1)
   QpsArgs Hh;
   memset(&Hh, 0, sizeof(Hh));
-  Hh.q = qa; Hh.q.lu = h->qs_lu; Hh.q.opt.precheck = 1;
+  Hh.q = qa; Hh.q.lu = q.lu.get(); Hh.q.opt.precheck = 1;
   if (!(Hh.q.opt.precheck_margin > 0.0)) Hh.q.opt.precheck_margin = 1e-3;
-  Hh.blk = h->qs_blk; Hh.qv = h->qs_qv; Hh.wrows = h->qs_w; Hh.xout = h->qs_x; Hh.st = h->qs_st;
-  CK(cudaMemsetAsync(h->qs_leader, 0xFF, (size_t)B * 4, st));
-  k_qps_prepare<<<pf_blocks, 64, sm_pf, st>>>(Hh, h->qs_leader);
+  Hh.blk = q.blk.get(); Hh.qv = q.qv.get(); Hh.wrows = q.w.get(); Hh.xout = q.x.get(); Hh.st = q.st.get();
+  CK(cudaMemsetAsync(q.leader.get(), 0xFF, (size_t)B * 4, st));
+  k_qps_prepare<<<pf_blocks, 64, sm_pf, st>>>(Hh, q.leader.get());
   h->launches++;
-  k_qps_keys<<<nb, 256, 0, st>>>(cstatus, qa.K, qa.segs, h->k_max, qa.weights, qa.wstride, B, h->qs_keys, h->qs_ids, h->qs_leader,
-                                h->qs_st);
-  size_t tb = h->qs_cub_bytes;
-  CK(cub::DeviceRadixSort::SortPairs(h->qs_cub, tb, h->qs_keys, h->qs_keys2, h->qs_ids, h->qs_ids2, B, 0, 64, st));
-  k_qps_heads<<<nb, 256, 0, st>>>(h->qs_keys2, B, head);
-  tb = h->qs_cub_bytes;
-  CK(cub::DeviceScan::InclusiveScan(h->qs_cub, tb, head, gstart, cub::Max(), B, st));
-  k_qps_flags<<<nb, 256, 0, st>>>(h->qs_keys2, gstart, B, flag);
-  tb = h->qs_cub_bytes;
-  CK(cub::DeviceScan::ExclusiveSum(h->qs_cub, tb, flag, tidx, B, st));
-  k_qps_emit<<<nb, 256, 0, st>>>(h->qs_keys2, h->qs_ids2, flag, tidx, B, tile_start, tile_count, h->qs_misc, h->qs_leader);
+  k_qps_keys<<<nb, 256, 0, st>>>(cstatus, qa.K, qa.segs, h->k_max, qa.weights, qa.wstride, B, q.keys.get(), q.ids.get(), q.leader.get(),
+                                q.st.get());
+  size_t tb = q.cub_bytes;
+  CK(cub::DeviceRadixSort::SortPairs(q.cub.get(), tb, q.keys.get(), q.keys2.get(), q.ids.get(), q.ids2.get(), B, 0, 64, st));
+  k_qps_heads<<<nb, 256, 0, st>>>(q.keys2.get(), B, head);
+  tb = q.cub_bytes;
+  CK(cub::DeviceScan::InclusiveScan(q.cub.get(), tb, head, gstart, cub::Max(), B, st));
+  k_qps_flags<<<nb, 256, 0, st>>>(q.keys2.get(), gstart, B, flag);
+  tb = q.cub_bytes;
+  CK(cub::DeviceScan::ExclusiveSum(q.cub.get(), tb, flag, tidx, B, st));
+  k_qps_emit<<<nb, 256, 0, st>>>(q.keys2.get(), q.ids2.get(), flag, tidx, B, tile_start, tile_count, q.misc.get(), q.leader.get());
   QpsArgs A;
-  A.q = qa; A.q.lu = h->qs_lu;
-  A.tile_start = tile_start; A.tile_count = tile_count; A.n_tiles = h->qs_misc; A.sorted = h->qs_ids2; A.tile_next = h->qs_misc + 1;
-  A.fs_scratch = h->qs_fs;
-  A.blk = h->qs_blk; A.qv = h->qs_qv; A.wrows = h->qs_w; A.xout = h->qs_x; A.st = h->qs_st;
+  A.q = qa; A.q.lu = q.lu.get();
+  A.tile_start = tile_start; A.tile_count = tile_count; A.n_tiles = q.misc.get(); A.sorted = q.ids2.get(); A.tile_next = q.misc.get() + 1;
+  A.fs_scratch = q.fs.get();
+  A.blk = q.blk.get(); A.qv = q.qv.get(); A.wrows = q.w.get(); A.xout = q.x.get(); A.st = q.st.get();
   CK(cudaFuncSetAttribute(k_qps_finish, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_pf));
   CK(cudaFuncSetAttribute(k_qps4, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Qps4Smem::BYTES));
-  k_qps_prepare<<<pf_blocks, 64, sm_pf, st>>>(A, h->qs_leader);
+  k_qps_prepare<<<pf_blocks, 64, sm_pf, st>>>(A, q.leader.get());
   const int per_sm = 2 * (Qps4Smem::BYTES + 1024 + 16) <= 227 * 1024 ? 2 : 1;
   const int grid = B < per_sm * h->sm_count ? B : per_sm * h->sm_count;
   k_qps4<<<grid, 128, Qps4Smem::BYTES, st>>>(A);
@@ -654,26 +668,26 @@ static int solve_device_impl(spectral_handle_t *h, int variant, int B, int N, in
   // K3a: weight tables
   const int wstride = sweep ? 1 : in->weights_stride;
   const int W = wstride ? B : 1;
-  k_tables<<<(2 * W + 127) / 128, 128, 0, st>>>(in->weights, h->mqm, W);
+  k_tables<<<(2 * W + 127) / 128, 128, 0, st>>>(in->weights, h->mqm.get(), W);
   h->launches++;
   if (tm) CK(cudaEventRecord(ev[evi++], st));
 
   // K1 + K2: corridors
-  CorridorArgs ca{sweep ? 1 : B, N, R, variant, h->k_max, delta_t, in->s_bounds, in->l_bounds, in->s_ref, in->l_ref, out->segs, out->K, h->cstatus};
+  CorridorArgs ca{sweep ? 1 : B, N, R, variant, h->k_max, delta_t, in->s_bounds, in->l_bounds, in->s_ref, in->l_ref, out->segs, out->K, h->cstatus.get()};
   if (spectral_corridor_prepare(N, R, &h->corridor_smem) != 0) return fail(h, SPECTRAL_ERR_CUDA, "corridor kernel: shared memory opt-in failed");
   spectral_launch_corridor(ca, st);
   h->launches++;
   CK(cudaGetLastError());
   if (sweep && B > 1) {
-    k_broadcast_corridor<<<(B + 255) / 256, 256, 0, st>>>(out->K, out->segs, h->cstatus, h->k_max, B);
+    k_broadcast_corridor<<<(B + 255) / 256, 256, 0, st>>>(out->K, out->segs, h->cstatus.get(), h->k_max, B);
     h->launches++;
   }
   if (tm) CK(cudaEventRecord(ev[evi++], st));
 
   // classification by segment count -> lane class lists
-  CK(cudaMemsetAsync(h->counts, 0, 4 * 2 * SP_NUM_CLASSES, st));
-  if (B <= 4096) k_classify_ordered<<<1, 1024, 0, st>>>(h->cstatus, out->K, B, h->lists, h->counts);
-  else k_classify<<<(B + 255) / 256, 256, 0, st>>>(h->cstatus, out->K, B, h->lists, h->counts);
+  CK(cudaMemsetAsync(h->counts.get(), 0, 4 * 2 * SP_NUM_CLASSES, st));
+  if (B <= 4096) k_classify_ordered<<<1, 1024, 0, st>>>(h->cstatus.get(), out->K, B, h->lists.get(), h->counts.get());
+  else k_classify<<<(B + 255) / 256, 256, 0, st>>>(h->cstatus.get(), out->K, B, h->lists.get(), h->counts.get());
   h->launches++;
   if (tm) CK(cudaEventRecord(ev[evi++], st));
 
@@ -682,25 +696,25 @@ static int solve_device_impl(spectral_handle_t *h, int variant, int B, int N, in
   qa.N = N; qa.k_max = h->k_max; qa.variant = variant; qa.delta = delta_t;
   qa.ds_bounds = in->ds_bounds; qa.dl_bounds = in->dl_bounds; qa.s_ref = in->s_ref; qa.l_ref = in->l_ref;
   qa.init = in->init; qa.scalars = in->scalars; qa.weights = in->weights; qa.wstride = wstride; qa.in_stride = sweep ? 0 : 1;
-  qa.mqm = h->mqm; qa.segs = out->segs; qa.K = out->K;
+  qa.mqm = h->mqm.get(); qa.segs = out->segs; qa.K = out->K;
   qa.opt.max_iter = opt.max_iter; qa.opt.scaling = opt.scaling; qa.opt.check_every = opt.check_termination;
   qa.opt.adapt_every = opt.adaptive_rho_interval; qa.opt.polish = opt.polish; qa.opt.polish_refine = opt.polish_refine_iter;
   qa.opt.eps_abs = opt.eps_abs; qa.opt.eps_rel = opt.eps_rel; qa.opt.eps_pinf = opt.eps_prim_inf; qa.opt.rho0 = opt.rho;
   qa.opt.sigma = opt.sigma; qa.opt.alpha = opt.alpha; qa.opt.adapt_tol = opt.adaptive_rho_tolerance;
   qa.opt.polish_delta = opt.polish_delta; qa.opt.polish_rounds = opt.polish_rounds;
   qa.opt.precheck = opt.infeasibility_precheck; qa.opt.precheck_margin = opt.precheck_margin;
-  qa.ctrl = out->ctrl; qa.axis_status = h->axis_status; qa.axis_iters = h->axis_iters; qa.axis_polished = h->axis_polished;
-  qa.axis_obj = h->axis_obj; qa.lu = out->lu;
+  qa.ctrl = out->ctrl; qa.axis_status = h->axis_status.get(); qa.axis_iters = h->axis_iters.get(); qa.axis_polished = h->axis_polished.get();
+  qa.axis_obj = h->axis_obj.get(); qa.lu = out->lu;
   // the solver classes are independent: fork them onto side streams, join before K5
   CK(cudaEventRecord(h->ev_fork, st));
   for (int cls = 0; cls < SP_NUM_CLASSES; cls++) {
     if (cls > 0 && class_kcap(cls - 1) >= h->k_max) break;  // class cannot occur with this handle's k_max
     cudaStream_t cs = cls == 0 ? st : h->side[cls - 1];
     if (cls > 0) CK(cudaStreamWaitEvent(cs, h->ev_fork, 0));
-    qa.list = h->lists + (size_t)cls * B; qa.count = h->counts + cls; qa.next = h->counts + SP_NUM_CLASSES + cls;
+    qa.list = h->lists.get() + (size_t)cls * B; qa.count = h->counts.get() + cls; qa.next = h->counts.get() + SP_NUM_CLASSES + cls;
     cudaEvent_t *ec = h->ev_cls[h->timed_calls % spectral_handle::kTimingSlots][cls];
     if (tm) CK(cudaEventRecord(ec[0], cs));
-    if (cls == 0 && opt.shared_kkt) { const int rc = launch_qps(h, qa, h->cstatus, B, cs); if (rc) return rc; }
+    if (cls == 0 && opt.shared_kkt) { const int rc = launch_qps(h, qa, h->cstatus.get(), B, cs); if (rc) return rc; }
     else if (cls == 0) CK((launch_qpa<8>(h, qa, B, cs)));
     else if (cls == 1) CK((launch_qpa<10>(h, qa, B, cs)));
     else if (cls == 2) CK((launch_qpd<12>(h, qa, B, cs)));
@@ -719,10 +733,10 @@ static int solve_device_impl(spectral_handle_t *h, int variant, int B, int N, in
   FinalArgs fa;
   fa.B = B; fa.N = N; fa.k_max = h->k_max; fa.variant = variant; fa.delta = delta_t; fa.s_ref = in->s_ref; fa.l_ref = in->l_ref;
   fa.init = in->init; fa.weights = in->weights; fa.wstride = wstride; fa.in_stride = sweep ? 0 : 1; fa.segs = out->segs; fa.K = out->K;
-  fa.cstatus = h->cstatus; fa.axis_status = h->axis_status; fa.axis_iters = h->axis_iters; fa.axis_polished = h->axis_polished;
-  fa.axis_obj = h->axis_obj; fa.ctrl = out->ctrl; fa.obj = out->obj; fa.a_cost = out->a_cost; fa.samples = out->samples;
+  fa.cstatus = h->cstatus.get(); fa.axis_status = h->axis_status.get(); fa.axis_iters = h->axis_iters.get(); fa.axis_polished = h->axis_polished.get();
+  fa.axis_obj = h->axis_obj.get(); fa.ctrl = out->ctrl; fa.obj = out->obj; fa.a_cost = out->a_cost; fa.samples = out->samples;
   fa.status = out->status; fa.iters = out->iters; fa.flags = out->flags; fa.npts = out->npts; fa.samples_cap = out->samples_cap;
-  k_finalize<<<(B + 127) / 128, 128, 0, st>>>(fa, h->work);
+  k_finalize<<<(B + 127) / 128, 128, 0, st>>>(fa, h->work.get());
   h->launches++;
   CK(cudaGetLastError());
   if (tm) {
@@ -732,18 +746,13 @@ static int solve_device_impl(spectral_handle_t *h, int variant, int B, int N, in
   return SPECTRAL_SUCCESS;
 }
 
-static int dev_alloc(spectral_handle *h, void **p, size_t bytes) {
-  CK(cudaMalloc(p, bytes));
-  return SPECTRAL_SUCCESS;
-}
-
+// a buffer of the host-buffer path that grows to the largest call so far; the old one is freed first (these are the large ones)
 template <typename T>
-static int ensure(spectral_handle *h, T **p, size_t *cur, size_t need) {
-  if (*cur >= need && *p) return SPECTRAL_SUCCESS;
-  if (*p) cudaFree(*p);
-  *p = nullptr;
-  CK(cudaMalloc((void **)p, need));
-  *cur = need;
+static int grow(spectral_handle *h, DevPtr<T> &p, size_t &bytes, size_t need) {
+  if (p && bytes >= need) return SPECTRAL_SUCCESS;
+  p.reset();
+  CK(cuda_alloc(p, need));
+  bytes = need;
   return SPECTRAL_SUCCESS;
 }
 
@@ -777,44 +786,44 @@ static int solve_async_impl(spectral_handle_t *h, int variant, int B, int N, int
                           hin->scalars, hin->weights};
   for (int i = 0; i < 9; i++) {
     if (!src[i]) return fail(h, SPECTRAL_ERR_INVALID, "null input");
-    int rc = ensure(h, &h->d_in[i], &h->d_in_bytes[i], in_bytes[i]);
+    int rc = grow(h, h->d_in[i], h->d_in_bytes[i], in_bytes[i]);
     if (rc) return rc;
-    CK(cudaMemcpyAsync(h->d_in[i], src[i], in_bytes[i], cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(h->d_in[i].get(), src[i], in_bytes[i], cudaMemcpyHostToDevice, st));
   }
-  {
+  if (!h->d_out.K) {
     const size_t mb = (size_t)h->max_batch;
-    int rc = SPECTRAL_SUCCESS;
-#define DEV_ALLOC(ptr, bytes) do { if (!(ptr) && rc == SPECTRAL_SUCCESS) rc = dev_alloc(h, (void **)&(ptr), (bytes)); } while (0)
-    DEV_ALLOC(h->d_K, mb * 4); DEV_ALLOC(h->d_status, mb * 4); DEV_ALLOC(h->d_iters, mb * 4); DEV_ALLOC(h->d_flags, mb * 4);
-    DEV_ALLOC(h->d_npts, mb * 4); DEV_ALLOC(h->d_segs, mb * km * sizeof(SpectralCube)); DEV_ALLOC(h->d_ctrl, mb * 12 * km * 8);
-    DEV_ALLOC(h->d_obj, mb * 8); DEV_ALLOC(h->d_cost, mb * 8);
-#undef DEV_ALLOC
-    if (rc) return rc;
+    HostPathBuffers m;
+    CK(cuda_alloc(m.K, mb * 4)); CK(cuda_alloc(m.status, mb * 4)); CK(cuda_alloc(m.iters, mb * 4)); CK(cuda_alloc(m.flags, mb * 4));
+    CK(cuda_alloc(m.npts, mb * 4)); CK(cuda_alloc(m.segs, mb * km * sizeof(SpectralCube))); CK(cuda_alloc(m.ctrl, mb * 12 * km * 8));
+    CK(cuda_alloc(m.obj, mb * 8)); CK(cuda_alloc(m.cost, mb * 8));
+    h->d_out = std::move(m);
   }
-  if (hout->samples) { int rc = ensure(h, &h->d_samples, &h->d_samples_bytes, b * (size_t)hout->samples_cap * 48); if (rc) return rc; }
-  if (hout->lu) { int rc = ensure(h, &h->d_lu, &h->d_lu_bytes, b * 2 * km * QP_ROWS * 16); if (rc) return rc; }
+  if (hout->samples) { int rc = grow(h, h->d_samples, h->d_samples_bytes, b * (size_t)hout->samples_cap * 48); if (rc) return rc; }
+  if (hout->lu) { int rc = grow(h, h->d_lu, h->d_lu_bytes, b * 2 * km * QP_ROWS * 16); if (rc) return rc; }
+  const HostPathBuffers &m = h->d_out;
   SpectralInputs din = *hin;
-  din.s_bounds = h->d_in[0]; din.l_bounds = h->d_in[1]; din.ds_bounds = h->d_in[2]; din.dl_bounds = h->d_in[3];
-  din.s_ref = h->d_in[4]; din.l_ref = h->d_in[5]; din.init = h->d_in[6]; din.scalars = h->d_in[7]; din.weights = h->d_in[8];
+  din.s_bounds = h->d_in[0].get(); din.l_bounds = h->d_in[1].get(); din.ds_bounds = h->d_in[2].get(); din.dl_bounds = h->d_in[3].get();
+  din.s_ref = h->d_in[4].get(); din.l_ref = h->d_in[5].get(); din.init = h->d_in[6].get(); din.scalars = h->d_in[7].get();
+  din.weights = h->d_in[8].get();
   SpectralOutputs dout;
   memset(&dout, 0, sizeof(dout));
-  dout.K = h->d_K; dout.segs = h->d_segs; dout.ctrl = h->d_ctrl; dout.obj = h->d_obj; dout.a_cost = h->d_cost;
-  dout.status = h->d_status; dout.iters = h->d_iters; dout.flags = h->d_flags; dout.npts = h->d_npts;
-  dout.samples = hout->samples ? h->d_samples : nullptr; dout.samples_cap = hout->samples_cap;
-  dout.lu = hout->lu ? h->d_lu : nullptr;
-  if (hout->lu) CK(cudaMemsetAsync(h->d_lu, 0, b * 2 * km * QP_ROWS * 16, st));
-  CK(cudaMemsetAsync(h->d_ctrl, 0, b * 12 * km * 8, st));
-  CK(cudaMemsetAsync(h->d_segs, 0, b * km * sizeof(SpectralCube), st));
-  if (hout->samples) CK(cudaMemsetAsync(h->d_samples, 0, b * (size_t)hout->samples_cap * 48, st));
+  dout.K = m.K.get(); dout.segs = m.segs.get(); dout.ctrl = m.ctrl.get(); dout.obj = m.obj.get(); dout.a_cost = m.cost.get();
+  dout.status = m.status.get(); dout.iters = m.iters.get(); dout.flags = m.flags.get(); dout.npts = m.npts.get();
+  dout.samples = hout->samples ? h->d_samples.get() : nullptr; dout.samples_cap = hout->samples_cap;
+  dout.lu = hout->lu ? h->d_lu.get() : nullptr;
+  if (hout->lu) CK(cudaMemsetAsync(dout.lu, 0, b * 2 * km * QP_ROWS * 16, st));
+  CK(cudaMemsetAsync(dout.ctrl, 0, b * 12 * km * 8, st));
+  CK(cudaMemsetAsync(dout.segs, 0, b * km * sizeof(SpectralCube), st));
+  if (hout->samples) CK(cudaMemsetAsync(dout.samples, 0, b * (size_t)hout->samples_cap * 48, st));
   int rc = solve_device_impl(h, variant, B, N, R, delta_t, &din, opt, &dout, st, sweep);
   if (rc) return rc;
 #define D2H(dst, srcp, bytes) do { if (dst) CK(cudaMemcpyAsync((dst), (srcp), (bytes), cudaMemcpyDeviceToHost, st)); } while (0)
-  D2H(hout->K, h->d_K, b * 4); D2H(hout->status, h->d_status, b * 4); D2H(hout->iters, h->d_iters, b * 4);
-  D2H(hout->flags, h->d_flags, b * 4); D2H(hout->npts, h->d_npts, b * 4);
-  D2H(hout->segs, h->d_segs, b * km * sizeof(SpectralCube)); D2H(hout->ctrl, h->d_ctrl, b * 12 * km * 8);
-  D2H(hout->obj, h->d_obj, b * 8); D2H(hout->a_cost, h->d_cost, b * 8);
-  D2H(hout->samples, h->d_samples, b * (size_t)hout->samples_cap * 48);
-  D2H(hout->lu, h->d_lu, b * 2 * km * QP_ROWS * 16);
+  D2H(hout->K, dout.K, b * 4); D2H(hout->status, dout.status, b * 4); D2H(hout->iters, dout.iters, b * 4);
+  D2H(hout->flags, dout.flags, b * 4); D2H(hout->npts, dout.npts, b * 4);
+  D2H(hout->segs, dout.segs, b * km * sizeof(SpectralCube)); D2H(hout->ctrl, dout.ctrl, b * 12 * km * 8);
+  D2H(hout->obj, dout.obj, b * 8); D2H(hout->a_cost, dout.a_cost, b * 8);
+  D2H(hout->samples, dout.samples, b * (size_t)hout->samples_cap * 48);
+  D2H(hout->lu, dout.lu, b * 2 * km * QP_ROWS * 16);
 #undef D2H
   return SPECTRAL_SUCCESS;
 }
@@ -851,7 +860,7 @@ extern "C" int spectral_argmin_device(spectral_handle_t *h, int B, const double 
   int blocks = (B + 255) / 256;
   const int cap = h->sm_count * 4 < 1024 ? h->sm_count * 4 : 1024;
   if (blocks > cap) blocks = cap;
-  k_argmin<<<blocks, 256, 0, st>>>(a_cost_dev, B, index_offset, h->partial, h->ticket, out_cost_dev, out_index_dev);
+  k_argmin<<<blocks, 256, 0, st>>>(a_cost_dev, B, index_offset, h->partial.get(), h->ticket.get(), out_cost_dev, out_index_dev);
   h->launches++;
   CK(cudaGetLastError());
   return SPECTRAL_SUCCESS;
@@ -859,23 +868,25 @@ extern "C" int spectral_argmin_device(spectral_handle_t *h, int B, const double 
 
 // ------------------------------------------------------------------ top-k selection (topk.cuh)
 static int ensure_topk_scratch(spectral_handle *h, cudaStream_t st) {
-  if (h->tk.cc) return SPECTRAL_SUCCESS;  // the last allocation: set only when all of them succeeded
+  if (h->tk.hist) return SPECTRAL_SUCCESS;
   const size_t hist_bytes = (size_t)TK_PASSES_MAX * TK_BINS * 4;
-  if (!h->tk.hist) CK(cudaMalloc(&h->tk.hist, hist_bytes));
-  if (!h->tk.st) CK(cudaMalloc(&h->tk.st, sizeof(TopkState)));
-  if (!h->tk.block_ties) CK(cudaMalloc(&h->tk.block_ties, TK_GRID_MAX * 4));
-  if (!h->tk.ck) CK(cudaMalloc(&h->tk.ck, TK_MAX * 8));
-  if (!h->tk.ci) CK(cudaMalloc(&h->tk.ci, TK_MAX * 8));
-  CK(cudaMemsetAsync(h->tk.hist, 0, hist_bytes, st));  // the kernels restore zero histograms, ticket and counter behind them
-  CK(cudaMemsetAsync(h->tk.st, 0, sizeof(TopkState), st));
-  CK(cudaMalloc(&h->tk.cc, TK_MAX * 8));
+  TopkBuffers t;
+  CK(cuda_alloc(t.hist, hist_bytes));
+  CK(cuda_alloc(t.st, sizeof(TopkState)));
+  CK(cuda_alloc(t.block_ties, TK_GRID_MAX * 4));
+  CK(cuda_alloc(t.ck, TK_MAX * 8));
+  CK(cuda_alloc(t.ci, TK_MAX * 8));
+  CK(cuda_alloc(t.cc, TK_MAX * 8));
+  CK(cudaMemsetAsync(t.hist.get(), 0, hist_bytes, st));  // the kernels restore zero histograms, ticket and counter behind them
+  CK(cudaMemsetAsync(t.st.get(), 0, sizeof(TopkState), st));
+  h->tk = std::move(t);
   return SPECTRAL_SUCCESS;
 }
 
 // npass + 2 launches: the radix passes (6 implicit, 12 explicit), compaction, finish (ties + sort + output)
 static int topk_run(spectral_handle *h, TopkArgs a, cudaStream_t st) {
   { const int rc = ensure_topk_scratch(h, st); if (rc) return rc; }
-  a.s = h->tk;
+  a.s = TopkScratch{h->tk.hist.get(), h->tk.st.get(), h->tk.block_ties.get(), h->tk.ck.get(), h->tk.ci.get(), h->tk.cc.get()};
   const long long per_block = (long long)TK_THREADS * TK_UNROLL;
   const int cap = 4 * h->sm_count < TK_GRID_MAX ? 4 * h->sm_count : TK_GRID_MAX;
   const long long want = ((long long)a.n + per_block - 1) / per_block;
@@ -1047,7 +1058,6 @@ struct NcclApi {
   ncclResult_t (*CommInitRank)(ncclComm_t *, int, ncclUniqueId, int) = nullptr;
   ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
   ncclResult_t (*AllGather)(const void *, void *, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
-  ncclResult_t (*Broadcast)(const void *, void *, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
   ncclResult_t (*AllReduce)(const void *, void *, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
   const char *(*GetErrorString)(ncclResult_t) = nullptr;
 };
@@ -1064,10 +1074,9 @@ NcclApi *nccl_api() {
       api.CommInitRank = (decltype(api.CommInitRank))dlsym(api.lib, "ncclCommInitRank");
       api.CommDestroy = (decltype(api.CommDestroy))dlsym(api.lib, "ncclCommDestroy");
       api.AllGather = (decltype(api.AllGather))dlsym(api.lib, "ncclAllGather");
-      api.Broadcast = (decltype(api.Broadcast))dlsym(api.lib, "ncclBroadcast");
       api.AllReduce = (decltype(api.AllReduce))dlsym(api.lib, "ncclAllReduce");
       api.GetErrorString = (decltype(api.GetErrorString))dlsym(api.lib, "ncclGetErrorString");
-      if (!api.GetUniqueId || !api.CommInitRank || !api.CommDestroy || !api.AllGather || !api.Broadcast || !api.AllReduce)
+      if (!api.GetUniqueId || !api.CommInitRank || !api.CommDestroy || !api.AllGather || !api.AllReduce)
         api.lib = nullptr;
     }
   }
@@ -1076,31 +1085,6 @@ NcclApi *nccl_api() {
 struct WinnerRec { double cost; long long idx; };
 // payload of a winner: K, then the segments, then the control points
 constexpr size_t kPayBytes = 16 + 32 * sizeof(SpectralCube) + 12 * 32 * 8;
-__global__ void k_pack_record(const double *cost, const long long *idx, WinnerRec *rec) { rec->cost = *cost; rec->idx = *idx; }
-__global__ void k_pick_winner(const WinnerRec *all, int nranks, WinnerRec *win, int *win_rank) {
-  ArgminPair best{1.0e300, 0x7fffffffffffffffLL};
-  int br = 0;
-  for (int r = 0; r < nranks; r++) {
-    const ArgminPair o{all[r].cost, all[r].idx};
-    const ArgminPair nb = argmin_better(best, o);
-    if (nb.idx != best.idx || nb.cost != best.cost) br = r;
-    best = nb;
-  }
-  win->cost = best.cost; win->idx = best.idx; *win_rank = br;
-}
-__global__ void k_pack_winner(const WinnerRec *win, long long offset, int B, int k_max, const int *K, const SpectralCube *segs, const double *ctrl,
-                              unsigned char *pay) {
-  const long long loc = win->idx - offset;
-  if (loc < 0 || loc >= B) return;  // not this rank's scenario
-  int *hdr = (int *)pay;
-  const int Kw = K[loc];
-  if (threadIdx.x == 0) { hdr[0] = Kw; hdr[1] = k_max; hdr[2] = 0; hdr[3] = 0; }
-  SpectralCube *ps = (SpectralCube *)(pay + 16);
-  double *pc = (double *)(pay + 16 + 32 * sizeof(SpectralCube));
-  for (int k = threadIdx.x; k < 32; k += blockDim.x)
-    if (k < Kw && k < k_max) ps[k] = segs[(size_t)loc * k_max + k];
-  for (int j = threadIdx.x; j < 12 * 32; j += blockDim.x) pc[j] = (j < 12 * Kw && j < 12 * k_max) ? ctrl[(size_t)loc * 12 * k_max + j] : 0.0;
-}
 // top-k exchange: slot j of the payload buffer gets winner j's payload from the rank that owns it (header: K, rank, 1, 0);
 // every other rank leaves the slot zero, so a byte-wise sum over ranks reproduces it exactly
 __global__ void k_pack_topk(const WinnerRec *win, int rank, long long offset, int B, int k_max, const int *K, const SpectralCube *segs,
@@ -1140,9 +1124,6 @@ extern "C" int spectral_comm_init(spectral_handle_t *h, int nranks, int rank, co
   CK(cudaSetDevice(h->device));
   if (h->comm) spectral_comm_destroy(h);
   h->nranks = nranks; h->rank = rank;
-  if (h->xg_rec) { cudaFree(h->xg_rec); h->xg_rec = nullptr; }
-  CK(cudaMalloc(&h->xg_rec, (size_t)(4 + nranks) * sizeof(WinnerRec)));
-  if (!h->xg_pay) CK(cudaMalloc(&h->xg_pay, kPayBytes));
   if (nranks == 1) return SPECTRAL_SUCCESS;
   NcclApi *n = nccl_api();
   if (!n || !id) return fail(h, SPECTRAL_ERR_CUDA, "NCCL is not available (libnccl.so.2 could not be loaded)");
@@ -1163,77 +1144,25 @@ extern "C" int spectral_comm_destroy(spectral_handle_t *h) {
   return SPECTRAL_SUCCESS;
 }
 
-extern "C" int spectral_sweep_argmin(spectral_handle_t *h, int B_local, const SpectralOutputs *dev_out, long long index_offset,
-                                     SpectralWinner *winner, void *cuda_stream) {
-  if (!h || !dev_out || !winner || B_local <= 0 || !dev_out->a_cost || !dev_out->K || !dev_out->segs || !dev_out->ctrl) return SPECTRAL_ERR_INVALID;
+// The k best entries of the sweep on every rank (spectral_sweep_topk; spectral_sweep_argmin is k = 1); the callers check the arguments
+static int sweep_select(spectral_handle *h, int B_local, const SpectralOutputs *dev_out, long long index_offset, int k,
+                        SpectralWinner *winners, int *n_out, cudaStream_t st) {
   CK(cudaSetDevice(h->device));
-  if (!h->xg_rec) { const int rc = spectral_comm_init(h, 1, 0, nullptr); if (rc) return rc; }
-  cudaStream_t st = (cudaStream_t)cuda_stream;
-  WinnerRec *rec = (WinnerRec *)h->xg_rec;          // [0] local, [1] winner, [2 ..] gathered, [2 + nranks] scratch (cost, idx)
-  WinnerRec *win = rec + 1, *all = rec + 2;
-  double *tmp_cost = (double *)(rec + 2 + h->nranks);
-  long long *tmp_idx = (long long *)(tmp_cost + 1);
-  int *win_rank = (int *)(rec + 3 + h->nranks);
-  int rc = spectral_argmin_device(h, B_local, dev_out->a_cost, index_offset, tmp_cost, tmp_idx, st);
-  if (rc) return rc;
-  k_pack_record<<<1, 1, 0, st>>>(tmp_cost, tmp_idx, rec);
-  NcclApi *n = h->nranks > 1 ? nccl_api() : nullptr;
-  if (h->nranks > 1) {
-    if (!n || !h->comm) return fail(h, SPECTRAL_ERR_INVALID, "spectral_comm_init has not been called on this handle");
-    if (n->AllGather(rec, all, sizeof(WinnerRec), ncclUint8, h->comm, st) != ncclSuccess) return fail(h, SPECTRAL_ERR_CUDA, "ncclAllGather");
-  } else {
-    CK(cudaMemcpyAsync(all, rec, sizeof(WinnerRec), cudaMemcpyDeviceToDevice, st));
-  }
-  k_pick_winner<<<1, 1, 0, st>>>(all, h->nranks, win, win_rank);
-  k_pack_winner<<<1, 128, 0, st>>>(win, index_offset, B_local, h->k_max, dev_out->K, dev_out->segs, dev_out->ctrl, h->xg_pay);
-  h->launches += 3;
-  WinnerRec hw;
-  int hr = 0;
-  CK(cudaMemcpyAsync(&hw, win, sizeof(WinnerRec), cudaMemcpyDeviceToHost, st));
-  CK(cudaMemcpyAsync(&hr, win_rank, sizeof(int), cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st));
-  if (h->nranks > 1 && n->Broadcast(h->xg_pay, h->xg_pay, kPayBytes, ncclUint8, hr, h->comm, st) != ncclSuccess)
-    return fail(h, SPECTRAL_ERR_CUDA, "ncclBroadcast");
-  static unsigned char hostpay[kPayBytes];  // (a handle is not thread-safe; one exchange at a time per process)
-  CK(cudaMemcpyAsync(hostpay, h->xg_pay, kPayBytes, cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st));
-  memset(winner, 0, sizeof(*winner));
-  winner->cost = hw.cost; winner->index = hw.idx; winner->rank = hr;
-  const int *hdr = (const int *)hostpay;
-  winner->K = hdr[0];
-  memcpy(winner->segs, hostpay + 16, 32 * sizeof(SpectralCube));
-  memcpy(winner->ctrl, hostpay + 16 + 32 * sizeof(SpectralCube), 12 * 32 * 8);
-  return SPECTRAL_SUCCESS;
-}
-
-extern "C" int spectral_sweep_topk(spectral_handle_t *h, int B_local, const SpectralOutputs *dev_out, long long index_offset, int k,
-                                   SpectralWinner *winners, int *n_out, void *cuda_stream) {
-  if (!h) return SPECTRAL_ERR_INVALID;
-  if (k < 1 || k > SPECTRAL_TOPK_MAX) return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: k must be in [1, SPECTRAL_TOPK_MAX]");
-  if (B_local < 0) return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: B_local must be non-negative");
-  if (index_offset < 0) return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: index_offset must be non-negative");
-  if (!dev_out || !winners || !n_out) return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: NULL pointer");
-  if (B_local > 0 && (!dev_out->a_cost || !dev_out->K || !dev_out->segs || !dev_out->ctrl))
-    return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: a_cost/K/segs/ctrl are required");
-  CK(cudaSetDevice(h->device));
-  cudaStream_t st = (cudaStream_t)cuda_stream;
   const bool multi = h->nranks > 1;
   NcclApi *n = multi ? nccl_api() : nullptr;
   if (multi && (!n || !h->comm)) return fail(h, SPECTRAL_ERR_INVALID, "spectral_comm_init has not been called on this handle");
   const int nr = multi ? h->nranks : 1;
-  if (h->tk_cap < k || h->tk_cap_ranks < nr) {  // sized by k and the number of ranks, never by the batch
-    if (h->tk_rec) cudaFree(h->tk_rec);
-    if (h->tk_pay) cudaFree(h->tk_pay);
-    if (h->tk_hostpay) cudaFreeHost(h->tk_hostpay);
-    if (h->tk_hostrec) cudaFreeHost(h->tk_hostrec);
-    h->tk_rec = nullptr; h->tk_pay = nullptr; h->tk_hostpay = nullptr; h->tk_hostrec = nullptr; h->tk_cap = 0;
-    CK(cudaMalloc(&h->tk_rec, (size_t)(2 + nr) * k * sizeof(WinnerRec)));
-    CK(cudaMalloc(&h->tk_pay, (size_t)k * kPayBytes));
-    CK(cudaHostAlloc(&h->tk_hostpay, (size_t)k * kPayBytes, cudaHostAllocDefault));
-    CK(cudaHostAlloc(&h->tk_hostrec, (size_t)k * sizeof(WinnerRec), cudaHostAllocDefault));
-    h->tk_cap = k; h->tk_cap_ranks = nr;
+  if (h->sw.cap < k || h->sw.ranks < nr) {
+    SweepBuffers s;
+    CK(cuda_alloc(s.rec, (size_t)(2 + nr) * k * sizeof(WinnerRec)));
+    CK(cuda_alloc(s.pay, (size_t)k * kPayBytes));
+    CK(cuda_alloc(s.host_pay, (size_t)k * kPayBytes));
+    CK(cuda_alloc(s.host_rec, (size_t)k * sizeof(WinnerRec)));
+    s.cap = k; s.ranks = nr;
+    h->sw = std::move(s);
   }
-  WinnerRec *loc = (WinnerRec *)h->tk_rec, *merged = loc + k, *all = loc + 2 * k;
+  unsigned char *pay = h->sw.pay.get();
+  WinnerRec *loc = (WinnerRec *)h->sw.rec.get(), *merged = loc + k, *all = loc + 2 * k;
   if (B_local > 0) {
     const int rc = topk_implicit(h, B_local, dev_out->a_cost, index_offset, k, &loc->cost, &loc->idx, 2, st);
     if (rc) return rc;
@@ -1253,26 +1182,26 @@ extern "C" int spectral_sweep_topk(spectral_handle_t *h, int B_local, const Spec
     win = merged;
   }
   // phase 2: payloads of the winners this rank owns, summed over ranks
-  CK(cudaMemsetAsync(h->tk_pay, 0, (size_t)k * kPayBytes, st));
-  k_pack_topk<<<k, 128, 0, st>>>(win, multi ? h->rank : 0, index_offset, B_local, h->k_max, dev_out->K, dev_out->segs, dev_out->ctrl, h->tk_pay);
+  CK(cudaMemsetAsync(pay, 0, (size_t)k * kPayBytes, st));
+  k_pack_topk<<<k, 128, 0, st>>>(win, multi ? h->rank : 0, index_offset, B_local, h->k_max, dev_out->K, dev_out->segs, dev_out->ctrl, pay);
   h->launches++;
   CK(cudaGetLastError());
-  if (multi && n->AllReduce(h->tk_pay, h->tk_pay, (size_t)k * kPayBytes, ncclUint8, ncclSum, h->comm, st) != ncclSuccess)
+  if (multi && n->AllReduce(pay, pay, (size_t)k * kPayBytes, ncclUint8, ncclSum, h->comm, st) != ncclSuccess)
     return fail(h, SPECTRAL_ERR_CUDA, "ncclAllReduce");
-  WinnerRec *hrec = (WinnerRec *)h->tk_hostrec;
+  WinnerRec *hrec = (WinnerRec *)h->sw.host_rec.get();
   CK(cudaMemcpyAsync(hrec, win, (size_t)k * sizeof(WinnerRec), cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
   int cnt = 0;
   while (cnt < k && hrec[cnt].idx >= 0) cnt++;
   if (cnt) {
-    CK(cudaMemcpyAsync(h->tk_hostpay, h->tk_pay, (size_t)cnt * kPayBytes, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(h->sw.host_pay.get(), pay, (size_t)cnt * kPayBytes, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
   }
   for (int j = 0; j < k; j++) {
     SpectralWinner *w = winners + j;
     memset(w, 0, sizeof(*w));
     if (j >= cnt) { w->cost = __builtin_huge_val(); w->index = -1; w->rank = -1; continue; }
-    const unsigned char *p = h->tk_hostpay + (size_t)j * kPayBytes;
+    const unsigned char *p = h->sw.host_pay.get() + (size_t)j * kPayBytes;
     const int *hdr = (const int *)p;
     w->cost = hrec[j].cost; w->index = hrec[j].idx; w->rank = hdr[1]; w->K = hdr[0];
     memcpy(w->segs, p + 16, 32 * sizeof(SpectralCube));
@@ -1280,6 +1209,26 @@ extern "C" int spectral_sweep_topk(spectral_handle_t *h, int B_local, const Spec
   }
   *n_out = cnt;
   return SPECTRAL_SUCCESS;
+}
+
+extern "C" int spectral_sweep_argmin(spectral_handle_t *h, int B_local, const SpectralOutputs *dev_out, long long index_offset,
+                                     SpectralWinner *winner, void *cuda_stream) {
+  if (!h || !dev_out || !winner || B_local <= 0 || !dev_out->a_cost || !dev_out->K || !dev_out->segs || !dev_out->ctrl) return SPECTRAL_ERR_INVALID;
+  if (index_offset < 0) return fail(h, SPECTRAL_ERR_INVALID, "sweep_argmin: index_offset must be non-negative");
+  int n = 0;
+  return sweep_select(h, B_local, dev_out, index_offset, 1, winner, &n, (cudaStream_t)cuda_stream);
+}
+
+extern "C" int spectral_sweep_topk(spectral_handle_t *h, int B_local, const SpectralOutputs *dev_out, long long index_offset, int k,
+                                   SpectralWinner *winners, int *n_out, void *cuda_stream) {
+  if (!h) return SPECTRAL_ERR_INVALID;
+  if (k < 1 || k > SPECTRAL_TOPK_MAX) return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: k must be in [1, SPECTRAL_TOPK_MAX]");
+  if (B_local < 0) return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: B_local must be non-negative");
+  if (index_offset < 0) return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: index_offset must be non-negative");
+  if (!dev_out || !winners || !n_out) return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: NULL pointer");
+  if (B_local > 0 && (!dev_out->a_cost || !dev_out->K || !dev_out->segs || !dev_out->ctrl))
+    return fail(h, SPECTRAL_ERR_INVALID, "sweep_topk: a_cost/K/segs/ctrl are required");
+  return sweep_select(h, B_local, dev_out, index_offset, k, winners, n_out, (cudaStream_t)cuda_stream);
 }
 
 extern "C" int spectral_measure_fp64_peak(spectral_handle_t *h, double *tflops) {

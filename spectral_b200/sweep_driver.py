@@ -4,9 +4,9 @@ Scenarios come from the config-4 generator (mixed trapezoid-prism + cuboid corri
 five base fixtures x two variants = ten families of obstacle-perturbed scenarios with extra slope breaks, dealt
 round-robin in chunks of 8192: global scenario index = chunk * 8192 + position.  Rank r takes a CONTIGUOUS range of the
 global index (SURVEY.md 8e), i.e. of chunks; no data-path collective.  The sweep ends with the ONE exchange of the path: the
-best trajectory (arg-min of a_cost, ties -> lowest global index) through the C-ABI's spectral_sweep_argmin (NCCL
-all-gather of the 16-byte records + broadcast of the winner from its owner).  The winner does not depend on the number
-of ranks.
+best trajectory (arg-min of a_cost, ties -> lowest global index) through the C-ABI's spectral_sweep_argmin (top-k with
+k = 1: NCCL all-gather of the 16-byte records, then an all-reduce of the winner's payload from its owner).  The winner
+does not depend on the number of ranks.
 """
 from __future__ import annotations
 

@@ -373,7 +373,7 @@ def test_device_resident_path_and_argmin(planner):
 
 
 def test_sweep_argmin_through_the_c_abi():
-    """Config-5 path at test size, one rank: spectral_sweep_argmin (k_argmin -> record -> winner payload) returns the arg-min
+    """Config-5 path at test size, one rank: spectral_sweep_argmin (top-k with k = 1 -> winner payload) returns the arg-min
     scenario's K / segments / control points; cutting the same sweep into two contiguous shards (what two ranks would run)
     gives the same winner -- it does not depend on the number of ranks (ties -> lowest global index)."""
     import torch

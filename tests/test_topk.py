@@ -213,6 +213,33 @@ def test_sweep_topk_on_real_solves(planner):
     pl.close()
 
 
+def test_sweep_argmin_without_a_cost_below_1e300(planner):
+    """Every cost NaN, every cost +inf, or a mix of NaN, +inf and values above 1e300: sweep_argmin still returns a real
+    scenario, the first in top-k order, with its own K, segments and control points (zero beyond K)."""
+    import torch
+    total, km, off = 600, planner.k_max, 7
+    _, K, segs, ctrl = _synthetic(total, km)
+    mixed = np.full(total, np.nan)
+    mixed[[3, 100, 450]] = [np.inf, 3e300, 2e300]
+    lib = planner._lib
+    for costs, j in ((np.full(total, np.nan), 0), (np.full(total, np.inf), 0), (mixed, 450)):
+        outs = dict(a_cost=torch.from_numpy(costs).cuda(), K=torch.from_numpy(K).cuda(), segs=torch.from_numpy(segs).cuda(),
+                    ctrl=torch.from_numpy(ctrl).cuda())
+        best = planner.sweep_argmin(outs, off)
+        _same_winners([best], planner.sweep_topk(outs, off, 1))
+        assert best["index"] == off + j and best["rank"] == 0 and best["K"] == K[j]
+        assert np.float64(best["cost"]).view(np.int64) == costs[j:j + 1].view(np.int64)[0]
+        assert best["segs"].tobytes() == segs[j, :112 * K[j]].tobytes() and best["ctrl"].tobytes() == ctrl[j, :12 * K[j]].tobytes()
+        out = api.SpectralOutputs()
+        out.a_cost = ctypes.cast(ctypes.c_void_p(outs["a_cost"].data_ptr()), ctypes.POINTER(ctypes.c_double))
+        out.K = ctypes.cast(ctypes.c_void_p(outs["K"].data_ptr()), ctypes.POINTER(ctypes.c_int))
+        out.segs = outs["segs"].data_ptr()
+        out.ctrl = ctypes.cast(ctypes.c_void_p(outs["ctrl"].data_ptr()), ctypes.POINTER(ctypes.c_double))
+        w = api.SpectralWinner()
+        assert lib.spectral_sweep_argmin(planner._h, total, ctypes.byref(out), off, ctypes.byref(w), None) == 0
+        assert not any(bytes(w.segs)[112 * K[j]:]) and not any(w.ctrl[12 * K[j]:])
+
+
 # ---------------------------------------------------------------- 6: two real NCCL ranks
 def _synthetic(total, k_max):
     rng = np.random.default_rng(2024)
@@ -246,17 +273,26 @@ def _nccl_worker(rank, world, total, k, id_q, res_q):
         pl = api.SpectralPlanner(device=rank, max_batch=1024, n_max=128, r_max=8, k_max=k_max)
         pl.comm_init(world, rank, uid)
         lo, hi = rank * total // world, (rank + 1) * total // world
-        sharded = pl.sweep_topk({n: t[lo:hi] for n, t in outs.items()}, lo, k)
+        shard = {n: t[lo:hi] for n, t in outs.items()}
+        sharded = pl.sweep_topk(shard, lo, k)
         # second call: rank 0 holds the whole sweep, rank 1 takes part with B_local = 0
         skew = pl.sweep_topk(outs, 0, k, B=total if rank == 0 else 0)
+        # sweep_argmin is sweep_topk with k = 1, on the sharded split and on a skewed one (it needs B_local >= 1: rank 1
+        # holds the last scenario only)
+        lo1 = 0 if rank == 0 else total - 1
+        shard1 = {n: t[lo1:] for n, t in outs.items()}
+        B1 = total - 1 if rank == 0 else 1
+        argmins = []
+        for part, off, B_part in ((shard, lo, None), (shard1, lo1, B1)):
+            argmins.append((_pack([pl.sweep_argmin(part, off, B=B_part)]), _pack(pl.sweep_topk(part, off, 1, B=B_part))))
         single = api.SpectralPlanner(device=rank, max_batch=1024, n_max=128, r_max=8, k_max=k_max)
         ref = single.sweep_topk(outs, 0, k)
         torch.cuda.synchronize()
         pl.close()
         single.close()
-        res_q.put((rank, "ok", _pack(sharded), _pack(skew), _pack(ref)))
+        res_q.put((rank, "ok", _pack(sharded), _pack(skew), _pack(ref), argmins))
     except Exception as e:  # reported to the parent, which fails the test
-        res_q.put((rank, "error: %r" % (e,), None, None, None))
+        res_q.put((rank, "error: %r" % (e,), None, None, None, None))
 
 
 def test_sweep_topk_two_nccl_ranks():
@@ -296,6 +332,9 @@ def test_sweep_topk_two_nccl_ranks():
         assert [w[:2] + w[3:] for w in sharded] == [w[:2] + w[3:] for w in ref]
         assert [w[2] for w in sharded] == [int(w[1] >= total // 2) for w in ref]
         assert [w[:2] + w[3:] for w in skew] == [w[:2] + w[3:] for w in ref] and all(w[2] == 0 for w in skew)
+        for argmin, top1 in results[r][5]:
+            assert argmin == top1
+            assert argmin[0][:2] + argmin[0][3:] == ref[0][:2] + ref[0][3:]
     j = ref[0][1]
     assert ref[0][4] == segs[j].tobytes()[:ref[0][3] * 112] and ref[0][5] == ctrl[j, :12 * ref[0][3]].tobytes()
 
@@ -356,6 +395,17 @@ def test_topk_invalid_arguments(planner):
     assert lib.spectral_sweep_topk(h, 8, ctypes.byref(out), 0, 4, None, ctypes.byref(n), None) == INVALID
     assert lib.spectral_sweep_topk(h, 8, ctypes.byref(out), 0, 4, ws, None, None) == INVALID
     assert lib.spectral_sweep_topk(h, 8, ctypes.byref(out), 0, 4, ws, ctypes.byref(n), None) == INVALID  # K/segs/ctrl missing
+    full = api.SpectralOutputs()
+    full.a_cost = ctypes.cast(P(outs["a_cost"]), ctypes.POINTER(ctypes.c_double))
+    full.K = ctypes.cast(P(outs["K"]), ctypes.POINTER(ctypes.c_int))
+    full.segs = outs["segs"].data_ptr()
+    full.ctrl = ctypes.cast(P(outs["ctrl"]), ctypes.POINTER(ctypes.c_double))
+    w = api.SpectralWinner()
+    assert lib.spectral_sweep_argmin(h, 8, ctypes.byref(full), -1, ctypes.byref(w), None) == INVALID
+    assert b"index_offset" in lib.spectral_last_error(h)
+    assert lib.spectral_sweep_argmin(h, 0, ctypes.byref(full), 0, ctypes.byref(w), None) == INVALID
+    assert lib.spectral_sweep_argmin(h, 8, ctypes.byref(out), 0, ctypes.byref(w), None) == INVALID   # K/segs/ctrl missing
+    assert lib.spectral_sweep_argmin(h, 8, ctypes.byref(full), 0, ctypes.byref(w), None) == 0
     # the handle still works after the refused calls
     oc2, oi2 = planner.topk_device(torch.arange(8, 0, -1, dtype=torch.float64, device="cuda"), 3)
     torch.cuda.synchronize()
